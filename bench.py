@@ -3,10 +3,12 @@
 
     python bench.py --gpus N --steps K --warmup W            # N > 1: launched by torch.distributed.run, one rank per GPU
     python bench.py --impl reference --steps K --warmup W    # the REFERENCE's own processor on the host CPU cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/*.npy
 
 A "step" is one transformer forward (= one denoise step, no CFG doubling) over one synthetic latent video with
 random-init weights of the named architecture.  One JSON line is printed by rank 0 (see README / DESIGN.md section 6
-for every field).  Workloads (BASELINE.json configs):
+for every field).  Inputs and weights are seeded, so two builds run with the same arguments can be compared output for
+output through --dump-outputs.  Workloads (BASELINE.json configs):
     wan14 (default): Wan2.1-T2V-14B, 720p x 81 f -> 21x45x80 = 75,600 tokens, 40 heads, 40 blocks  [configs[2]]
     wan13          : Wan2.1-T2V-1.3B, 480p x 81 f -> 21x30x52 = 32,760 tokens, 12 heads, 30 blocks [configs[1]]
 The default is the same for every N so that the driver's 1/2/4/8 scaling ratios compare like with like (12 heads
@@ -19,7 +21,9 @@ self-attention layer (12 heads, 32,760 tokens) through the reference's WanAttnPr
 extrapolation: its `value` is the measured time of its step, and `cpu_baseline.sample` says what share of the full
 workload one such step is.  The GPU arm runs the SAME layer on the same inputs through vorta_b200's processor of the
 same name (`like_for_like`, resident and with host buffers) next to the reference timed on the box's cores in the
-same run (`cpu_baseline`), and compares the two outputs.
+same run (`cpu_baseline`), and compares the two outputs.  The reference is not part of this repository: where neither
+its source (VORTA_REFERENCE_ROOT) nor a staged copy is present, `--impl reference` exits with that message and the GPU
+arm reports `cpu_baseline` as unavailable instead of timing anything else under its name.
 """
 from __future__ import annotations
 
@@ -78,6 +82,26 @@ def recorded_traffic(workload):
     except (OSError, ValueError, KeyError, TypeError):
         pass
     return out
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(directory, arrays):
+    """Writes each tensor of `arrays` as <directory>/<name>.npy in float32, within DUMP_BYTES in all.  A tensor larger
+    than its even share is replaced by a 1-D sample of its flattened elements: one position drawn from a fixed seed in
+    each of `share` equal strides, so two runs with the same arguments sample the same positions."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    share = (DUMP_BYTES - 4096 * len(arrays)) // (4 * len(arrays))        # elements; 4 KB left for each .npy header
+    for name, t in arrays.items():
+        t = t.detach().float().cpu()
+        if t.numel() > share:
+            edges = torch.arange(share + 1, dtype=torch.float64) * (t.numel() / share)
+            u = torch.rand(share, dtype=torch.float64, generator=torch.Generator().manual_seed(0))
+            t = t.flatten()[(edges[:-1] + u * (edges[1:] - edges[:-1])).long().clamp_(max=t.numel() - 1)]
+        np.save(os.path.join(directory, f"{name}.npy"), t.numpy())
 
 
 class ClockSampler:
@@ -189,15 +213,28 @@ def reference_leg(wl, n_timed, n_warm, threads=None, keep_output=False):
                 out=out if keep_output else None, flops=RL.algorithmic_flops(cpu_sample_cfg(wl)))
 
 
+def reference_missing():
+    """None when the reference's own files can be imported, else why not (the reference is not part of this
+    repository, and nothing else is timed under its name)."""
+    from oracle import ref_loader
+    if ref_loader.available():
+        return None
+    return ("reference not available: neither VORTA_REFERENCE_ROOT (a checkout of wenhao728/VORTA) nor a staged copy "
+            "under oracle/_ref (oracle/stage_ref.py)")
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return                                   # rank 0 alone runs the CPU arm; the other ranks exit 0
+    missing = reference_missing()
+    if missing:
+        raise SystemExit(f"bench.py --impl reference: {missing}")
     cores = host_cores()
     os.environ["OMP_NUM_THREADS"] = str(cores)   # torchrun exports OMP_NUM_THREADS=1; must be set before torch loads
     os.environ["MKL_NUM_THREADS"] = str(cores)
     wl = WORKLOADS[args.workload]
-    r = reference_leg(wl, args.steps, args.warmup, threads=cores)
+    r = reference_leg(wl, args.steps, args.warmup, threads=cores, keep_output=bool(args.dump_outputs))
     value = statistics.mean(r["ms"])
     share = sample_share(wl)
     sample = (f"each step = ONE real call of the reference's own WanAttnProcessorTripleEval "
@@ -216,6 +253,8 @@ def run_reference(args):
                 like_for_like=dict(workload="BASELINE configs[0]", reference_cpu_ms=value),
                 e2e=dict(value=value, unit="ms", h2d_bytes_per_step=0, d2h_bytes_per_step=0),
                 gpu_launches=0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(hidden_states=r["out"]))
     print(json.dumps(line), flush=True)
 
 
@@ -327,9 +366,14 @@ def run_workload(wl, args, rank, world, device, with_e2e=True):
 
     call = make_step(model, wl, device, kw)
 
+    last = {}
+
     @torch.no_grad()
     def step_resident():
-        return call(lat_d, ts_d, txt_d)[0]
+        out = call(lat_d, ts_d, txt_d)[0]
+        if args.dump_outputs:          # kept only for a dump: holding it across steps changes what the allocator reuses
+            last["sample"] = out
+        return out
 
     @torch.no_grad()
     def step_e2e():
@@ -361,6 +405,7 @@ def run_workload(wl, args, rank, world, device, with_e2e=True):
     sampler.start()
     ms = time_steps(step_resident, args.steps, args.warmup, dist_on, profile=args.profile, after_warmup=reset_counters)
     clocks = sampler.stop()
+    outputs = {name: t.float().cpu() for name, t in last.items()} if args.dump_outputs else None
     ops.timing_enable(False)
     kinds = ops.timing_collect_kinds()
     launches_step = ops.stats()[0] / args.steps
@@ -400,7 +445,7 @@ def run_workload(wl, args, rank, world, device, with_e2e=True):
     return dict(ms=ms, e2e_ms=e2e_ms, clocks=clocks, counts=counts, attn_ms_step=attn_ms_step,
                 attn_flops_step=attn_flops_step, per_kind=per, launches_step=launches_step, job_flops=job_flops,
                 attn_ms_max=attn_ms_max, attn_ms_ranks=attn_ms_ranks, nvlink_tx_step=nvlink_tx_step,
-                formula_flops_step=formula,
+                formula_flops_step=formula, outputs=outputs,
                 h2d=lat_h.numel() * 2 + txt_h.numel() * 2 + 4, d2h=out_h.numel() * 2, cfg=cfg)
 
 
@@ -444,7 +489,10 @@ def like_for_like_leg(args, device, with_cpu=True):
                gpu_tflops=flops["total"] / (ms * 1e-3) / 1e12,
                api="vorta_b200.attention.WanAttnProcessorTripleEval.__call__ (the reference's processor signature)")
     cpu = None
-    if with_cpu:
+    missing = reference_missing() if with_cpu else None
+    if missing:
+        cpu = dict(kind="reference", available=False, value=None, unit="ms", reason=missing)
+    elif with_cpu:
         out_gpu = resident().float().cpu()
         r = reference_leg(WORKLOADS[args.workload], 2, 1, keep_output=True)
         ref = r["out"].float()
@@ -655,6 +703,8 @@ def run_gpu(args):
                                cross_attn_tflops=rate(a["per_kind"]["dense"]["flops_step"],
                                                       a["per_kind"]["dense"]["ms_step"]))
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, r["outputs"])
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -670,6 +720,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-aux", action="store_true")
     ap.add_argument("--profile", action="store_true", help="bracket one warmed-up step with cudaProfilerStart/Stop")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     if args.impl == "reference":

@@ -789,6 +789,41 @@ def test_bf16_router_matches_reference_router_in_bf16():
     assert strict > 0.5 * total
 
 
+def test_bf16_router_matches_golden_reference_router_in_bf16(golden):
+    """The same bar as above without the reference's files: the weights, inputs and fp32 scores of the reference's own
+    ``Router`` (tests/golden/router.pt).  The reference's forward, softmax(linear(silu(temb)).unflatten(1, (H, 3))) in
+    plain torch functions (router.py:41-43), first reproduces the reference's fp32 scores, which pins the expression and
+    the (head, branch) layout; evaluated in bf16 on the GPU it is then what the reference's module computes in bf16."""
+    import torch.nn.functional as F
+
+    def reference_forward(temb, w, b, H):
+        return torch.softmax(F.linear(F.silu(temb), w, b).unflatten(1, (H, 3)), dim=-1)
+
+    strict = total = 0
+    for rec in golden("router.pt"):
+        H = rec["H"]
+        assert torch.allclose(reference_forward(rec["temb"], rec["weight"], rec["bias"], H), rec["score"], atol=1e-6)
+        w, b, temb = (rec[n].to(dev(), torch.bfloat16) for n in ("weight", "bias", "temb"))
+        with torch.no_grad():
+            want = reference_forward(temb, w, b, H)                                      # (B, H, 3) bf16
+        got = ops.router_forward(temb, w, b, H)[0][0]
+        assert torch.equal(got, got.to(torch.bfloat16).float())
+        ulp = want.float().abs() * 2.0 ** -7
+        assert bool(((got - want.float()).abs() <= ulp).all())
+        for tau in (0.3, 0.36):
+            _, branch = ops.router_forward(temb, w, b, H, tau)
+            s, idx = want[0].topk(1, dim=-1)                                              # wan.py:398-400
+            idx = idx.clone()
+            idx[s < tau] = 0
+            top2 = want[0].float().topk(2, dim=-1).values
+            clear = ((top2[:, 0] - top2[:, 1]) > 2 * ulp[0].max(dim=-1).values) & \
+                    ((top2[:, 0] - tau).abs() > 2 * ulp[0].max(dim=-1).values)
+            assert torch.equal(branch[0][clear].cpu(), idx.squeeze(-1)[clear].to(torch.int32).cpu())
+            strict += int(clear.sum())
+            total += H
+    assert strict > 0.5 * total
+
+
 def test_sliding_direct_raster_loads(monkeypatch):
     """Opt-in path (VB_ATTN_SLIDING_DIRECT=1): sliding heads fetch tile-major blocks straight from the raster tensors
     through a 5-D tensor map (one w-row box per TMA operation) instead of reading a tile-major copy.  Must give the

@@ -289,32 +289,18 @@ int vb_ulysses_pack_heads(const void* x, void* send, int32_t s_loc, int32_t head
 int vb_ulysses_pack_qkv(const void* q, const void* k, const void* v, const int64_t* stride_s, const int64_t* stride_h,
                         void* send, int32_t s_loc, int32_t heads, int32_t world, const int32_t* head_at,
                         vb_stream_t stream);
-/* Fused Ulysses "in" exchange over NVLink peer memory: rank `rank` stores the heads of slots [p*H/P, (p+1)*H/P) of its S_loc
- * tokens of q, k, v straight into peer p's receive buffer peer_qkv[p], laid out (3, rows_total, H/P, 128) with
- * this rank's tokens at rows [rank*S_loc, (rank+1)*S_loc).  Replaces pack + all-to-all (ulysses/utils.py:60-81). */
-int vb_ulysses_scatter_qkv(const void* q, const void* k, const void* v, const int64_t* stride_s,
-                           const int64_t* stride_h, void* const* peer_qkv, int64_t rows_total, int32_t s_loc,
-                           int32_t heads, int32_t world, int32_t rank, const int32_t* head_at, vb_stream_t stream);
 int vb_ulysses_unpack_heads(const void* recv, void* y, int32_t s_loc, int32_t heads, int32_t world,
                             const int32_t* head_at, vb_stream_t stream);
-/* The same exchange with an explicit placement: entry e sends head entry_head[e] of this rank's S_loc tokens of q, k, v
- * to slot entry_slot[e] of peer entry_peer[e], whose receive buffer is laid out (3, rows_total, slots, 128).  Ranks may
- * hold different numbers of heads, and a head may be sent to two peers (VB_BRANCH_FULL_LO / _HI units).  n_entries <= 128;
- * host pointers. */
+/* Fused Ulysses "in" exchange over NVLink peer memory, replacing pack + all-to-all (ulysses/utils.py:60-81): entry e
+ * stores head entry_head[e] of this rank's S_loc tokens of q, k, v straight into slot entry_slot[e] of peer
+ * entry_peer[e]'s receive buffer peer_qkv[entry_peer[e]], laid out (3, rows_total, slots, 128) with this rank's tokens
+ * at rows [rank*S_loc, (rank+1)*S_loc).  Ranks may hold different numbers of heads, and a head may be sent to two peers
+ * (VB_BRANCH_FULL_LO / _HI units).  n_entries <= 128; host pointers. */
 int vb_ulysses_scatter_qkv_slots(const void* q, const void* k, const void* v, const int64_t* stride_s,
                                  const int64_t* stride_h, void* const* peer_qkv, int64_t rows_total, int32_t s_loc,
                                  int32_t slots, int32_t world, int32_t rank, const int32_t* entry_peer,
                                  const int32_t* entry_slot, const int32_t* entry_head, int32_t n_entries,
                                  vb_stream_t stream);
-
-/* One or two of the three tensors only (tensor_mask: bit 0 = q, 1 = k, 2 = v; contiguous bits; unselected pointers may be
- * NULL) and an optional cap on the grid (max_ctas > 0): lets the host issue K's and V's stores on a side stream while the
- * next projection GEMM runs, instead of one exposed pass after all three projections. */
-int vb_ulysses_scatter_slots_partial(const void* q, const void* k, const void* v, const int64_t* stride_s,
-                                     const int64_t* stride_h, void* const* peer_qkv, int64_t rows_total, int32_t s_loc,
-                                     int32_t slots, int32_t world, int32_t rank, const int32_t* entry_peer,
-                                     const int32_t* entry_slot, const int32_t* entry_head, int32_t n_entries,
-                                     int32_t tensor_mask, int32_t max_ctas, vb_stream_t stream);
 
 #ifdef __cplusplus
 }

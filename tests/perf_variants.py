@@ -1,4 +1,7 @@
-"""Same workloads through several builds of the library (VB_LIB_PATH is read at import: one subprocess per build)."""
+"""Same workloads through several builds of the library (VB_LIB_PATH is read at import: one subprocess per build).
+The builds alternate per round, so each sees the same clocks and power state.  Rates are TFLOP/s, medians of 3 timings.
+
+    python tests/perf_variants.py NAME ...     # vorta_b200/lib/exp/libvb_NAME.so against the in-tree build"""
 import os
 import subprocess
 import sys
@@ -13,9 +16,17 @@ def timed(fn, iters=10):
     for _ in range(iters): fn()
     torch.cuda.synchronize(); ops.timing_enable(False)
     ms, n, fl = ops.timing_collect(); return ms / iters, fl / iters
+W14, W13 = (21, 45, 80), (21, 30, 52)
+CASES = (("dense16k", (1, 1, 16384), (1, 1, 16384), (1, 1, 2), 37, [0] * 37),
+         ("wan14 full H=8", W14, (3, 9, 16), (3, 3, 2), 8, [0] * 8),
+         ("wan14 coreset H=16", W14, (3, 9, 16), (3, 3, 2), 16, [1] * 16),
+         ("wan14 sliding H=16", W14, (3, 9, 16), (3, 3, 2), 16, [2] * 16),
+         ("wan14mix", W14, (3, 9, 16), (3, 3, 2), 40, [0] * 9 + [1] * 18 + [2] * 13),
+         ("wan14 native sliding (5,9,8) H=16", (20, 45, 80), (5, 9, 8), (2, 3, 2), 16, [2] * 16),
+         ("wan13 sliding H=12", W13, (3, 10, 4), (3, 3, 2), 12, [2] * 12),
+         ("wan13 mix 4f/4c/4s H=12", W13, (3, 10, 4), (3, 3, 2), 12, [0] * 4 + [1] * 4 + [2] * 4))
 out = []
-for name, lat, tile, lw, H, branch in (("dense16k", (1, 1, 16384), (1, 1, 16384), (1, 1, 2), 37, [0] * 37),
-                                       ("wan14mix", (21, 45, 80), (3, 9, 16), (3, 3, 2), 40, [0] * 9 + [1] * 18 + [2] * 13)):
+for name, lat, tile, lw, H, branch in CASES:
     plan = ops.Plan(lat, tile, (3, 3, 3) if lat[0] > 1 else (1, 1, 1), lw, 0.5)
     S = plan.seq_len
     q, k, v = (torch.randn((1, S, H, 128), device="cuda").bfloat16().transpose(1, 2) for _ in range(3))
@@ -24,6 +35,12 @@ for name, lat, tile, lw, H, branch in (("dense16k", (1, 1, 16384), (1, 1, 16384)
         ms, fl = timed(lambda: ops.routed_attention(plan, q, k, v, branch=branch))
         rates.append(fl / ms / 1e9)
     out.append("%%s %%.1f" %% (name, statistics.median(rates)))
+    del q, k, v, plan
+    torch.cuda.empty_cache()
+q = torch.randn((1, 75600, 40, 128), device="cuda").bfloat16().transpose(1, 2)
+k, v = (torch.randn((1, 512, 40, 128), device="cuda").bfloat16().transpose(1, 2) for _ in range(2))
+ms = statistics.median(timed(lambda: ops.attn_dense(q, k, v), iters=20)[0] for _ in range(3))
+out.append("wan14 cross attention 40 x 75600 x 512 %%.3f ms" %% ms)
 print(" | ".join(out))
 ''' % ROOT
 

@@ -824,26 +824,6 @@ def test_bf16_router_matches_golden_reference_router_in_bf16(golden):
     assert strict > 0.5 * total
 
 
-def test_sliding_direct_raster_loads(monkeypatch):
-    """Opt-in path (VB_ATTN_SLIDING_DIRECT=1): sliding heads fetch tile-major blocks straight from the raster tensors
-    through a 5-D tensor map (one w-row box per TMA operation) instead of reading a tile-major copy.  Must give the
-    same bits as the default path: same kernel order, same arithmetic, only the loads differ.  Tile widths 16, 8 and 4
-    (sub-atom boxes of SWIZZLE_128B) and a text tail (linear rows behind the grid rows)."""
-    for lat, tile, lw, tl, tv in (((6, 18, 32), (3, 9, 16), (3, 3, 2), 0, 0), ((6, 18, 16), (3, 9, 8), (3, 3, 2), 0, 0),
-                                  ((10, 12, 16), (5, 6, 4), (2, 3, 2), 0, 0), ((6, 12, 8), (3, 6, 4), (2, 3, 2), 40, 23)):
-        plan = ops.Plan(lat, tile, (3, 3, 3), lw, 0.5, text_len=tl, text_valid=tv)
-        S, H = plan.seq_len, 3
-        g = torch.Generator().manual_seed(S)
-        q, k, v = (torch.randn((1, S + tl, H, 128), generator=g).to(torch.bfloat16).to(dev()).transpose(1, 2)
-                   for _ in range(3))
-        monkeypatch.delenv("VB_ATTN_SLIDING_DIRECT", raising=False)
-        want = ops.routed_attention(plan, q, k, v, branch=[2, 0, 2])
-        monkeypatch.setenv("VB_ATTN_SLIDING_DIRECT", "1")
-        got = ops.routed_attention(plan, q, k, v, branch=[2, 0, 2])
-        monkeypatch.delenv("VB_ATTN_SLIDING_DIRECT", raising=False)
-        assert torch.equal(got, want)
-
-
 def test_query_half_units_equal_the_whole_head():
     """VB_BRANCH_FULL_LO / _HI (Ulysses units finer than a head): the two query halves of a full-attention head, run as
     separate head slots (as two ranks would), write disjoint rows whose union is bit-identical to the whole head;

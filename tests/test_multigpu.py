@@ -10,22 +10,20 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-@pytest.mark.parametrize("mode", ["peer", "peer-split", "peer-overlap", "nccl", "nccl-contiguous"])
+@pytest.mark.parametrize("mode", ["peer", "peer-split", "nccl", "nccl-contiguous"])
 @pytest.mark.parametrize("world", [2, 4, 8])
 def test_sequence_parallel_equals_single_gpu(world, mode):
     """mode "peer": exchange fused into the kernels over NVLink peer memory; "nccl": all-to-all collectives;
     "-contiguous": the reference's contiguous head chunks instead of the cost-balanced placement."""
     balance = "0" if mode.endswith("-contiguous") else "1"
     split = {"peer-split": "1"}.get(mode)          # force query-half units even at 2 ranks
-    overlap = {"peer-overlap": "1"}.get(mode)      # K / V stores on a side stream (opt-in path)
     mode = mode.split("-")[0]
     if torch.cuda.device_count() < world:
         pytest.skip(f"needs {world} GPUs")
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={world}",
-           "--master-addr", "127.0.0.1", "--master-port", str(29600 + world + (10 if mode == "nccl" else 0) + (20 if balance == "0" else 0) + (40 if split else 0) + (60 if overlap else 0)), os.path.join(ROOT, "tests", "mgpu_check.py")]
+           "--master-addr", "127.0.0.1", "--master-port", str(29600 + world + (10 if mode == "nccl" else 0) + (20 if balance == "0" else 0) + (40 if split else 0)), os.path.join(ROOT, "tests", "mgpu_check.py")]
     res = subprocess.run(cmd, capture_output=True, text=True, timeout=600, env=dict(os.environ, VB_ULYSSES=mode, VB_ULYSSES_BALANCE=balance,
-                                                                                   **({"VB_ULYSSES_SPLIT": split} if split else {}),
-                                                                                   **({"VB_ULYSSES_OVERLAP": overlap} if overlap else {})))
+                                                                                   **({"VB_ULYSSES_SPLIT": split} if split else {})))
     print(res.stdout[-3000:])
     assert res.returncode == 0, res.stdout[-3000:] + res.stderr[-3000:]
     assert "MISMATCH" not in res.stdout

@@ -40,8 +40,7 @@ EXPORTED_SYMBOLS = (
     "vb_block_ln_modulate", "vb_block_gate_residual", "vb_block_rmsnorm_rope", "vb_block_headnorm_rope",
     "vb_stats_reset", "vb_stats_launches", "vb_stats_attn_flops", "vb_timing_enable", "vb_timing_collect",
     "vb_timing_collect_kinds",
-    "vb_ulysses_pack_heads", "vb_ulysses_pack_qkv", "vb_ulysses_scatter_qkv", "vb_ulysses_unpack_heads",
-    "vb_ulysses_scatter_qkv_slots", "vb_ulysses_scatter_slots_partial",
+    "vb_ulysses_pack_heads", "vb_ulysses_pack_qkv", "vb_ulysses_unpack_heads", "vb_ulysses_scatter_qkv_slots",
 )
 
 
@@ -147,16 +146,9 @@ def _declare(lib: C.CDLL) -> None:
     lib.vb_ulysses_pack_heads.argtypes = [vp, vp, i32, i32, i32, i32, i64, i64, C.POINTER(i32), vp]
     lib.vb_ulysses_pack_qkv.restype = C.c_int
     lib.vb_ulysses_pack_qkv.argtypes = [vp, vp, vp, C.POINTER(i64), C.POINTER(i64), vp, i32, i32, i32, C.POINTER(i32), vp]
-    lib.vb_ulysses_scatter_qkv.restype = C.c_int
-    lib.vb_ulysses_scatter_qkv.argtypes = [vp, vp, vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(vp), i64, i32, i32, i32, i32,
-                                           C.POINTER(i32), vp]
     lib.vb_ulysses_scatter_qkv_slots.restype = C.c_int
     lib.vb_ulysses_scatter_qkv_slots.argtypes = [vp, vp, vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(vp), i64, i32, i32,
                                                  i32, i32, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), i32, vp]
-    lib.vb_ulysses_scatter_slots_partial.restype = C.c_int
-    lib.vb_ulysses_scatter_slots_partial.argtypes = [vp, vp, vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(vp), i64, i32,
-                                                     i32, i32, i32, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), i32,
-                                                     i32, i32, vp]
     lib.vb_ulysses_unpack_heads.restype = C.c_int
     lib.vb_ulysses_unpack_heads.argtypes = [vp, vp, i32, i32, i32, C.POINTER(i32), vp]
 

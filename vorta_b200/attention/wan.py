@@ -21,7 +21,7 @@ import torch
 from .. import _lib as L
 from .. import ops
 from ..ulysses import SP_STATE, balance, exchange_out, exchange_qkv, local_heads, shrink_dim
-from ..ulysses.peer import get_exchange, layer_placement, local_units, overlap_enabled
+from ..ulysses.peer import get_exchange, layer_placement, local_units
 from ._plans import get_plan, infer_lowres_window
 from .coreset_select import LowresGroupInfo
 
@@ -240,38 +240,6 @@ class WanAttnProcessorTripleEval(WanAttnProcessorTripleTrain):
         if branch is None:
             branch = _top1_branches(routing_score, tau_sparse)
         plan = self._plan(lowres_group_info, flex_attn_mask_func, window_size, tile_size, latent_shape)
-        if SP_STATE.enabled and hidden_states.shape[0] == 1 and overlap_enabled():
-            ex = get_exchange(attn.heads, hidden_states.shape[1], hidden_states.device)
-            if ex is not None:
-                return self._output_proj(attn, self._overlapped(attn, hidden_states, rotary_emb, plan, branch, ex), None)
         query, key, value, _ = self._input_proj(attn, hidden_states, encoder_hidden_states=None, rotary_emb=rotary_emb)
         hidden_states = self._routed_attention(query, key, value, plan, branch=branch)
         return self._output_proj(attn, hidden_states, hidden_states_img=None)
-
-    def _overlapped(self, attn, hidden_states, rotary_emb, plan, branch, ex) -> torch.Tensor:
-        """``_input_proj`` + exchange + attention with the NVLink stores of K and V overlapped with the projection that
-        follows them: K is projected (and normalised / rotated) first and leaves on a side stream while the V GEMM
-        runs, V leaves while the Q GEMM runs, only Q's stores are exposed.  Same data, same kernels: results are
-        bit-identical to the sequential order."""
-        heads = attn.heads
-        P, r = SP_STATE.sp_size, SP_STATE.group_local_rank
-        cos = sin = None
-        if rotary_emb is not None:
-            cos, sin = _rope_tables(shrink_dim(rotary_emb, dim=2))
-
-        def as_heads(t):
-            return t.unflatten(2, (heads, -1)).transpose(1, 2)
-
-        placement = layer_placement(branch, plan, heads, P, ex.slots)
-        ex.overlap_begin(placement)
-        key = as_heads(_norm_rope(attn.norm_k, attn.to_k(hidden_states), cos, sin))
-        ex.overlap_send(1, key, side=True)
-        value = as_heads(attn.to_v(hidden_states))
-        ex.overlap_send(2, value, side=True)
-        query = as_heads(_norm_rope(attn.norm_q, attn.to_q(hidden_states), cos, sin))
-        ex.overlap_send(0, query, side=False)
-        q, k, v = ex.overlap_end(hidden_states.device)
-        ids, out_heads = local_units(placement, r, branch, ex.slots)
-        ops.routed_attention(plan, q, k, v, branch=ids, out_peers=ex.out_ptrs, out_peer_rows=ex.s_loc,
-                             out_peer_strides=(0, 128, heads * 128), out_heads=out_heads)
-        return ex.finish_out()

@@ -67,18 +67,12 @@ int launch_rmsnorm_rope(const void* x, const void* weight, const float* cs, cons
 int launch_headnorm_rope(const void* x, const void* weight, const float* cs, const float* sn, void* out, int batch,
                          int rows, int heads, int rope_rows, int dst_rows, int dst_row0, float eps,
                          cudaStream_t stream);
-int launch_ulysses_scatter_qkv(const void* q, const void* k, const void* v, const int64_t* stride_s,
-                               const int64_t* stride_h, void* const* peer_qkv, int64_t rows_total, int s_loc, int heads,
-                               int world, int rank, const int32_t* head_at, cudaStream_t stream);
 int launch_ulysses_scatter_slots(const void* q, const void* k, const void* v, const int64_t* stride_s,
                                  const int64_t* stride_h, void* const* peer_qkv, int64_t rows_total, int s_loc, int slots,
                                  int world, int rank, const int32_t* entry_peer, const int32_t* entry_slot,
-                                 const int32_t* entry_head, int n_entries, int tensor_mask, int max_ctas,
-                                 cudaStream_t stream);
+                                 const int32_t* entry_head, int n_entries, cudaStream_t stream);
 int make_qkv_tensor_map(CUtensorMap* map, const void* base, int64_t n_rows, int64_t heads, int64_t batch,
                         int64_t stride_b, int64_t stride_h, int64_t stride_s);
-int make_grid_tensor_map(CUtensorMap* map, const void* base, const int32_t* latent, int32_t tile_w, int64_t heads,
-                         int64_t stride_h, int64_t stride_s);
 int launch_attn(const AttnTmaps& tmaps, const AttnParams& params, int n_ctas, cudaStream_t stream);
 
 
@@ -123,7 +117,7 @@ struct Schedule {
   void finalize() {
     bool all_single = !pairs.empty();
     for (const QPair& qp : pairs) all_single = all_single && qp.nq == 1;
-    if (all_single && getenv("VB_ATTN_NO_SPLIT") == nullptr) {
+    if (all_single) {
       std::vector<QPair> out;
       std::vector<int> open_by_blocks;        // index in `out` of an unpaired single-tile item, per block count
       for (const QPair& qp : pairs) {
@@ -207,7 +201,6 @@ struct vb_plan {
   std::vector<WindowGroup> groups;
   std::vector<int32_t> query_map;             // (S + text_len): sliding-branch query position -> raster token
   Schedule full, coreset, sliding;            // sliding: queries in window-group order
-  Schedule sliding_tiles;                     // one range per tile, queries in tile-major order (raster-load path)
   // device tables
   int32_t* d_center_tok = nullptr;
   int32_t* d_margin_tok = nullptr;
@@ -238,18 +231,17 @@ static int build_text_dependent(vb_plan* pl) {
   pl->coreset.runs.push_back({0, pl->S_c + tv});
   pl->coreset.add_query_range(0, pl->S_c + tv, 0, 1, pl->S_c + tv);
   // ---- sliding tile (sliding_attn_flex.py:93-127): keys in tile-major order; one query range per window group
-  //      (sliding) and one per tile (sliding_tiles)
   pl->sliding.clear();
-  pl->sliding_tiles.clear();
   const int tau = pl->tile_tokens;
-  auto add_window = [&](Schedule& sc, const int* lo, const int* hi, int row0, int n_rows) -> int {
+  Schedule& sc = pl->sliding;
+  for (const vb_plan::WindowGroup& g : pl->groups) {
     const int run_begin = static_cast<int>(sc.runs.size());
     int64_t keys = 0;
-    for (int x = lo[0]; x <= hi[0]; ++x)
-      for (int y = lo[1]; y <= hi[1]; ++y) {
+    for (int x = g.lo[0]; x <= g.hi[0]; ++x)
+      for (int y = g.lo[1]; y <= g.hi[1]; ++y) {
         KvRun r;
-        r.start = ((x * pl->nt[1] + y) * pl->nt[2] + lo[2]) * tau;
-        r.len = (hi[2] - lo[2] + 1) * tau;
+        r.start = ((x * pl->nt[1] + y) * pl->nt[2] + g.lo[2]) * tau;
+        r.len = (g.hi[2] - g.lo[2] + 1) * tau;
         keys += r.len;
         if (static_cast<int>(sc.runs.size()) > run_begin && sc.runs.back().start + sc.runs.back().len == r.start) {
           sc.runs.back().len += r.len;   // contiguous in tile-major order: merge
@@ -263,38 +255,24 @@ static int build_text_dependent(vb_plan* pl) {
     }
     const int run_count = static_cast<int>(sc.runs.size()) - run_begin;
     VB_REQUIRE(run_count <= 32, VB_ERR_UNSUPPORTED, "sliding window needs %d key runs per tile (max 32)", run_count);
-    sc.add_query_range(row0, n_rows, run_begin, run_count, keys);
-    if (row0 == 0) pl->keys_per_query = keys - tv;
-    return VB_OK;
-  };
-  for (const vb_plan::WindowGroup& g : pl->groups) {
-    const int rc = add_window(pl->sliding, g.lo, g.hi, g.row0, g.n_tiles * tau);
-    if (rc != VB_OK) return rc;
+    sc.add_query_range(g.row0, g.n_tiles * tau, run_begin, run_count, keys);
+    if (g.row0 == 0) pl->keys_per_query = keys - tv;
   }
-  for (int tile_id = 0; tile_id < pl->n_tiles; ++tile_id) {
-    const int32_t* w = &pl->tile_window[static_cast<size_t>(tile_id) * 6];
-    const int rc = add_window(pl->sliding_tiles, w, w + 3, tile_id * tau, tau);
-    if (rc != VB_OK) return rc;
-  }
-  if (tv > 0) {   // valid text queries see every non-pad key (:108); two runs, so that no 128-key block straddles the
-                  // video / text boundary (video rows come through the raster-grid tensor map, text rows through the linear one)
-    for (Schedule* sc : {&pl->sliding, &pl->sliding_tiles}) {
-      const int run_begin = static_cast<int>(sc->runs.size());
-      sc->runs.push_back({0, S});
-      sc->runs.push_back({S, tv});
-      sc->add_query_range(S, tv, run_begin, 2, S + tv);
-    }
+  if (tv > 0) {   // valid text queries see every non-pad key (:108) as two runs, video and text: one run [0, S + tv)
+                  // would cut the keys into different 128-key blocks and so change these rows' output bits
+    const int run_begin = static_cast<int>(sc.runs.size());
+    sc.runs.push_back({0, S});
+    sc.runs.push_back({S, tv});
+    sc.add_query_range(S, tv, run_begin, 2, S + tv);
   }
   pl->full.finalize();
   pl->coreset.finalize();
   pl->sliding.finalize();
-  pl->sliding_tiles.finalize();
   if (pl->has_device) {
     int rc;
     if ((rc = pl->full.upload()) != VB_OK) return rc;
     if ((rc = pl->coreset.upload()) != VB_OK) return rc;
     if ((rc = pl->sliding.upload()) != VB_OK) return rc;
-    if ((rc = pl->sliding_tiles.upload()) != VB_OK) return rc;
   }
   return VB_OK;
 }
@@ -302,7 +280,7 @@ static int build_text_dependent(vb_plan* pl) {
 extern "C" {
 
 const char* vb_last_error(void) { return get_error(); }
-int vb_version(void) { return 100; }
+int vb_version(void) { return 101; }
 
 int vb_device_check(void) {
   int dev = 0, major = 0, minor = 0, count = 0;
@@ -412,7 +390,6 @@ int vb_plan_create(vb_plan** out, const vb_plan_desc* desc) {
   {
     std::vector<std::vector<int>> members;
     std::map<std::array<int, 6>, int> index_of;             // window -> group
-    const bool group_windows = getenv("VB_ATTN_NO_WINDOW_GROUPS") == nullptr;     // A/B switch: one group per tile
     for (int a = 0; a < pl->nt[0]; ++a)
       for (int b = 0; b < pl->nt[1]; ++b)
         for (int c = 0; c < pl->nt[2]; ++c) {
@@ -423,7 +400,7 @@ int vb_plan_create(vb_plan** out, const vb_plan_desc* desc) {
           window_range(b, pl->nt[1], d.window[1], lo, hi); w[1] = lo; w[4] = hi;
           window_range(c, pl->nt[2], d.window[2], lo, hi); w[2] = lo; w[5] = hi;
           const std::array<int, 6> key = {w[0], w[1], w[2], w[3], w[4], w[5]};
-          auto hit = group_windows ? index_of.find(key) : index_of.end();
+          auto hit = index_of.find(key);
           int found;
           if (hit != index_of.end()) {
             found = hit->second;
@@ -434,7 +411,7 @@ int vb_plan_create(vb_plan** out, const vb_plan_desc* desc) {
             found = static_cast<int>(pl->groups.size());
             pl->groups.push_back(g);
             members.emplace_back();
-            if (group_windows) index_of.emplace(key, found);
+            index_of.emplace(key, found);
           }
           members[found].push_back(tile_id);
         }
@@ -483,7 +460,6 @@ void vb_plan_destroy(vb_plan* pl) {
   pl->full.release();
   pl->coreset.release();
   pl->sliding.release();
-  pl->sliding_tiles.release();
   if (pl->d_query_map) cudaFree(pl->d_query_map);
   if (pl->d_center_tok) cudaFree(pl->d_center_tok);
   if (pl->d_margin_tok) cudaFree(pl->d_margin_tok);
@@ -645,7 +621,6 @@ struct BranchLaunch {
   const int32_t* bcast_map;
   int64_t bcast_stride_b, bcast_stride_h;
   int32_t bcast_rows, bcast_n;
-  const vb_plan* grid_plan;      // non-null: q, k, v are the caller's raster tensors, rows are tile-major (AttnSeg::grid_rows)
 };
 }  // namespace
 
@@ -697,20 +672,6 @@ static int launch_segments(const Segment* const* segs, int n_seg, const vb_attn_
     s.out_map = bl.out_map; s.out_map_stride_b = bl.out_map_stride_b; s.out_map_stride_h = bl.out_map_stride_h;
     s.bcast_map = bl.bcast_map; s.bcast_stride_b = bl.bcast_stride_b; s.bcast_stride_h = bl.bcast_stride_h;
     s.bcast_rows = bl.bcast_rows; s.bcast_n = bl.bcast_n;
-    if (bl.grid_plan != nullptr) {
-      const vb_plan* gp = bl.grid_plan;
-      const void* base[3] = {bl.q, bl.k, bl.v};
-      const int64_t* st[3] = {bl.qs, bl.ks, bl.vs};
-      for (int t = 0; t < 3; ++t)
-        if ((rc = make_grid_tensor_map(&tm.grid[t], base[t], gp->d.latent, gp->d.tile[2], bl.n_heads_tensor, st[t][1],
-                                       st[t][2])))
-          return rc;
-      s.grid_rows = gp->S;
-      for (int d = 0; d < 3; ++d) {
-        s.tile[d] = gp->d.tile[d];
-        s.ntile[d] = gp->nt[d];
-      }
-    }
     s.n_pairs = static_cast<int32_t>(bl.sched->pairs.size());
     double seg_flops = bl.sched->flops_per_head;
     if (sg.pair_count > 0) {      // a query sub-range of the schedule: its share of the head's FLOPs goes by query rows
@@ -751,10 +712,6 @@ static int launch_segments(const Segment* const* segs, int n_seg, const vb_attn_
   }
   p.batch0 = batch0;
   p.dbg = a.debug;
-  if (a.debug != nullptr) {   // bring-up only: descriptor stride overrides for the V operand
-    if (const char* e = getenv("VB_DBG_V_LBO")) p.dbg_v_lbo = static_cast<uint32_t>(atoi(e));
-    if (const char* e = getenv("VB_DBG_V_SBO")) p.dbg_v_sbo = static_cast<uint32_t>(atoi(e));
-  }
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   if (g_timing) {
     VB_CUDA_OK(cudaEventCreate(&ev0));
@@ -883,7 +840,7 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
   // longest-CTA-first (full: S/128 key blocks per CTA, coreset: ~S/256, sliding: <= 27 tiles)
   Segment deferred[kMaxSegments];
   int n_deferred = 0;
-  const bool merge = !blend && a.heads <= kMaxHeads && getenv("VB_ATTN_SPLIT_LAUNCHES") == nullptr;
+  const bool merge = !blend && a.heads <= kMaxHeads;
   VB_REQUIRE(!blend || parts.empty(), VB_ERR_INVALID, "query-part ids need top-1 mode");
   auto for_batches = [&](const BranchLaunch& bl, const std::vector<int32_t>& hs, int e, bool slot_is_index,
                          int pair_begin = 0, int pair_count = 0) -> int {
@@ -1010,65 +967,39 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
   if (!by_branch[2].empty()) {
     const std::vector<int32_t>& hs = by_branch[2];
     const int nh = static_cast<int>(hs.size());
-    // Direct path (opt-in, VB_ATTN_SLIDING_DIRECT=1): the kernel fetches tile-major blocks from the caller's raster
-    // tensors through a 5-D tensor map, one w-row box per TMA operation, so no tile-major copy is written.  Correct
-    // (tests/test_gpu_parity.py::test_sliding_direct_raster_loads) but NOT the default: a 128-row block becomes
-    // 2 * 128 / tile_w boxes of tile_w x 128 B, and the TMA unit is bound by the box count, not the bytes — Wan-14B
-    // (tile_w 16, 16 boxes of 2 KB per block) 753 vs 1127 TFLOP/s with the layout pass (1050 including it), Wan-1.3B
-    // (tile_w 4, 64 boxes of 512 B) 182 vs 655 (profiles/r2e_perf_*.log).  The same measurement rules out
-    // tile::gather4 row gathers for the coreset branch (64 operations of 512 B per block; the instruction itself works,
-    // tests/micro/gather4_probe.cu).  The layout pass costs ~0.5 % of a Wan-14B step.
-    const int tw = pl->d.tile[2];
-    const char* direct_env = getenv("VB_ATTN_SLIDING_DIRECT");
-    const bool direct = direct_env != nullptr && direct_env[0] == '1' && a.batch == 1 && kBlockN % tw == 0 && tw >= 4;
-    if (direct) {
-      NvtxRange nvtx("vb: sliding tile (raster loads, no layout pass)");
-      BranchLaunch bl;
-      memset(&bl, 0, sizeof(bl));
-      bl.q = static_cast<const __nv_bfloat16*>(a.q);
-      bl.k = static_cast<const __nv_bfloat16*>(a.k);
-      bl.v = static_cast<const __nv_bfloat16*>(a.v);
-      for (int i = 0; i < 3; ++i) { bl.qs[i] = a.q_stride[i]; bl.ks[i] = a.k_stride[i]; bl.vs[i] = a.v_stride[i]; }
-      bl.n_rows_q = S + TV; bl.n_rows_kv = S + TV; bl.n_heads_tensor = a.heads;   // linear maps: text rows keep their place
-      bl.sched = &pl->sliding_tiles;
-      bl.out_map = pl->d_tile_map; bl.out_map_stride_b = 0; bl.out_map_stride_h = 0;
-      bl.grid_plan = pl;
-      if ((rc = for_batches(bl, hs, 2, false)) != VB_OK) return rc;
-    } else {
-      // layout pass: K and V in tile-major order, Q in window-group order (vb_plan::groups); the epilogue scatters
-      // the output rows back to raster order through the same query map
-      NvtxRange nvtx("vb: sliding tile-major layout");
-      const int64_t rows = N;
-      const int64_t bh = static_cast<int64_t>(a.batch) * nh;
-      __nv_bfloat16* tq = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
-      __nv_bfloat16* tk = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
-      __nv_bfloat16* tv = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
-      HeadList heads_s;
-      if ((rc = head_list_of(hs, &heads_s)) != VB_OK) return rc;
-      VB_REQUIRE(tq && tk && tv, VB_ERR_INVALID, "workspace exhausted");
-      GatherParams gp;
-      memset(&gp, 0, sizeof(gp));
-      gp.n_tensors = 3; gp.map = pl->d_tile_map; gp.map0 = pl->d_query_map; gp.map_stride_b = 0; gp.map_stride_h = 0;
-      gp.src[0] = static_cast<const __nv_bfloat16*>(a.q); gp.dst[0] = tq;
-      gp.src[1] = static_cast<const __nv_bfloat16*>(a.k); gp.dst[1] = tk;
-      gp.src[2] = static_cast<const __nv_bfloat16*>(a.v); gp.dst[2] = tv;
-      for (int i = 0; i < 3; ++i) {
-        gp.src_stride[0][i] = a.q_stride[i]; gp.src_stride[1][i] = a.k_stride[i]; gp.src_stride[2][i] = a.v_stride[i];
-      }
-      gp.dst_stride[0] = nh * rows * kHeadDim; gp.dst_stride[1] = rows * kHeadDim; gp.dst_stride[2] = kHeadDim;
-      gp.head_list = heads_s; gp.batch = a.batch; gp.heads = nh; gp.n_rows = static_cast<int32_t>(rows);
-      if ((rc = launch_gather_rows(gp, stream)) != VB_OK) return rc;
-      ++g_launches;
-      BranchLaunch bl;
-      memset(&bl, 0, sizeof(bl));
-      bl.q = tq; bl.k = tk; bl.v = tv;
-      const int64_t st[3] = {nh * rows * kHeadDim, rows * kHeadDim, kHeadDim};
-      for (int i = 0; i < 3; ++i) { bl.qs[i] = st[i]; bl.ks[i] = st[i]; bl.vs[i] = st[i]; }
-      bl.n_rows_q = S + TV; bl.n_rows_kv = S + TV; bl.n_heads_tensor = nh;
-      bl.sched = &pl->sliding;
-      bl.out_map = pl->d_query_map; bl.out_map_stride_b = 0; bl.out_map_stride_h = 0;
-      if ((rc = for_batches(bl, hs, 2, true)) != VB_OK) return rc;
+    // layout pass: K and V in tile-major order, Q in window-group order (vb_plan::groups); the epilogue scatters the
+    // output rows back to raster order through the same query map
+    NvtxRange nvtx("vb: sliding tile-major layout");
+    const int64_t rows = N;
+    const int64_t bh = static_cast<int64_t>(a.batch) * nh;
+    __nv_bfloat16* tq = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
+    __nv_bfloat16* tk = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
+    __nv_bfloat16* tv = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
+    HeadList heads_s;
+    if ((rc = head_list_of(hs, &heads_s)) != VB_OK) return rc;
+    VB_REQUIRE(tq && tk && tv, VB_ERR_INVALID, "workspace exhausted");
+    GatherParams gp;
+    memset(&gp, 0, sizeof(gp));
+    gp.n_tensors = 3; gp.map = pl->d_tile_map; gp.map0 = pl->d_query_map; gp.map_stride_b = 0; gp.map_stride_h = 0;
+    gp.src[0] = static_cast<const __nv_bfloat16*>(a.q); gp.dst[0] = tq;
+    gp.src[1] = static_cast<const __nv_bfloat16*>(a.k); gp.dst[1] = tk;
+    gp.src[2] = static_cast<const __nv_bfloat16*>(a.v); gp.dst[2] = tv;
+    for (int i = 0; i < 3; ++i) {
+      gp.src_stride[0][i] = a.q_stride[i]; gp.src_stride[1][i] = a.k_stride[i]; gp.src_stride[2][i] = a.v_stride[i];
     }
+    gp.dst_stride[0] = nh * rows * kHeadDim; gp.dst_stride[1] = rows * kHeadDim; gp.dst_stride[2] = kHeadDim;
+    gp.head_list = heads_s; gp.batch = a.batch; gp.heads = nh; gp.n_rows = static_cast<int32_t>(rows);
+    if ((rc = launch_gather_rows(gp, stream)) != VB_OK) return rc;
+    ++g_launches;
+    BranchLaunch bl;
+    memset(&bl, 0, sizeof(bl));
+    bl.q = tq; bl.k = tk; bl.v = tv;
+    const int64_t st[3] = {nh * rows * kHeadDim, rows * kHeadDim, kHeadDim};
+    for (int i = 0; i < 3; ++i) { bl.qs[i] = st[i]; bl.ks[i] = st[i]; bl.vs[i] = st[i]; }
+    bl.n_rows_q = S + TV; bl.n_rows_kv = S + TV; bl.n_heads_tensor = nh;
+    bl.sched = &pl->sliding;
+    bl.out_map = pl->d_query_map; bl.out_map_stride_b = 0; bl.out_map_stride_h = 0;
+    if ((rc = for_batches(bl, hs, 2, true)) != VB_OK) return rc;
   }
 
   if (n_deferred > 0) {
@@ -1236,15 +1167,6 @@ int vb_ulysses_pack_qkv(const void* q, const void* k, const void* v, const int64
   if (rc == VB_OK) ++g_launches;
   return rc;
 }
-int vb_ulysses_scatter_qkv(const void* q, const void* k, const void* v, const int64_t* stride_s,
-                           const int64_t* stride_h, void* const* peer_qkv, int64_t rows_total, int32_t s_loc,
-                           int32_t heads, int32_t world, int32_t rank, const int32_t* head_at, vb_stream_t stream) {
-  VB_REQUIRE(q && k && v && stride_s && stride_h && peer_qkv, VB_ERR_INVALID, "null argument");
-  int rc = launch_ulysses_scatter_qkv(q, k, v, stride_s, stride_h, peer_qkv, rows_total, s_loc, heads, world, rank,
-                                      head_at, static_cast<cudaStream_t>(stream));
-  if (rc == VB_OK) ++g_launches;
-  return rc;
-}
 int vb_ulysses_scatter_qkv_slots(const void* q, const void* k, const void* v, const int64_t* stride_s,
                                  const int64_t* stride_h, void* const* peer_qkv, int64_t rows_total, int32_t s_loc,
                                  int32_t slots, int32_t world, int32_t rank, const int32_t* entry_peer,
@@ -1253,20 +1175,7 @@ int vb_ulysses_scatter_qkv_slots(const void* q, const void* k, const void* v, co
   VB_REQUIRE(q && k && v && stride_s && stride_h && peer_qkv && entry_peer && entry_slot && entry_head, VB_ERR_INVALID,
              "null argument");
   int rc = launch_ulysses_scatter_slots(q, k, v, stride_s, stride_h, peer_qkv, rows_total, s_loc, slots, world, rank,
-                                        entry_peer, entry_slot, entry_head, n_entries, 7, 0,
-                                        static_cast<cudaStream_t>(stream));
-  if (rc == VB_OK) ++g_launches;
-  return rc;
-}
-int vb_ulysses_scatter_slots_partial(const void* q, const void* k, const void* v, const int64_t* stride_s,
-                                     const int64_t* stride_h, void* const* peer_qkv, int64_t rows_total, int32_t s_loc,
-                                     int32_t slots, int32_t world, int32_t rank, const int32_t* entry_peer,
-                                     const int32_t* entry_slot, const int32_t* entry_head, int32_t n_entries,
-                                     int32_t tensor_mask, int32_t max_ctas, vb_stream_t stream) {
-  VB_REQUIRE(stride_s && stride_h && peer_qkv && entry_peer && entry_slot && entry_head, VB_ERR_INVALID, "null argument");
-  int rc = launch_ulysses_scatter_slots(q, k, v, stride_s, stride_h, peer_qkv, rows_total, s_loc, slots, world, rank,
-                                        entry_peer, entry_slot, entry_head, n_entries, tensor_mask, max_ctas,
-                                        static_cast<cudaStream_t>(stream));
+                                        entry_peer, entry_slot, entry_head, n_entries, static_cast<cudaStream_t>(stream));
   if (rc == VB_OK) ++g_launches;
   return rc;
 }

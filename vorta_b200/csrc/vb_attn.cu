@@ -23,9 +23,6 @@
 // softmax warps find S(j+1) complete when they finish block j and do not wait in steady state.  (With P aliased on S
 // and one S per tile the chain softmax -> PV -> QK was serial per tile: 1600 + 300 + 1024 cycles per block, tensor pipe
 // 61 % busy; profiles/r1g_timeline_dense16k.log vs r1l_timeline_decoupled.log.)
-#include <stdlib.h>
-#include <string.h>
-
 #include <algorithm>
 
 #include "vb_common.cuh"
@@ -206,11 +203,6 @@ vb_attn_fwd_kernel(const __grid_constant__ AttnTmaps tmaps, const __grid_constan
       tma_prefetch_desc(&tmaps.m[i][0]);
       tma_prefetch_desc(&tmaps.m[i][1]);
       tma_prefetch_desc(&tmaps.m[i][2]);
-      if (p.seg[i].grid_rows > 0) {
-        tma_prefetch_desc(&tmaps.grid[0]);
-        tma_prefetch_desc(&tmaps.grid[1]);
-        tma_prefetch_desc(&tmaps.grid[2]);
-      }
     }
   }
   if (warp == kMmaWarp) {
@@ -232,8 +224,7 @@ vb_attn_fwd_kernel(const __grid_constant__ AttnTmaps tmaps, const __grid_constan
 
   if (warp == kTmaWarp) {
     // ======================================= TMA producer =======================================
-    // The whole warp runs the loop converged (one lane would do for linear rows; the raster path below issues one box
-    // per lane).  Lane 0 owns the work counter, every expect_tx arrive and the linear loads.
+    // The whole warp runs the loop converged; lane 0 owns the work counter, every expect_tx arrive and every load.
     uint32_t load_idx = 0;                 // position in the K/V ring, running through all items
     uint32_t q_uses[2] = {0, 0};           // items that used Q_t so far
     for (uint32_t n = 0;; ++n) {
@@ -258,41 +249,25 @@ vb_attn_fwd_kernel(const __grid_constant__ AttnTmaps tmaps, const __grid_constan
       const CUtensorMap* tmap_v = &tmaps.m[it.seg_idx][2];
       const int nq = it.pair.nq, hk = it.head.hk, batch = it.batch;
       // 128 rows [row0, row0 + 128) of one operand -> dst (two 64-channel halves of 16 KB), completion on bar
-      auto load_rows = [&](const CUtensorMap* lin, int which, int row0, uint8_t* dst, uint64_t* bar) {
-        if (lane == 0) mbar_arrive_expect_tx(bar, kTileBytes);
-        __syncwarp();
-        if (seg.grid_rows > 0 && row0 < seg.grid_rows) {
-          // tile-major rows of the raster grid: one (64 channels x tile_w tokens) box per w-row and channel half;
-          // rows behind the last tile have t >= T and are zero-filled by the TMA unit (the bytes still count)
-          const CUtensorMap* gm = &tmaps.grid[which];
-          const int tw = seg.tile[2], thw = seg.tile[1] * tw, tau = seg.tile[0] * thw;
-          const int n12 = seg.ntile[1] * seg.ntile[2];
-          for (int i = lane; i < 2 * (kBlockN / tw); i += 32) {
-            const int box = i >> 1, half = i & 1;
-            const int r = row0 + box * tw;
-            const int tile = r / tau, intra = r - tile * tau;
-            const int it_ = intra / thw, rem = intra - it_ * thw, ih = rem / tw, iw = rem - ih * tw;
-            const int ta = tile / n12, tr = tile - ta * n12, tb_ = tr / seg.ntile[2], tc = tr - tb_ * seg.ntile[2];
-            tma_load_5d(dst + half * kHalfBytes + box * tw * 128, gm, bar, half * 64, tc * tw + iw,
-                        tb_ * seg.tile[1] + ih, ta * seg.tile[0] + it_, hk);
-          }
-        } else if (lane == 0) {
-          tma_load_4d(dst, lin, bar, 0, row0, hk, batch);
-          tma_load_4d(dst + kHalfBytes, lin, bar, 64, row0, hk, batch);
+      auto load_rows = [&](const CUtensorMap* m, int row0, uint8_t* dst, uint64_t* bar) {
+        if (lane == 0) {
+          mbar_arrive_expect_tx(bar, kTileBytes);
+          tma_load_4d(dst, m, bar, 0, row0, hk, batch);
+          tma_load_4d(dst + kHalfBytes, m, bar, 64, row0, hk, batch);
         }
       };
-      auto load_kv = [&](const CUtensorMap* m, int which, int row0) {
+      auto load_kv = [&](const CUtensorMap* m, int row0) {
         const uint32_t slot = load_idx % kNumSlots;
         const uint32_t phase = (load_idx / kNumSlots) & 1u;
         mbar_wait(&bar_slot_empty[slot], phase ^ 1u);
-        load_rows(m, which, row0, smem_kv + slot * kTileBytes, &bar_slot_full[slot]);
+        load_rows(m, row0, smem_kv + slot * kTileBytes, &bar_slot_full[slot]);
         ++load_idx;
       };
       auto load_q = [&]() {
         for (int t = 0; t < nq; ++t) {
           if (q_uses[t] > 0) mbar_wait(&sm.bar_q_empty[t], (q_uses[t] - 1) & 1u);
           ++q_uses[t];
-          load_rows(tmap_q, 0, it.pair.q_row0[t], smem_q + t * kTileBytes, &bar_q_full[t]);
+          load_rows(tmap_q, it.pair.q_row0[t], smem_q + t * kTileBytes, &bar_q_full[t]);
         }
       };
       BlockWalker w0(seg.runs + it.pair.run_begin, it.pair.run_count);
@@ -300,12 +275,12 @@ vb_attn_fwd_kernel(const __grid_constant__ AttnTmaps tmaps, const __grid_constan
       int row0, valid;
       // the first K block does not depend on the previous item having released Q: request it first
       for (int j = 0; w0.next(row0, valid); ++j) {
-        load_kv(tmap_k, 1, row0);
+        load_kv(tmap_k, row0);
         if (j == 0) load_q();
-        load_kv(tmap_v, 2, row0);
+        load_kv(tmap_v, row0);
         if (it.pair.split && w1.next(row0, valid)) {      // K1 V1 of the same block step
-          load_kv(tmap_k, 1, row0);
-          load_kv(tmap_v, 2, row0);
+          load_kv(tmap_k, row0);
+          load_kv(tmap_v, row0);
         }
       }
     }
@@ -717,31 +692,8 @@ int make_qkv_tensor_map(CUtensorMap* map, const void* base, int64_t n_rows, int6
   return VB_OK;
 }
 
-// 5-D bf16 tensor map over the raster token grid of ONE batch element: (channel = 128, W, H, T, head) with a
-// (64, tile_w, 1, 1, 1) box, SWIZZLE_128B; token (t, h, w) sits at ((t * H + h) * W + w) * stride_s.
-int make_grid_tensor_map(CUtensorMap* map, const void* base, const int32_t* latent, int32_t tile_w, int64_t heads,
-                         int64_t stride_h, int64_t stride_s) {
-  PFN_encodeTiled enc = get_encode_fn();
-  VB_REQUIRE(enc != nullptr, VB_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
-  VB_REQUIRE((reinterpret_cast<uintptr_t>(base) & 15) == 0 && stride_s % 8 == 0 && stride_h % 8 == 0, VB_ERR_INVALID,
-             "tensor base and strides must be 16-byte aligned");
-  const int64_t T = latent[0], H = latent[1], W = latent[2];
-  cuuint64_t dims[5] = {static_cast<cuuint64_t>(kHeadDim), static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H),
-                        static_cast<cuuint64_t>(T), static_cast<cuuint64_t>(heads)};
-  auto fix = [](int64_t s) { return static_cast<cuuint64_t>((s > 0 ? s : 8) * 2); };
-  cuuint64_t strides[4] = {fix(stride_s), fix(W * stride_s), fix(H * W * stride_s), fix(stride_h)};
-  cuuint32_t box[5] = {64, static_cast<cuuint32_t>(tile_w), 1, 1, 1};
-  cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  VB_REQUIRE(r == CUDA_SUCCESS, VB_ERR_CUDA, "cuTensorMapEncodeTiled (5-D grid) failed with CUresult %d", (int)r);
-  return VB_OK;
-}
-
 // `params.seg[i].cta_begin` must already hold the prefix sums; n_items = total work items over the segments.  The grid
-// is one persistent CTA per SM (224 KB of shared memory: one CTA fits); VB_ATTN_GRID=items launches one CTA per item
-// instead (the round-1 schedule, kept for A/B measurements).
+// is one persistent CTA per SM (224 KB of shared memory: one CTA fits).
 int launch_attn(const AttnTmaps& tmaps, const AttnParams& params_in, int n_items, cudaStream_t stream) {
   static bool configured[64] = {false};      // the attribute is per device
   static int sm_count[64] = {0};
@@ -764,9 +716,7 @@ int launch_attn(const AttnTmaps& tmaps, const AttnParams& params_in, int n_items
   if (n_items == 0) return VB_OK;
   AttnParams params = params_in;
   params.work_counter = counters[dev] + (next_counter[dev]++ % kCounters);
-  const char* grid_env = getenv("VB_ATTN_GRID");       // read per launch: perf scripts flip it between launches
-  const bool per_item = grid_env != nullptr && strcmp(grid_env, "items") == 0;
-  const int n_ctas = per_item ? n_items : std::min(n_items, sm_count[dev]);
+  const int n_ctas = std::min(n_items, sm_count[dev]);
   vb_attn_fwd_kernel<<<static_cast<unsigned>(n_ctas), kAttnThreads, kAttnSmemBytes, stream>>>(tmaps, params);
   VB_CUDA_OK(cudaGetLastError());
   return VB_OK;

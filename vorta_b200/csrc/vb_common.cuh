@@ -83,13 +83,6 @@ struct AttnSeg {
   int32_t n_pairs, n_heads;     // CTAs of the segment = n_pairs * n_heads * n_batch, pair index fastest
   int32_t head0;                // the segment's heads are AttnParams::heads[head0 .. head0 + n_heads)
   int32_t cta_begin;            // linear item index of the segment's first work item
-  // Sliding-tile heads read the caller's RASTER tensors directly: kernel rows are tile-major positions, and a 128-row
-  // block is fetched as 128 / tile_w boxes of one w-row each through a 5-D (channel, W, H, T, head) tensor map
-  // (AttnTmaps::grid), so no tile-major copy of Q / K / V is ever written (reference: tile_layout, tile.py:7-41).
-  // grid_rows > 0 enables it: rows < grid_rows are video tokens (tile-major), rows >= grid_rows (text) use the linear maps.
-  int32_t grid_rows;            // T*H*W, or 0 = rows are linear in the segment's tensors
-  int32_t tile[3];              // tile size (t, h, w)
-  int32_t ntile[3];             // tiles per axis
 };
 
 struct AttnParams {
@@ -112,14 +105,12 @@ struct AttnParams {
   int32_t blend_stage;          // 0 = top-1 mode
   int32_t blend_heads, blend_branch;
   float* dbg;                   // optional debug dump (bring-up only), nullptr in production
-  uint32_t dbg_v_lbo, dbg_v_sbo;  // bring-up overrides of the V descriptor strides (0 = default)
   AttnSeg seg[kMaxSegments];
   AttnHead heads[kMaxHeads];
 };
 
 struct AttnTmaps {
   CUtensorMap m[kMaxSegments][3];   // q, k, v of each segment (4-D: channel, row, head, batch)
-  CUtensorMap grid[3];              // q, k, v of the sliding segment over the raster token grid (5-D), see AttnSeg
 };
 
 // Source head of each processed head slot, passed BY VALUE inside the launch parameters (<= 64 bytes): a layer's

@@ -554,73 +554,23 @@ struct ScatterQkvParams {
   int64_t stride_s[3], stride_h[3];
   uint4* peer[8];
 };
-// Stores every (token, head) row of q, k, v into the receive buffer of the rank that owns the head: the Ulysses "in"
-// exchange as plain NVLink stores (16-byte vectors, 256-byte rows), no staging copy and no collective call.
-__global__ void __launch_bounds__(256)
-vb_ulysses_scatter_qkv_kernel(const ScatterQkvParams p, const HeadTable tab, int64_t rows_total, int s_loc, int heads,
-                              int world, int rank) {
-  const int hp = heads / world;
-  const int64_t rows = static_cast<int64_t>(s_loc) * heads;
-  const int64_t total = rows * 3 * 16;
-  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
-       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const int c = static_cast<int>(i & 15);
-    int64_t r = i >> 4;
-    // order (tensor, peer, token, head-in-chunk): consecutive threads walk one peer's rows contiguously
-    const int hh = static_cast<int>(r % hp);
-    r /= hp;
-    const int64_t sidx = r % s_loc;
-    r /= s_loc;
-    const int peer = static_cast<int>(r % world);
-    const int t = static_cast<int>(r / world);
-    const int hsrc = tab.at[peer * hp + hh];
-    const uint4 val = p.src[t][(sidx * p.stride_s[t] + hsrc * p.stride_h[t]) / 8 + c];
-    const int64_t dst = ((static_cast<int64_t>(t) * rows_total + static_cast<int64_t>(rank) * s_loc + sidx) * hp + hh) * 16 + c;
-    p.peer[peer][dst] = val;
-  }
-}
-
-int launch_ulysses_scatter_qkv(const void* q, const void* k, const void* v, const int64_t* stride_s,
-                               const int64_t* stride_h, void* const* peer_qkv, int64_t rows_total, int s_loc, int heads,
-                               int world, int rank, const int32_t* head_at, cudaStream_t stream) {
-  VB_REQUIRE(world > 0 && world <= 8 && heads % world == 0, VB_ERR_INVALID, "heads %d / world %d not supported", heads,
-             world);
-  ScatterQkvParams p;
-  p.src[0] = static_cast<const uint4*>(q);
-  p.src[1] = static_cast<const uint4*>(k);
-  p.src[2] = static_cast<const uint4*>(v);
-  for (int i = 0; i < 3; ++i) {
-    VB_REQUIRE(stride_s[i] % 8 == 0 && stride_h[i] % 8 == 0, VB_ERR_INVALID, "strides must be multiples of 8 elements");
-    p.stride_s[i] = stride_s[i];
-    p.stride_h[i] = stride_h[i];
-  }
-  for (int i = 0; i < 8; ++i) p.peer[i] = i < world ? static_cast<uint4*>(peer_qkv[i]) : nullptr;
-  HeadTable tab;
-  if (int rc = fill_head_table(tab, head_at, heads)) return rc;
-  const int64_t total = static_cast<int64_t>(s_loc) * heads * 3 * 16;
-  if (total == 0) return VB_OK;
-  const int grid = static_cast<int>((total + 255) / 256 < 148 * 16 ? (total + 255) / 256 : 148 * 16);
-  vb_ulysses_scatter_qkv_kernel<<<grid, 256, 0, stream>>>(p, tab, rows_total, s_loc, heads, world, rank);
-  VB_CUDA_OK(cudaGetLastError());
-  return VB_OK;
-}
-
 struct SlotTable {
   uint8_t peer[kMaxHeadTable], slot[kMaxHeadTable], head[kMaxHeadTable];
 };
-// Placement-table form of the scatter: entry e = (peer, slot, head); order (tensor, entry, token) so that consecutive
-// threads walk one peer's rows of one head.
+// The Ulysses "in" exchange as plain NVLink stores (16-byte vectors, 256-byte rows), no staging copy and no collective
+// call: entry e = (peer, slot, head) stores head `head` of every local token of q, k, v into slot `slot` of peer
+// `peer`'s receive buffer.  Order (tensor, entry, token) so that consecutive threads walk one peer's rows of one head.
 __global__ void __launch_bounds__(256)
 vb_ulysses_scatter_slots_kernel(const ScatterQkvParams p, const SlotTable tab, int n_entries, int64_t rows_total,
-                                int s_loc, int slots, int rank, int t_begin, int t_count) {
+                                int s_loc, int slots, int rank) {
   const int64_t per_tensor = static_cast<int64_t>(n_entries) * s_loc;
-  const int64_t total = per_tensor * t_count * 16;
+  const int64_t total = per_tensor * 3 * 16;
   for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
        i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const int c = static_cast<int>(i & 15);
     int64_t r = i >> 4;
-    const int t = static_cast<int>(r / per_tensor) + t_begin;
-    r -= (t - t_begin) * per_tensor;
+    const int t = static_cast<int>(r / per_tensor);
+    r -= t * per_tensor;
     const int e = static_cast<int>(r % n_entries);      // entry fastest: neighbouring threads read neighbouring heads of a token
     const int64_t sidx = r / n_entries;
     const uint4 val = p.src[t][(sidx * p.stride_s[t] + tab.head[e] * p.stride_h[t]) / 8 + c];
@@ -630,18 +580,10 @@ vb_ulysses_scatter_slots_kernel(const ScatterQkvParams p, const SlotTable tab, i
   }
 }
 
-// tensor_mask: bit t set = scatter tensor t (q, k, v = bits 0, 1, 2; the set bits must be contiguous); max_ctas > 0 caps
-// the grid so that the stores can share the GPU with a GEMM running on another stream.
 int launch_ulysses_scatter_slots(const void* q, const void* k, const void* v, const int64_t* stride_s,
                                  const int64_t* stride_h, void* const* peer_qkv, int64_t rows_total, int s_loc, int slots,
                                  int world, int rank, const int32_t* entry_peer, const int32_t* entry_slot,
-                                 const int32_t* entry_head, int n_entries, int tensor_mask, int max_ctas,
-                                 cudaStream_t stream) {
-  VB_REQUIRE(tensor_mask == 1 || tensor_mask == 2 || tensor_mask == 4 || tensor_mask == 3 || tensor_mask == 6 ||
-                 tensor_mask == 7,
-             VB_ERR_INVALID, "tensor_mask %d must select a contiguous range of q, k, v", tensor_mask);
-  const int t_begin = (tensor_mask & 1) ? 0 : ((tensor_mask & 2) ? 1 : 2);
-  const int t_count = __builtin_popcount(static_cast<unsigned>(tensor_mask));
+                                 const int32_t* entry_head, int n_entries, cudaStream_t stream) {
   VB_REQUIRE(world > 0 && world <= 8 && slots > 0 && slots <= 255, VB_ERR_INVALID, "world %d / slots %d not supported",
              world, slots);
   VB_REQUIRE(n_entries >= 0 && n_entries <= kMaxHeadTable, VB_ERR_UNSUPPORTED, "at most %d placement entries, got %d",
@@ -655,8 +597,6 @@ int launch_ulysses_scatter_slots(const void* q, const void* k, const void* v, co
     p.stride_s[i] = stride_s[i];
     p.stride_h[i] = stride_h[i];
   }
-  for (int i = t_begin; i < t_begin + t_count; ++i)
-    VB_REQUIRE(p.src[i] != nullptr, VB_ERR_INVALID, "tensor %d selected by tensor_mask is null", i);
   for (int i = 0; i < 8; ++i) p.peer[i] = i < world ? static_cast<uint4*>(peer_qkv[i]) : nullptr;
   SlotTable tab;
   memset(&tab, 0, sizeof(tab));
@@ -669,12 +609,10 @@ int launch_ulysses_scatter_slots(const void* q, const void* k, const void* v, co
     tab.slot[e] = static_cast<uint8_t>(entry_slot[e]);
     tab.head[e] = static_cast<uint8_t>(entry_head[e]);
   }
-  const int64_t total = static_cast<int64_t>(n_entries) * s_loc * t_count * 16;
+  const int64_t total = static_cast<int64_t>(n_entries) * s_loc * 3 * 16;
   if (total == 0) return VB_OK;
-  int grid = static_cast<int>((total + 255) / 256 < 148 * 16 ? (total + 255) / 256 : 148 * 16);
-  if (max_ctas > 0) grid = std::min(grid, max_ctas);
-  vb_ulysses_scatter_slots_kernel<<<grid, 256, 0, stream>>>(p, tab, n_entries, rows_total, s_loc, slots, rank, t_begin,
-                                                            t_count);
+  const int grid = static_cast<int>((total + 255) / 256 < 148 * 16 ? (total + 255) / 256 : 148 * 16);
+  vb_ulysses_scatter_slots_kernel<<<grid, 256, 0, stream>>>(p, tab, n_entries, rows_total, s_loc, slots, rank);
   VB_CUDA_OK(cudaGetLastError());
   return VB_OK;
 }

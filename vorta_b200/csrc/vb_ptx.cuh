@@ -115,18 +115,6 @@ __device__ __forceinline__ void tma_load_4d(void* smem_dst, const CUtensorMap* m
       : "memory");
 }
 
-// 5-D tiled load: (c0 = channel, c1 = w, c2 = h, c3 = t, c4 = head)
-__device__ __forceinline__ void tma_load_5d(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1,
-                                            int c2, int c3, int c4) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
-      :
-      : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1),
-        "r"(c2), "r"(c3), "r"(c4)
-      : "memory");
-}
-
 // ----------------------------------------------------------------------------------------------
 // tcgen05: TMEM allocation
 // ----------------------------------------------------------------------------------------------

@@ -4,8 +4,8 @@ The reference (vorta/ulysses/utils.py:15-93) and the NCCL path of this package m
 collectives plus layout copies.  Here every rank maps every peer's receive buffers (torch symmetric memory, one
 allocation per geometry) and
 
-  * "in"  : ``vb_ulysses_scatter_qkv`` stores each (token, head) row of Q, K, V straight into the buffer of the rank that
-            owns the head — one pass, no staging buffer, no collective;
+  * "in"  : ``vb_ulysses_scatter_qkv_slots`` stores each (token, head) row of Q, K, V straight into the buffer of the
+            rank that owns the head — one pass, no staging buffer, no collective;
   * "out" : the attention kernel's epilogue stores each output row straight into the buffer of the rank that owns the
             token (``vb_attn_args.out_peer_ptrs``), already in the (S_loc, H, 128) layout the output projection reads.
 
@@ -27,7 +27,6 @@ from .. import _lib as L
 from . import balance
 from .parallel_states import SP_STATE
 
-_SIDE_CTAS = int(os.environ.get("VB_ULYSSES_SIDE_CTAS", "32"))      # grid cap of the side-stream store kernels
 _EXCHANGES: Dict[tuple, "PeerExchange"] = {}
 _DISABLED_REASON: Optional[str] = None
 
@@ -65,7 +64,6 @@ class PeerExchange:
         # bytes this rank stores into OTHER ranks' buffers over NVLink, counted from the placement tables (the NVLink data
         # counters of nvidia-smi read N/A on this pool): "in" = Q/K/V rows of scatter_qkv, "out" = attention output rows
         self.nvlink_tx_bytes = 0
-        self._side = None
 
     def _tables(self, placement):
         peers, slots, heads = [], [], []
@@ -81,18 +79,17 @@ class PeerExchange:
         arr = C.c_int32 * n
         return arr(*peers), arr(*slots), arr(*heads), n
 
-    def _scatter(self, tensors, tables, mask: int, max_ctas: int = 0) -> None:
-        """tensors: [q, k, v] (1, H, S_loc, 128) views or None for the ones ``mask`` does not select."""
+    def _scatter(self, tensors, tables) -> None:
+        """tensors: [q, k, v] (1, H, S_loc, 128) views."""
         i64x3 = C.c_int64 * 3
-        ref = next(t for t in tensors if t is not None)
-        ptr = [t.data_ptr() if t is not None else None for t in tensors]
-        st_s = i64x3(*[t.stride(2) if t is not None else 8 for t in tensors])
-        st_h = i64x3(*[t.stride(1) if t is not None else 8 for t in tensors])
+        ref = tensors[0]
+        st_s = i64x3(*[t.stride(2) for t in tensors])
+        st_h = i64x3(*[t.stride(1) for t in tensors])
         peers, slots, heads, n = tables
         with torch.cuda.device(ref.device):
-            L.check(L.lib().vb_ulysses_scatter_slots_partial(
-                ptr[0], ptr[1], ptr[2], st_s, st_h, self.qkv_ptrs, self.S + self.text_len, self.s_loc, self.slots, self.P,
-                self.rank, peers, slots, heads, n, mask, max_ctas, torch.cuda.current_stream(ref.device).cuda_stream))
+            L.check(L.lib().vb_ulysses_scatter_qkv_slots(
+                *[t.data_ptr() for t in tensors], st_s, st_h, self.qkv_ptrs, self.S + self.text_len, self.s_loc,
+                self.slots, self.P, self.rank, peers, slots, heads, n, torch.cuda.current_stream(ref.device).cuda_stream))
 
     def scatter_qkv(self, q: torch.Tensor, k: torch.Tensor, v: torch.Tensor,
                     placement: Sequence[Sequence[Tuple[int, int]]], text: Optional[Sequence[torch.Tensor]] = None
@@ -103,49 +100,14 @@ class PeerExchange:
         views of the local receive buffer, valid after barrier A (issued here); only the first len(placement[rank])
         slots hold data.  ``text``: the replicated (1, H, T, 128) text rows of q, k, v; the rows of this rank's heads are
         copied behind the video rows locally (no traffic)."""
-        self._scatter([q, k, v], self._tables(placement), 7)
-        return self._finish_scatter(placement, text, q.device)
-
-    def _finish_scatter(self, placement, text, device):
+        self._scatter([q, k, v], self._tables(placement))
         if self.text_len:
             mine = [h for h, _ in placement[self.rank]]
-            sel = torch.tensor(mine, device=device)
+            sel = torch.tensor(mine, device=q.device)
             for i, t in enumerate(text):          # (1, H, T, 128) -> rows [S, S + T) of my first len(mine) slots
                 self.qkv[i, self.S:, :len(mine)].copy_(t[0].index_select(0, sel).transpose(0, 1))
         self.h_qkv.barrier(channel=0)
         return tuple(self.qkv[i].unsqueeze(0).transpose(1, 2) for i in range(3))
-
-    # ---- overlapped form: K and V leave on a side stream while the next projection GEMM runs -----------------------
-    def overlap_begin(self, placement):
-        """Start an exchange whose tensors are handed over one by one (``overlap_send``) as the projections produce
-        them; ``overlap_end`` issues barrier A.  The side stream has high priority and its store kernels use a capped
-        grid, so they share the GPU with the GEMM of the next projection instead of running exposed after all three."""
-        if self._side is None:
-            self._side = torch.cuda.Stream(device=self.qkv.device, priority=-1)
-        self._tables_now = self._tables(placement)
-        self._placement_now = placement
-        self._pending = False
-
-    def overlap_send(self, which: int, x: torch.Tensor, side: bool) -> None:
-        """x: (1, H, S_loc, 128) view of tensor ``which`` (0 = q, 1 = k, 2 = v), complete on the current stream."""
-        tensors = [None, None, None]
-        tensors[which] = x
-        if not side:
-            self._scatter(tensors, self._tables_now, 1 << which)
-            return
-        main = torch.cuda.current_stream(x.device)
-        ready = torch.cuda.Event()
-        ready.record(main)
-        self._side.wait_event(ready)
-        x.record_stream(self._side)
-        with torch.cuda.stream(self._side):
-            self._scatter(tensors, self._tables_now, 1 << which, max_ctas=_SIDE_CTAS)
-        self._pending = True
-
-    def overlap_end(self, device, text=None):
-        if self._pending:
-            torch.cuda.current_stream(device).wait_stream(self._side)
-        return self._finish_scatter(self._placement_now, text, device)
 
     def zero_padded_text(self, text_valid: int) -> None:
         """Rows of padded text queries are written by nobody (hunyuan.py:176 pads with zeros): clear them locally."""
@@ -225,10 +187,3 @@ def nvlink_tx_bytes(reset: bool = False) -> int:
             ex.nvlink_tx_bytes = 0
     return total
 
-
-def overlap_enabled() -> bool:
-    """VB_ULYSSES_OVERLAP=1 (opt-in) sends K and V on a side stream while the next projection GEMM runs.  Measured
-    slower than one pass after all three projections — Wan-14B on 2 GPUs 1688 vs 1620 ms / step, alternating runs on one
-    box (profiles/r2p_*): the cuBLAS GEMMs are persistent over all SMs, so the 32 store CTAs delay whole GEMM waves
-    instead of filling idle SMs, and a 32-CTA grid does not saturate NVLink.  Results are bit-identical either way."""
-    return os.environ.get("VB_ULYSSES_OVERLAP", "0") == "1"

@@ -22,6 +22,7 @@ CASES = (("dense16k", (1, 1, 16384), (1, 1, 16384), (1, 1, 2), 37, [0] * 37),
          ("wan14 coreset H=16", W14, (3, 9, 16), (3, 3, 2), 16, [1] * 16),
          ("wan14 sliding H=16", W14, (3, 9, 16), (3, 3, 2), 16, [2] * 16),
          ("wan14mix", W14, (3, 9, 16), (3, 3, 2), 40, [0] * 9 + [1] * 18 + [2] * 13),
+         ("wan14 blend H=40", W14, (3, 9, 16), (3, 3, 2), 40, None),
          ("wan14 native sliding (5,9,8) H=16", (20, 45, 80), (5, 9, 8), (2, 3, 2), 16, [2] * 16),
          ("wan13 sliding H=12", W13, (3, 10, 4), (3, 3, 2), 12, [2] * 12),
          ("wan13 mix 4f/4c/4s H=12", W13, (3, 10, 4), (3, 3, 2), 12, [0] * 4 + [1] * 4 + [2] * 4))
@@ -30,9 +31,11 @@ for name, lat, tile, lw, H, branch in CASES:
     plan = ops.Plan(lat, tile, (3, 3, 3) if lat[0] > 1 else (1, 1, 1), lw, 0.5)
     S = plan.seq_len
     q, k, v = (torch.randn((1, S, H, 128), device="cuda").bfloat16().transpose(1, 2) for _ in range(3))
+    # branch None: blend mode, every branch on every head weighted by routing scores
+    kw = dict(branch=branch) if branch else dict(weights=torch.softmax(torch.randn((1, H, 3), device="cuda"), -1))
     rates = []
     for _ in range(3):
-        ms, fl = timed(lambda: ops.routed_attention(plan, q, k, v, branch=branch))
+        ms, fl = timed(lambda: ops.routed_attention(plan, q, k, v, **kw))
         rates.append(fl / ms / 1e9)
     out.append("%%s %%.1f" %% (name, statistics.median(rates)))
     del q, k, v, plan

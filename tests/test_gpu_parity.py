@@ -481,7 +481,8 @@ def test_branches_vs_oracle(lat, tile, win, lw, H, tl, tv):
 
 
 def test_batch_and_head_strides():
-    """Batch > 1, head-major (B, H, S, D) memory as well as token-major, and more than one 64-head launch chunk."""
+    """Batch > 1, head-major (B, H, S, D) memory as well as token-major, and more than one 64-head launch chunk (routed
+    and dense)."""
     lat, tile, win, lw = (2, 8, 8), (1, 4, 4), (3, 3, 3), (2, 2, 2)
     S, B, H = 128, 2, 3
     g = torch.Generator().manual_seed(3)
@@ -497,6 +498,58 @@ def test_batch_and_head_strides():
     out = ops.routed_attention(plan, q.to(dev()), k.to(dev()), v.to(dev()), weights=w)
     ref = O.routed_attention(q.float(), k.float(), v.float(), info, lat, win, tile, weights=w)
     assert_attn_close(out, ref)
+    # 72 heads run as launches of 64 + 8 heads; heads are independent, so two calls of 36 heads give the same bits
+    H = 72
+    q, k, v = (torch.randn((B, S, H, 128), generator=g).to(torch.bfloat16).to(dev()).transpose(1, 2) for _ in range(3))
+    out = ops.routed_attention(plan, q, k, v, branch=[0] * H)
+    for hs in (slice(0, 36), slice(36, H)):
+        assert torch.equal(ops.routed_attention(plan, q[:, hs], k[:, hs], v[:, hs], branch=[0] * 36), out[:, hs])
+    q = torch.randn((B, 300, H, 128), generator=g).to(torch.bfloat16).to(dev()).transpose(1, 2)
+    k, v = (torch.randn((B, 77, H, 128), generator=g).to(torch.bfloat16).to(dev()).transpose(1, 2) for _ in range(2))
+    out = ops.attn_dense(q, k, v)
+    for hs in (slice(0, 36), slice(36, H)):
+        assert torch.equal(ops.attn_dense(q[:, hs], k[:, hs], v[:, hs]), out[:, hs])
+
+
+def test_layer_launch_structure():
+    """What a layer issues, through the launch and FLOP counters and the per-caller timing: a top-1 layer with every
+    branch and a query-half pair (two coreset selections, two pooling gathers, the sliding layout gather, ONE attention
+    launch, the zeroing of padded text rows); the same layer blended (one attention launch per branch); 72 full heads and
+    72 dense heads (two launches each, at most 64 heads per launch)."""
+    def measure(fn):
+        torch.cuda.synchronize()
+        ops.timing_enable(True)
+        ops.timing_collect()
+        ops.stats_reset()
+        try:
+            fn()
+            torch.cuda.synchronize()
+        finally:
+            ops.timing_enable(False)
+        kinds = ops.timing_collect_kinds()
+        return ops.stats(), kinds["routed"][1:], kinds["dense"][1:]
+
+    g = torch.Generator().manual_seed(23)
+    plan = ops.Plan((6, 12, 8), (3, 6, 4), (3, 3, 3), (2, 3, 2), 0.5, text_len=40, text_valid=23)
+    S, H = plan.seq_len, 5
+    q, k, v = (torch.randn((1, S + 40, H, 128), generator=g).to(torch.bfloat16).to(dev()).transpose(1, 2)
+               for _ in range(3))
+    w = torch.softmax(torch.randn((1, H, 3), generator=g), -1)
+    branch = [0, 1, 2, L.BRANCH_FULL_LO, L.BRANCH_FULL_HI]
+    fl = 600639488.0
+    assert measure(lambda: ops.routed_attention(plan, q, k, v, branch=branch, flags=L.ATTN_CORESET_KV_FROM_K)) == \
+        ((7, fl), (1, fl), (0, 0.0))
+    fl = 2084666880.0
+    assert measure(lambda: ops.routed_attention(plan, q, k, v, weights=w, flags=L.ATTN_CORESET_KV_FROM_K)) == \
+        ((9, fl), (3, fl), (0, 0.0))
+    plan = ops.Plan((2, 8, 8), (1, 4, 4), (3, 3, 3), (2, 2, 2), 0.5)
+    q, k, v = (torch.randn((2, 72, 128, 128), generator=g).to(torch.bfloat16).to(dev()) for _ in range(3))
+    fl = 1207959552.0
+    assert measure(lambda: ops.routed_attention(plan, q, k, v, branch=[0] * 72)) == ((2, fl), (2, fl), (0, 0.0))
+    q = torch.randn((1, 72, 300, 128), generator=g).to(torch.bfloat16).to(dev())
+    k, v = (torch.randn((1, 72, 77, 128), generator=g).to(torch.bfloat16).to(dev()) for _ in range(2))
+    fl = 851558400.0
+    assert measure(lambda: ops.attn_dense(q, k, v)) == ((2, fl), (0, 0.0), (2, fl))
 
 
 def test_dense_attention_independent_lengths():

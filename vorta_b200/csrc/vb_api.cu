@@ -41,7 +41,6 @@ struct TimedLaunch {
   double flops;
 };
 static thread_local std::vector<TimedLaunch> g_events;
-static thread_local int g_launch_kind = VB_TIMING_ROUTED;
 
 // ---- kernels implemented in the other translation units -----------------------------------------
 int launch_coreset_select(const SelectParams& p, cudaStream_t stream);
@@ -528,6 +527,19 @@ int vb_router_forward(const void* temb, int temb_dtype, const void* w, const voi
   return rc;
 }
 
+// Coreset selection over x, (b, h, s) element strides, for `heads` head slots of every batch element: slot i reads head
+// i, and no output table is set yet.
+static SelectParams select_params(const vb_plan* pl, const void* x, const int64_t* stride, int batch, int heads) {
+  SelectParams p;
+  memset(&p, 0, sizeof(p));
+  p.x = static_cast<const __nv_bfloat16*>(x);
+  p.stride_b = stride[0]; p.stride_h = stride[1]; p.stride_s = stride[2];
+  p.center_tok = pl->d_center_tok; p.margin_tok = pl->d_margin_tok;
+  p.batch = batch; p.heads = heads; p.G = pl->G; p.n_margin = pl->g - 1; p.n_unpooled = pl->n_u;
+  p.seq_len = pl->S; p.text_len = pl->d.text_len;
+  return p;
+}
+
 int vb_coreset_select(const vb_plan* pl, const void* x, int64_t stride_b, int64_t stride_h, int64_t stride_s,
                       int32_t batch, int32_t heads, int64_t* unpooled_argsort, int64_t* pooled_argsort,
                       int32_t* kept_tok, int32_t* dropped_tok, vb_stream_t stream) {
@@ -535,12 +547,8 @@ int vb_coreset_select(const vb_plan* pl, const void* x, int64_t stride_b, int64_
   VB_REQUIRE(pl->has_device, VB_ERR_UNSUPPORTED, "no CUDA device: vorta_b200 has no CPU path");
   VB_REQUIRE(stride_s % 8 == 0 && stride_h % 8 == 0 && stride_b % 8 == 0, VB_ERR_INVALID,
              "strides must be multiples of 8 elements");
-  SelectParams p;
-  p.x = static_cast<const __nv_bfloat16*>(x);
-  p.stride_b = stride_b; p.stride_h = stride_h; p.stride_s = stride_s;
-  p.center_tok = pl->d_center_tok; p.margin_tok = pl->d_margin_tok; p.head_list.used = 0;
-  p.batch = batch; p.heads = heads; p.G = pl->G; p.n_margin = pl->g - 1; p.n_unpooled = pl->n_u;
-  p.seq_len = pl->S; p.text_len = pl->d.text_len;
+  const int64_t stride[3] = {stride_b, stride_h, stride_s};
+  SelectParams p = select_params(pl, x, stride, batch, heads);
   p.unpooled_argsort = unpooled_argsort; p.pooled_argsort = pooled_argsort;
   p.kept_tok = kept_tok; p.dropped_tok = dropped_tok;
   int rc = launch_coreset_select(p, static_cast<cudaStream_t>(stream));
@@ -611,136 +619,156 @@ struct Carver {
   }
 };
 
-struct BranchLaunch {
-  const __nv_bfloat16 *q, *k, *v;
-  int64_t qs[3], ks[3], vs[3];   // b, h, s strides
-  int64_t n_rows_q, n_rows_kv, n_heads_tensor;
-  const Schedule* sched;
-  const int32_t* out_map;
-  int64_t out_map_stride_b, out_map_stride_h;
-  const int32_t* bcast_map;
-  int64_t bcast_stride_b, bcast_stride_h;
-  int32_t bcast_rows, bcast_n;
+// One branch of a layer, or one query part of the full branch, with the head slots it covers: one AttnSeg of a launch.
+struct Segment {
+  const __nv_bfloat16 *q = nullptr, *k = nullptr, *v = nullptr;
+  int64_t qs[3] = {}, ks[3] = {}, vs[3] = {};   // b, h, s strides
+  int64_t n_rows_q = 0, n_rows_kv = 0, n_heads_tensor = 0;
+  const Schedule* sched = nullptr;
+  int pair_begin = 0, n_pairs = 0;              // the segment's work items: sched->pairs[pair_begin, + n_pairs)
+  const int32_t* out_map = nullptr;
+  int64_t out_map_stride_b = 0, out_map_stride_h = 0;
+  const int32_t* bcast_map = nullptr;
+  int64_t bcast_stride_b = 0, bcast_stride_h = 0;
+  int32_t bcast_rows = 0, bcast_n = 0;
+  std::vector<AttnHead> heads;
+  double flops_per_head = 0.0;                  // of the segment's work items
 };
-}  // namespace
 
-// Blend-mode state of the launch being assembled (vb_attn_fwd sets it around run_branch)
+// Where the attention output goes: `ptr`, or the peer buffers of the fused Ulysses exchange (vb_attn_args::out_peer_*).
+struct Output {
+  __nv_bfloat16* ptr;
+  int64_t stride[3];                            // b, h, s
+  __nv_bfloat16* peers[8];
+  int32_t peer_count, peer_rows;
+};
+
+// Blend mode: the routing scores, the fp32 sums, and which of the three accumulation stages a launch is.
 struct BlendState {
   const float* w;
   float* acc;
   int stage, branch, heads;
 };
-static thread_local const BlendState* g_blend = nullptr;
+}  // namespace
 
-// One branch with the head slots it covers; pair_count > 0 restricts it to a sub-range of the schedule's work items
-// (the query halves of VB_BRANCH_FULL_LO / _HI).
-struct Segment {
-  BranchLaunch bl;
-  std::vector<AttnHead> heads;
-  int pair_begin = 0, pair_count = 0;
-};
-
-// Launch up to kMaxSegments branches as ONE grid (segments in the given order = longest CTAs first), covering
-// batches [batch0, batch0 + nbatch).  The caller guarantees that the segments write disjoint outputs or that a single
-// segment is passed (blend mode accumulates branch after branch and therefore launches them one by one).
-static int launch_segments(const Segment* const* segs, int n_seg, const vb_attn_args& a, int batch0, int nbatch,
-                           cudaStream_t stream) {
-  AttnTmaps tm;
-  AttnParams p;
-  memset(&tm, 0, sizeof(tm));
-  memset(&p, 0, sizeof(p));
-  int rc, n_used = 0, head0 = 0;
-  int64_t n_ctas = 0;
-  double flops = 0.0;
-  for (int i = 0; i < n_seg; ++i) {
-    const Segment& sg = *segs[i];
-    const BranchLaunch& bl = sg.bl;
-    if (sg.heads.empty() || bl.sched->pairs.empty()) continue;
-    if (sg.pair_count < 0 || sg.pair_begin + sg.pair_count > static_cast<int>(bl.sched->pairs.size())) continue;
-    VB_REQUIRE(head0 + sg.heads.size() <= static_cast<size_t>(kMaxHeads), VB_ERR_INVALID,
-               "more than %d heads in one attention launch", kMaxHeads);
-    CUtensorMap* m = tm.m[n_used];
-    if ((rc = make_qkv_tensor_map(&m[0], bl.q, bl.n_rows_q, bl.n_heads_tensor, a.batch, bl.qs[0], bl.qs[1], bl.qs[2])))
-      return rc;
-    if ((rc = make_qkv_tensor_map(&m[1], bl.k, bl.n_rows_kv, bl.n_heads_tensor, a.batch, bl.ks[0], bl.ks[1], bl.ks[2])))
-      return rc;
-    if ((rc = make_qkv_tensor_map(&m[2], bl.v, bl.n_rows_kv, bl.n_heads_tensor, a.batch, bl.vs[0], bl.vs[1], bl.vs[2])))
-      return rc;
-    AttnSeg& s = p.seg[n_used];
-    s.pairs = bl.sched->d_pairs;
-    s.runs = bl.sched->d_runs;
-    s.out_map = bl.out_map; s.out_map_stride_b = bl.out_map_stride_b; s.out_map_stride_h = bl.out_map_stride_h;
-    s.bcast_map = bl.bcast_map; s.bcast_stride_b = bl.bcast_stride_b; s.bcast_stride_h = bl.bcast_stride_h;
-    s.bcast_rows = bl.bcast_rows; s.bcast_n = bl.bcast_n;
-    s.n_pairs = static_cast<int32_t>(bl.sched->pairs.size());
-    double seg_flops = bl.sched->flops_per_head;
-    if (sg.pair_count > 0) {      // a query sub-range of the schedule: its share of the head's FLOPs goes by query rows
-      int64_t rows_all = 0, rows_sub = 0;
-      for (size_t i = 0; i < bl.sched->pairs.size(); ++i) {
-        const QPair& qp = bl.sched->pairs[i];
-        const int64_t r = qp.q_rows[0] + (qp.nq == 2 ? qp.q_rows[1] : 0);
-        rows_all += r;
-        if (static_cast<int>(i) >= sg.pair_begin && static_cast<int>(i) < sg.pair_begin + sg.pair_count) rows_sub += r;
-      }
-      s.pairs = bl.sched->d_pairs + sg.pair_begin;
-      s.n_pairs = sg.pair_count;
-      seg_flops *= static_cast<double>(rows_sub) / static_cast<double>(std::max<int64_t>(rows_all, 1));
-    }
-    s.n_heads = static_cast<int32_t>(sg.heads.size());
-    s.head0 = head0;
-    s.cta_begin = static_cast<int32_t>(n_ctas);
-    for (size_t h = 0; h < sg.heads.size(); ++h) p.heads[head0 + h] = sg.heads[h];
-    head0 += s.n_heads;
-    n_ctas += static_cast<int64_t>(s.n_pairs) * s.n_heads * nbatch;
-    flops += seg_flops * s.n_heads * nbatch;
-    ++n_used;
-  }
-  if (n_used == 0) return VB_OK;
-  VB_REQUIRE(n_ctas < (1ll << 31), VB_ERR_UNSUPPORTED, "attention grid too large");
-  p.n_seg = n_used;
-  p.n_items = static_cast<int32_t>(n_ctas);
-  p.out = static_cast<__nv_bfloat16*>(a.out);
-  p.out_stride_b = a.out_stride[0]; p.out_stride_h = a.out_stride[1]; p.out_stride_s = a.out_stride[2];
-  p.out_peer_count = a.out_peer_count;
-  p.out_peer_rows = a.out_peer_rows;
-  for (int i = 0; i < 8; ++i)
-    p.out_peers[i] = i < a.out_peer_count ? static_cast<__nv_bfloat16*>(a.out_peer_ptrs[i]) : nullptr;
-  p.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(kHeadDim));
-  if (g_blend != nullptr) {
-    p.blend_w = g_blend->w; p.blend_acc = g_blend->acc; p.blend_stage = g_blend->stage;
-    p.blend_heads = g_blend->heads; p.blend_branch = g_blend->branch;
-  }
-  p.batch0 = batch0;
-  p.dbg = a.debug;
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-  if (g_timing) {
-    VB_CUDA_OK(cudaEventCreate(&ev0));
-    VB_CUDA_OK(cudaEventCreate(&ev1));
-    VB_CUDA_OK(cudaEventRecord(ev0, stream));
-  }
-  rc = launch_attn(tm, p, static_cast<int>(n_ctas), stream);
-  if (rc != VB_OK) return rc;
-  if (g_timing) {
-    VB_CUDA_OK(cudaEventRecord(ev1, stream));
-    g_events.push_back({ev0, ev1, g_launch_kind, flops});
-  }
-  ++g_launches;
-  g_flops += flops;
-  return VB_OK;
+// A segment over all of `sched` for q, k, v with (b, h, s) element strides; no head slots yet.
+static Segment segment_of(const void* q, const void* k, const void* v, const int64_t* qs, const int64_t* ks,
+                          const int64_t* vs, int64_t n_rows_q, int64_t n_rows_kv, int64_t n_heads_tensor,
+                          const Schedule& sched) {
+  Segment sg;
+  sg.q = static_cast<const __nv_bfloat16*>(q);
+  sg.k = static_cast<const __nv_bfloat16*>(k);
+  sg.v = static_cast<const __nv_bfloat16*>(v);
+  for (int i = 0; i < 3; ++i) { sg.qs[i] = qs[i]; sg.ks[i] = ks[i]; sg.vs[i] = vs[i]; }
+  sg.n_rows_q = n_rows_q; sg.n_rows_kv = n_rows_kv; sg.n_heads_tensor = n_heads_tensor;
+  sg.sched = &sched;
+  sg.n_pairs = static_cast<int>(sched.pairs.size());
+  sg.flops_per_head = sched.flops_per_head;
+  return sg;
 }
 
-// Launch one branch for the head slots in `heads`, in chunks of <= kMaxHeads.
-static int run_branch(const BranchLaunch& bl, const vb_attn_args& a, const std::vector<AttnHead>& heads, int batch0,
-                      int nbatch, cudaStream_t stream) {
-  for (size_t h0 = 0; h0 < heads.size(); h0 += kMaxHeads) {
-    Segment sg;
-    sg.bl = bl;
-    sg.heads.assign(heads.begin() + h0, heads.begin() + std::min(heads.size(), h0 + static_cast<size_t>(kMaxHeads)));
-    const Segment* one = &sg;
-    int rc = launch_segments(&one, 1, a, batch0, nbatch, stream);
-    if (rc != VB_OK) return rc;
+// A segment over q, k, v gathered into contiguous (batch, nh, rows, 128) workspace tensors, n_rows of them attended.
+static Segment workspace_segment(__nv_bfloat16* const qkv[3], int nh, int64_t rows, int64_t n_rows,
+                                 const Schedule& sched) {
+  const int64_t st[3] = {nh * rows * kHeadDim, rows * kHeadDim, kHeadDim};
+  return segment_of(qkv[0], qkv[1], qkv[2], st, st, st, n_rows, n_rows, nh, sched);
+}
+
+// Tensors first .. first + n - 1 of the layer's (q, k, v) as the sources of a gather into dst[first ..].
+static void gather_from_args(GatherParams& gp, const vb_attn_args& a, int first, int n, __nv_bfloat16* const dst[3]) {
+  const void* src[3] = {a.q, a.k, a.v};
+  const int64_t* stride[3] = {a.q_stride, a.k_stride, a.v_stride};
+  gp.n_tensors = n;
+  for (int t = 0; t < n; ++t) {
+    gp.src[t] = static_cast<const __nv_bfloat16*>(src[first + t]);
+    gp.dst[t] = dst[first + t];
+    for (int i = 0; i < 3; ++i) gp.src_stride[t][i] = stride[first + t][i];
   }
-  return VB_OK;
+}
+
+// Launches the head slots of n_seg <= kMaxSegments segments, in the given order (longest CTAs first), as grids of at
+// most kMaxHeads heads: a grid takes head slots until it is full, so a segment with more heads spans several launches.
+// The segments write disjoint outputs, or there is one of them (blend mode accumulates branch after branch).
+static int launch_segments(const Segment* segs, int n_seg, int batch, const Output& out, float* dbg,
+                           const BlendState* blend, int kind, cudaStream_t stream) {
+  AttnTmaps tm;
+  AttnParams p;
+  int rc, n_used, head0;
+  int64_t n_ctas;
+  double flops;
+  auto start_grid = [&]() {
+    memset(&tm, 0, sizeof(tm));
+    memset(&p, 0, sizeof(p));
+    n_used = head0 = 0;
+    n_ctas = 0;
+    flops = 0.0;
+  };
+  auto launch_grid = [&]() -> int {
+    if (n_used == 0) return VB_OK;
+    VB_REQUIRE(n_ctas < (1ll << 31), VB_ERR_UNSUPPORTED, "attention grid too large");
+    p.n_seg = n_used;
+    p.n_items = static_cast<int32_t>(n_ctas);
+    p.out = out.ptr;
+    p.out_stride_b = out.stride[0]; p.out_stride_h = out.stride[1]; p.out_stride_s = out.stride[2];
+    p.out_peer_count = out.peer_count;
+    p.out_peer_rows = out.peer_rows;
+    for (int i = 0; i < 8; ++i) p.out_peers[i] = out.peers[i];
+    p.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(kHeadDim));
+    if (blend != nullptr) {
+      p.blend_w = blend->w; p.blend_acc = blend->acc; p.blend_stage = blend->stage;
+      p.blend_heads = blend->heads; p.blend_branch = blend->branch;
+    }
+    p.dbg = dbg;
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    if (g_timing) {
+      VB_CUDA_OK(cudaEventCreate(&ev0));
+      VB_CUDA_OK(cudaEventCreate(&ev1));
+      VB_CUDA_OK(cudaEventRecord(ev0, stream));
+    }
+    const int r = launch_attn(tm, p, static_cast<int>(n_ctas), stream);
+    if (r != VB_OK) return r;
+    if (g_timing) {
+      VB_CUDA_OK(cudaEventRecord(ev1, stream));
+      g_events.push_back({ev0, ev1, kind, flops});
+    }
+    ++g_launches;
+    g_flops += flops;
+    start_grid();
+    return VB_OK;
+  };
+  start_grid();
+  for (int i = 0; i < n_seg; ++i) {
+    const Segment& sg = segs[i];
+    if (sg.n_pairs == 0) continue;
+    for (size_t h = 0; h < sg.heads.size();) {
+      if (head0 == kMaxHeads && (rc = launch_grid()) != VB_OK) return rc;
+      const int n = static_cast<int>(std::min(sg.heads.size() - h, static_cast<size_t>(kMaxHeads - head0)));
+      CUtensorMap* m = tm.m[n_used];
+      if ((rc = make_qkv_tensor_map(&m[0], sg.q, sg.n_rows_q, sg.n_heads_tensor, batch, sg.qs[0], sg.qs[1], sg.qs[2])))
+        return rc;
+      if ((rc = make_qkv_tensor_map(&m[1], sg.k, sg.n_rows_kv, sg.n_heads_tensor, batch, sg.ks[0], sg.ks[1], sg.ks[2])))
+        return rc;
+      if ((rc = make_qkv_tensor_map(&m[2], sg.v, sg.n_rows_kv, sg.n_heads_tensor, batch, sg.vs[0], sg.vs[1], sg.vs[2])))
+        return rc;
+      AttnSeg& s = p.seg[n_used];
+      s.pairs = sg.sched->d_pairs + sg.pair_begin;
+      s.runs = sg.sched->d_runs;
+      s.out_map = sg.out_map; s.out_map_stride_b = sg.out_map_stride_b; s.out_map_stride_h = sg.out_map_stride_h;
+      s.bcast_map = sg.bcast_map; s.bcast_stride_b = sg.bcast_stride_b; s.bcast_stride_h = sg.bcast_stride_h;
+      s.bcast_rows = sg.bcast_rows; s.bcast_n = sg.bcast_n;
+      s.n_pairs = sg.n_pairs;
+      s.n_heads = n;
+      s.head0 = head0;
+      s.cta_begin = static_cast<int32_t>(n_ctas);
+      for (int j = 0; j < n; ++j) p.heads[head0 + j] = sg.heads[h + j];
+      head0 += n;
+      h += n;
+      n_ctas += static_cast<int64_t>(s.n_pairs) * s.n_heads * batch;
+      flops += sg.flops_per_head * s.n_heads * batch;
+      ++n_used;
+    }
+  }
+  return launch_grid();
 }
 
 int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
@@ -816,12 +844,13 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
     blend_state.heads = a.heads;
   }
 
-  auto head_entries = [&](const std::vector<int32_t>& hs, int e, bool slot_is_index, int b) {
+  // head slots of a segment over heads hs; hk is the head in the segment's q / k / v: the layer's head, or the slot of a
+  // workspace copy that holds only hs
+  auto head_entries = [&](const std::vector<int32_t>& hs, bool slot_is_index) {
     std::vector<AttnHead> v(hs.size());
     for (size_t i = 0; i < hs.size(); ++i) {
       v[i].hk = slot_is_index ? static_cast<int32_t>(i) : hs[i];
       v[i].ho = a.out_heads ? a.out_heads[hs[i]] : hs[i];
-      v[i].weight = 1.f;
       v[i].wi = hs[i];
     }
     return v;
@@ -834,54 +863,43 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
     for (size_t i = 0; i < hs.size(); ++i) out->h[i] = static_cast<uint8_t>(hs[i]);
     return VB_OK;
   };
-  // blend weights differ per batch element; top-1 routing is shared by the batch (wan.py:398)
-  // top-1 mode: every head is in exactly one branch, so the branches write disjoint outputs and run as segments of ONE
-  // launch after all selection / gather passes have been issued; kept in branch order full, coreset, sliding, which is
-  // longest-CTA-first (full: S/128 key blocks per CTA, coreset: ~S/256, sliding: <= 27 tiles)
-  Segment deferred[kMaxSegments];
-  int n_deferred = 0;
+  // top-1 mode: every head is in exactly one segment, so the segments write disjoint outputs and run as ONE launch after
+  // all selection / gather passes; kept in branch order full, query parts, coreset, sliding, which is longest-CTA-first
+  // (full: S/128 key blocks per CTA, coreset: ~S/256, sliding: <= 27 tiles)
   const bool merge = !blend && a.heads <= kMaxHeads;
   VB_REQUIRE(!blend || parts.empty(), VB_ERR_INVALID, "query-part ids need top-1 mode");
-  auto for_batches = [&](const BranchLaunch& bl, const std::vector<int32_t>& hs, int e, bool slot_is_index,
-                         int pair_begin = 0, int pair_count = 0) -> int {
-    if (merge) {
-      deferred[n_deferred].bl = bl;
-      deferred[n_deferred].heads = head_entries(hs, e, slot_is_index, 0);
-      deferred[n_deferred].pair_begin = pair_begin;
-      deferred[n_deferred].pair_count = pair_count;
-      ++n_deferred;
-      return VB_OK;
-    }
-    VB_REQUIRE(pair_count == 0, VB_ERR_UNSUPPORTED, "query-half work units need the merged top-1 launch");
-    // blend: branch e is stage e + 1 of the fp32 accumulation; ONE launch covers every batch element (the scores are read
-    // per (batch, head) from the device table)
-    if (blend) {
-      blend_state.stage = e + 1;
-      blend_state.branch = e;
-      g_blend = &blend_state;
-    }
-    const int r = run_branch(bl, a, head_entries(hs, e, slot_is_index, 0), 0, a.batch, stream);
-    g_blend = nullptr;
-    return r;
-  };
+  std::vector<Segment> segs;
 
   // ---------------- branch 0: full attention, straight from the caller's tensors ----------------
   if (!by_branch[0].empty() || !parts.empty()) {
-    BranchLaunch bl;
-    memset(&bl, 0, sizeof(bl));
-    bl.q = static_cast<const __nv_bfloat16*>(a.q);
-    bl.k = static_cast<const __nv_bfloat16*>(a.k);
-    bl.v = static_cast<const __nv_bfloat16*>(a.v);
-    for (int i = 0; i < 3; ++i) { bl.qs[i] = a.q_stride[i]; bl.ks[i] = a.k_stride[i]; bl.vs[i] = a.v_stride[i]; }
-    bl.n_rows_q = S + TV; bl.n_rows_kv = S + TV; bl.n_heads_tensor = a.heads;
-    bl.sched = &pl->full;
-    if (!by_branch[0].empty() && (rc = for_batches(bl, by_branch[0], 0, false)) != VB_OK) return rc;
-    // query parts: work items [k N / n, (k + 1) N / n) of the same schedule (other ranks run the other parts)
-    const int64_t n_items_full = static_cast<int64_t>(pl->full.pairs.size());
+    const Segment full =
+        segment_of(a.q, a.k, a.v, a.q_stride, a.k_stride, a.v_stride, S + TV, S + TV, a.heads, pl->full);
+    if (!by_branch[0].empty()) {
+      segs.push_back(full);
+      segs.back().heads = head_entries(by_branch[0], false);
+    }
+    // query parts: work items [k N / n, (k + 1) N / n) of the same schedule (other ranks run the other parts); a part's
+    // share of the head's FLOPs goes by query rows
+    const std::vector<QPair>& items = pl->full.pairs;
+    auto rows_of = [&](int begin, int end) {
+      int64_t rows = 0;
+      for (int i = begin; i < end; ++i) rows += items[i].q_rows[0] + (items[i].nq == 2 ? items[i].q_rows[1] : 0);
+      return rows;
+    };
+    const int64_t n_items = static_cast<int64_t>(items.size());
+    const int64_t rows_all = rows_of(0, static_cast<int>(n_items));
     for (const auto& part : parts) {
       const int n = (part.first - 16) >> 3, k = (part.first - 16) & 7;
-      const int begin = static_cast<int>(n_items_full * k / n), end = static_cast<int>(n_items_full * (k + 1) / n);
-      if (end > begin && (rc = for_batches(bl, part.second, 0, false, begin, end - begin)) != VB_OK) return rc;
+      const int begin = static_cast<int>(n_items * k / n), end = static_cast<int>(n_items * (k + 1) / n);
+      if (end <= begin) continue;
+      VB_REQUIRE(merge, VB_ERR_UNSUPPORTED, "query-half work units need the merged top-1 launch");
+      segs.push_back(full);
+      Segment& sg = segs.back();
+      sg.heads = head_entries(part.second, false);
+      sg.pair_begin = begin;
+      sg.n_pairs = end - begin;
+      sg.flops_per_head = pl->full.flops_per_head * (static_cast<double>(rows_of(begin, end)) /
+                                                     static_cast<double>(std::max<int64_t>(rows_all, 1)));
     }
   }
 
@@ -892,9 +910,8 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
     const int nh = static_cast<int>(hs.size());
     const int64_t rows = pl->S_c + TL;
     const int64_t bh = static_cast<int64_t>(a.batch) * nh;
-    __nv_bfloat16* pq = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
-    __nv_bfloat16* pk = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
-    __nv_bfloat16* pv = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
+    __nv_bfloat16* pooled[3];
+    for (__nv_bfloat16*& t : pooled) t = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
     int32_t* kept_q = static_cast<int32_t*>(ws.take(bh * rows * 4));
     int32_t* drop_q = static_cast<int32_t*>(ws.take(bh * pl->G * std::max(pl->n_p, 1) * 4));
     int32_t* kept_k = kept_q;
@@ -902,21 +919,15 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
     if (kv_from_k) kept_k = static_cast<int32_t*>(ws.take(bh * rows * 4));
     HeadList heads_c;
     if ((rc = head_list_of(hs, &heads_c)) != VB_OK) return rc;
-    VB_REQUIRE(pq && pk && pv && kept_q && drop_q && kept_k, VB_ERR_INVALID, "workspace exhausted");
+    VB_REQUIRE(pooled[0] && pooled[1] && pooled[2] && kept_q && drop_q && kept_k, VB_ERR_INVALID, "workspace exhausted");
 
-    SelectParams sp;
-    sp.x = static_cast<const __nv_bfloat16*>(a.q);
-    sp.stride_b = a.q_stride[0]; sp.stride_h = a.q_stride[1]; sp.stride_s = a.q_stride[2];
-    sp.center_tok = pl->d_center_tok; sp.margin_tok = pl->d_margin_tok; sp.head_list = heads_c;
-    sp.batch = a.batch; sp.heads = nh; sp.G = pl->G; sp.n_margin = pl->g - 1; sp.n_unpooled = pl->n_u;
-    sp.seq_len = S; sp.text_len = TL;
-    sp.unpooled_argsort = nullptr; sp.pooled_argsort = nullptr; sp.kept_tok = kept_q; sp.dropped_tok = drop_q;
+    SelectParams sp = select_params(pl, a.q, a.q_stride, a.batch, nh);
+    sp.head_list = heads_c; sp.kept_tok = kept_q; sp.dropped_tok = drop_q;
     if ((rc = launch_coreset_select(sp, stream)) != VB_OK) return rc;
     ++g_launches;
     if (kv_from_k) {
-      sp.x = static_cast<const __nv_bfloat16*>(a.k);
-      sp.stride_b = a.k_stride[0]; sp.stride_h = a.k_stride[1]; sp.stride_s = a.k_stride[2];
-      sp.kept_tok = kept_k; sp.dropped_tok = nullptr;
+      sp = select_params(pl, a.k, a.k_stride, a.batch, nh);
+      sp.head_list = heads_c; sp.kept_tok = kept_k;
       if ((rc = launch_coreset_select(sp, stream)) != VB_OK) return rc;
       ++g_launches;
     }
@@ -924,43 +935,28 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
     GatherParams gp;
     memset(&gp, 0, sizeof(gp));
     gp.dst_stride[0] = nh * rows * kHeadDim; gp.dst_stride[1] = rows * kHeadDim; gp.dst_stride[2] = kHeadDim;
-    gp.map_stride_b = nh * rows; gp.map_stride_h = rows;
+    gp.map = kept_q; gp.map_stride_b = nh * rows; gp.map_stride_h = rows;
     gp.head_list = heads_c; gp.batch = a.batch; gp.heads = nh; gp.n_rows = static_cast<int32_t>(rows);
     if (!kv_from_k) {
-      gp.n_tensors = 3; gp.map = kept_q;
-      gp.src[0] = static_cast<const __nv_bfloat16*>(a.q); gp.dst[0] = pq;
-      gp.src[1] = static_cast<const __nv_bfloat16*>(a.k); gp.dst[1] = pk;
-      gp.src[2] = static_cast<const __nv_bfloat16*>(a.v); gp.dst[2] = pv;
-      for (int i = 0; i < 3; ++i) {
-        gp.src_stride[0][i] = a.q_stride[i]; gp.src_stride[1][i] = a.k_stride[i]; gp.src_stride[2][i] = a.v_stride[i];
-      }
+      gather_from_args(gp, a, 0, 3, pooled);
       if ((rc = launch_gather_rows(gp, stream)) != VB_OK) return rc;
       ++g_launches;
     } else {
-      gp.n_tensors = 1; gp.map = kept_q;
-      gp.src[0] = static_cast<const __nv_bfloat16*>(a.q); gp.dst[0] = pq;
-      for (int i = 0; i < 3; ++i) gp.src_stride[0][i] = a.q_stride[i];
+      gather_from_args(gp, a, 0, 1, pooled);
       if ((rc = launch_gather_rows(gp, stream)) != VB_OK) return rc;
-      gp.n_tensors = 2; gp.map = kept_k;
-      gp.src[0] = static_cast<const __nv_bfloat16*>(a.k); gp.dst[0] = pk;
-      gp.src[1] = static_cast<const __nv_bfloat16*>(a.v); gp.dst[1] = pv;
-      for (int i = 0; i < 3; ++i) { gp.src_stride[0][i] = a.k_stride[i]; gp.src_stride[1][i] = a.v_stride[i]; }
+      gp.map = kept_k;
+      gather_from_args(gp, a, 1, 2, pooled);
       if ((rc = launch_gather_rows(gp, stream)) != VB_OK) return rc;
       g_launches += 2;
     }
-    BranchLaunch bl;
-    memset(&bl, 0, sizeof(bl));
-    bl.q = pq; bl.k = pk; bl.v = pv;
-    const int64_t st[3] = {nh * rows * kHeadDim, rows * kHeadDim, kHeadDim};
-    for (int i = 0; i < 3; ++i) { bl.qs[i] = st[i]; bl.ks[i] = st[i]; bl.vs[i] = st[i]; }
-    bl.n_rows_q = pl->S_c + TV; bl.n_rows_kv = pl->S_c + TV; bl.n_heads_tensor = nh;
-    bl.sched = &pl->coreset;
-    bl.out_map = kept_q; bl.out_map_stride_b = nh * rows; bl.out_map_stride_h = rows;
+    Segment sg = workspace_segment(pooled, nh, rows, pl->S_c + TV, pl->coreset);
+    sg.heads = head_entries(hs, true);
+    sg.out_map = kept_q; sg.out_map_stride_b = nh * rows; sg.out_map_stride_h = rows;
     if (pl->n_p > 0) {   // dropped margins receive their centre's output (coreset_select.py:157)
-      bl.bcast_map = drop_q; bl.bcast_stride_b = static_cast<int64_t>(nh) * pl->G * pl->n_p;
-      bl.bcast_stride_h = static_cast<int64_t>(pl->G) * pl->n_p; bl.bcast_rows = pl->G; bl.bcast_n = pl->n_p;
+      sg.bcast_map = drop_q; sg.bcast_stride_b = static_cast<int64_t>(nh) * pl->G * pl->n_p;
+      sg.bcast_stride_h = static_cast<int64_t>(pl->G) * pl->n_p; sg.bcast_rows = pl->G; sg.bcast_n = pl->n_p;
     }
-    if ((rc = for_batches(bl, hs, 1, true)) != VB_OK) return rc;
+    segs.push_back(std::move(sg));
   }
 
   // ---------------- branch 2: sliding tile ----------------
@@ -972,41 +968,46 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
     NvtxRange nvtx("vb: sliding tile-major layout");
     const int64_t rows = N;
     const int64_t bh = static_cast<int64_t>(a.batch) * nh;
-    __nv_bfloat16* tq = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
-    __nv_bfloat16* tk = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
-    __nv_bfloat16* tv = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
+    __nv_bfloat16* tiled[3];
+    for (__nv_bfloat16*& t : tiled) t = static_cast<__nv_bfloat16*>(ws.take(bh * rows * kHeadDim * 2));
     HeadList heads_s;
     if ((rc = head_list_of(hs, &heads_s)) != VB_OK) return rc;
-    VB_REQUIRE(tq && tk && tv, VB_ERR_INVALID, "workspace exhausted");
+    VB_REQUIRE(tiled[0] && tiled[1] && tiled[2], VB_ERR_INVALID, "workspace exhausted");
     GatherParams gp;
     memset(&gp, 0, sizeof(gp));
-    gp.n_tensors = 3; gp.map = pl->d_tile_map; gp.map0 = pl->d_query_map; gp.map_stride_b = 0; gp.map_stride_h = 0;
-    gp.src[0] = static_cast<const __nv_bfloat16*>(a.q); gp.dst[0] = tq;
-    gp.src[1] = static_cast<const __nv_bfloat16*>(a.k); gp.dst[1] = tk;
-    gp.src[2] = static_cast<const __nv_bfloat16*>(a.v); gp.dst[2] = tv;
-    for (int i = 0; i < 3; ++i) {
-      gp.src_stride[0][i] = a.q_stride[i]; gp.src_stride[1][i] = a.k_stride[i]; gp.src_stride[2][i] = a.v_stride[i];
-    }
+    gp.map = pl->d_tile_map; gp.map0 = pl->d_query_map; gp.map_stride_b = 0; gp.map_stride_h = 0;
+    gather_from_args(gp, a, 0, 3, tiled);
     gp.dst_stride[0] = nh * rows * kHeadDim; gp.dst_stride[1] = rows * kHeadDim; gp.dst_stride[2] = kHeadDim;
     gp.head_list = heads_s; gp.batch = a.batch; gp.heads = nh; gp.n_rows = static_cast<int32_t>(rows);
     if ((rc = launch_gather_rows(gp, stream)) != VB_OK) return rc;
     ++g_launches;
-    BranchLaunch bl;
-    memset(&bl, 0, sizeof(bl));
-    bl.q = tq; bl.k = tk; bl.v = tv;
-    const int64_t st[3] = {nh * rows * kHeadDim, rows * kHeadDim, kHeadDim};
-    for (int i = 0; i < 3; ++i) { bl.qs[i] = st[i]; bl.ks[i] = st[i]; bl.vs[i] = st[i]; }
-    bl.n_rows_q = S + TV; bl.n_rows_kv = S + TV; bl.n_heads_tensor = nh;
-    bl.sched = &pl->sliding;
-    bl.out_map = pl->d_query_map; bl.out_map_stride_b = 0; bl.out_map_stride_h = 0;
-    if ((rc = for_batches(bl, hs, 2, true)) != VB_OK) return rc;
+    Segment sg = workspace_segment(tiled, nh, rows, S + TV, pl->sliding);
+    sg.heads = head_entries(hs, true);
+    sg.out_map = pl->d_query_map;
+    segs.push_back(std::move(sg));
   }
 
-  if (n_deferred > 0) {
+  Output out;
+  memset(&out, 0, sizeof(out));
+  out.ptr = static_cast<__nv_bfloat16*>(a.out);
+  for (int i = 0; i < 3; ++i) out.stride[i] = a.out_stride[i];
+  for (int i = 0; i < a.out_peer_count; ++i) out.peers[i] = static_cast<__nv_bfloat16*>(a.out_peer_ptrs[i]);
+  out.peer_count = a.out_peer_count;
+  out.peer_rows = a.out_peer_rows;
+  if (merge) {
     NvtxRange nvtx("vb: attention launch (full + coreset + sliding segments)");
-    const Segment* order[kMaxSegments];
-    for (int i = 0; i < n_deferred; ++i) order[i] = &deferred[i];
-    if ((rc = launch_segments(order, n_deferred, a, 0, a.batch, stream)) != VB_OK) return rc;
+    rc = launch_segments(segs.data(), static_cast<int>(segs.size()), a.batch, out, a.debug, nullptr, VB_TIMING_ROUTED,
+                         stream);
+    if (rc != VB_OK) return rc;
+  } else {
+    // one branch at a time.  Blend: segment e is branch e, stage e + 1 of the fp32 accumulation; ONE launch covers every
+    // batch element (the scores are read per (batch, head) from the device table)
+    for (size_t e = 0; e < segs.size(); ++e) {
+      blend_state.stage = static_cast<int>(e) + 1;
+      blend_state.branch = static_cast<int>(e);
+      rc = launch_segments(&segs[e], 1, a.batch, out, a.debug, blend ? &blend_state : nullptr, VB_TIMING_ROUTED, stream);
+      if (rc != VB_OK) return rc;
+    }
   }
 
   // ---------------- padded text queries produce zeros (hunyuan.py:176; flex fully-masked rows) ----------------
@@ -1046,25 +1047,14 @@ int vb_attn_dense(const void* q, const void* k, const void* v, void* out, const 
     }
     cache.push_back({DenseKey{dev, n_q, n_k}, sched});
   }
-  vb_attn_args a;
-  memset(&a, 0, sizeof(a));
-  a.out = out; a.batch = batch; a.heads = heads;
-  for (int i = 0; i < 3; ++i) a.out_stride[i] = out_stride[i];
-  BranchLaunch bl;
-  memset(&bl, 0, sizeof(bl));
-  bl.q = static_cast<const __nv_bfloat16*>(q);
-  bl.k = static_cast<const __nv_bfloat16*>(k);
-  bl.v = static_cast<const __nv_bfloat16*>(v);
-  for (int i = 0; i < 3; ++i) { bl.qs[i] = q_stride[i]; bl.ks[i] = k_stride[i]; bl.vs[i] = v_stride[i]; }
-  bl.n_rows_q = n_q; bl.n_rows_kv = n_k; bl.n_heads_tensor = heads;
-  bl.sched = sched;
-  std::vector<AttnHead> hs(heads);
-  for (int h = 0; h < heads; ++h) hs[h] = AttnHead{h, h, 1.f, 0};
+  Output o;
+  memset(&o, 0, sizeof(o));
+  o.ptr = static_cast<__nv_bfloat16*>(out);
+  for (int i = 0; i < 3; ++i) o.stride[i] = out_stride[i];
+  Segment sg = segment_of(q, k, v, q_stride, k_stride, v_stride, n_q, n_k, heads, *sched);
+  for (int h = 0; h < heads; ++h) sg.heads.push_back(AttnHead{h, h, 0});
   NvtxRange nvtx("vb_attn_dense");
-  g_launch_kind = VB_TIMING_DENSE;
-  const int rc = run_branch(bl, a, hs, 0, batch, static_cast<cudaStream_t>(stream_));
-  g_launch_kind = VB_TIMING_ROUTED;
-  return rc;
+  return launch_segments(&sg, 1, batch, o, nullptr, nullptr, VB_TIMING_DENSE, static_cast<cudaStream_t>(stream_));
 }
 
 int vb_block_ln_modulate(const void* x, const float* weight, const float* bias, const float* scale, const float* shift,

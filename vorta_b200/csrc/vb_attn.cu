@@ -132,7 +132,7 @@ __device__ __forceinline__ Item decode_item(const AttnParams& p, int item) {
   dst[1] = __ldg(src + 1);
   dst[2] = __ldg(src + 2);
   it.head = p.heads[seg.head0 + (local / seg.n_pairs) % seg.n_heads];
-  it.batch = local / (seg.n_pairs * seg.n_heads) + p.batch0;
+  it.batch = local / (seg.n_pairs * seg.n_heads);
   return it;
 }
 
@@ -564,7 +564,7 @@ vb_attn_fwd_kernel(const __grid_constant__ AttnTmaps tmaps, const __grid_constan
       const bool row_ok = row < pair.q_rows[t];
       const int krow = pair.q_row0[t] + row;      // row in kernel order
       const int stage = p.blend_stage;
-      const float w_head = stage == 0 ? head.weight
+      const float w_head = stage == 0 ? 1.f
                                       : __ldg(p.blend_w + (static_cast<int64_t>(batch) * p.blend_heads + head.wi) * 3 +
                                               p.blend_branch);
       const float inv = w_head / l_sum;

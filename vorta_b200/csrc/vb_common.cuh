@@ -63,8 +63,7 @@ struct KvRun {
 struct AttnHead {
   int32_t hk;       // head coordinate inside the Q/K/V tensor maps
   int32_t ho;       // head index in the output tensor
-  float weight;     // epilogue scale in top-1 mode (1); blend mode reads AttnParams::blend_w instead
-  int32_t wi;       // blend mode: head index into AttnParams::blend_w
+  int32_t wi;       // blend mode: head index into AttnParams::blend_w (top-1 mode scales by 1)
 };
 
 // One branch of a layer inside an attention launch: its own work table, Q/K/V tensor maps (AttnTmaps::m[i]) and row
@@ -96,7 +95,6 @@ struct AttnParams {
   int32_t n_items;              // work items of the launch (all segments)
   unsigned int* work_counter;   // device counter handing out items beyond the first gridDim.x; 0 before and after a launch
   int32_t n_seg;
-  int32_t batch0;               // batch index of the first batch slice (blend mode launches one batch at a time)
   // Blend (Train) mode, out = sum_e w[b,h,e] * O_e (wan.py:296-300): the three branches run as three launches, stage =
   // 1, 2, 3.  Stage 1 stores w * O in fp32 into blend_acc, stage 2 adds to it, stage 3 adds and writes the bf16 output, so
   // the sum is formed in fp32 and rounded once.  blend_w: device (batch, blend_heads, 3) fp32 routing scores.

@@ -1,6 +1,10 @@
 """Multi-GPU parity check, launched by torchrun (one rank per GPU): the Ulysses-parallel processors must reproduce
 the single-GPU result (the N-GPU == 1-GPU contract of SURVEY.md section 5).  Prints one line per case; exits
-non-zero on a mismatch.  Driven by tests/test_multigpu.py."""
+non-zero on a mismatch.  Driven by tests/test_multigpu.py.
+
+Usage: mgpu_check.py [MODE].  MODE "peer-split" forces query-half units at every world size, a MODE ending in
+"-contiguous" keeps the reference's contiguous head chunks on the NCCL path; the exchange itself is chosen by the
+VB_ULYSSES environment variable."""
 import os
 import sys
 
@@ -11,10 +15,15 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import fixtures as FX  # noqa: E402
 from vorta_b200.attention import (HunyuanVideoFlashAttnProcessorTripleEval, WanAttnProcessorTripleEval,  # noqa: E402
                                   WanAttnProcessorTripleTrain, get_group_info)
-from vorta_b200.ulysses import SP_STATE, all_gather  # noqa: E402
+from vorta_b200.ulysses import SP_STATE, all_gather, balance, peer  # noqa: E402
 
 
 def main():
+    mode = sys.argv[1] if len(sys.argv) > 1 else "peer"
+    if mode == "peer-split":
+        balance.split_enabled = lambda world: True
+    if mode.endswith("-contiguous"):
+        balance.balance_heads = lambda branch, costs, world: None
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -112,14 +121,13 @@ def main():
         v, t = hev(hattn, mine, ehs, mask, rope, routing_score=score, tau_sparse=0.3, **kw)
         check("hunyuan single-stream eval (video)", all_gather(v, dim=1), ref_v)
         check("hunyuan single-stream eval (text)", t, ref_t)
-    from vorta_b200.ulysses import balance, peer
     from vorta_b200.attention.wan import _top1_branches
     if rank == 0:
         br = _top1_branches(score, 0.3)
         placed = balance.place_units(br, [6.0, 1.6, 1.0], world, balance.max_slots(H, world),
                                      allow_split=balance.split_enabled(world))
-        print("exchange:", os.environ.get("VB_ULYSSES", "peer"), "| peer disabled reason:", peer.disabled_reason(),
-              "| peer exchanges built:", len(peer._EXCHANGES), "| head balancing:", balance.enabled(),
+        print("mode:", mode, "| exchange:", os.environ.get("VB_ULYSSES", "peer"), "| peer disabled reason:",
+              peer.disabled_reason(), "| peer exchanges built:", len(peer._EXCHANGES),
               "| branches:", br, "| units per rank (head, part):", placed, flush=True)
     dist.barrier()
     dist.destroy_process_group()

@@ -344,13 +344,12 @@ def test_sliding_work_items_cover_every_query_once_with_its_window(lat, tile, wi
     assert n_slots <= plan.num_tiles * -(-tau // 128) + (-(-tv // 128) if tv else 0)
 
 
-def test_placement_with_query_half_units(monkeypatch):
+def test_placement_with_query_half_units():
     """balance.place_units: deterministic; every head is held exactly once — whole, or as a lower and an upper query
     half (full-attention heads only); at most `slots` units per rank; never worse than the whole-head placement, and
     clearly better where a rank holds only a few heads (HunyuanVideo: 24 heads on 8 ranks)."""
     import random
     from vorta_b200.ulysses import balance
-    monkeypatch.setenv("VB_ULYSSES_SPLIT_WAYS", "2,4")        # exercise halves and quarters (default: halves)
     costs = [6.5, 1.8, 1.25]
     rnd = random.Random(3)
     gain = []
@@ -370,7 +369,7 @@ def test_placement_with_query_half_units(monkeypatch):
                 if parts == [balance.WHOLE]:
                     continue
                 n = balance.part_kn(parts[0])[1]           # a split head: every part k of n exactly once
-                assert branch[h] == 0 and n in (2, 4)
+                assert branch[h] == 0 and n == 2
                 assert sorted(parts) == [balance.part_code(k, n) for k in range(n)]
 
             def load(p):
@@ -382,3 +381,35 @@ def test_placement_with_query_half_units(monkeypatch):
             if (H, P) == (24, 8):
                 gain.append(load(whole) / load(placed))
     assert max(gain) > 1.04 and min(gain) >= 1.0
+
+
+_PLACEMENT_PLANS = {          # the bench workloads' geometries (bench.py WORKLOADS)
+    "wan14": dict(latent_shape=(21, 45, 80), tile_size=(3, 9, 16), window_size=(3, 3, 3),
+                  lowres_window_size=(3, 3, 2)),
+    "hunyuan": dict(latent_shape=(33, 45, 80), tile_size=(3, 9, 16), window_size=(3, 3, 3),
+                    lowres_window_size=(3, 3, 2), text_len=256, text_valid=64),
+}
+
+
+def test_ulysses_placements_match_recorded_answers():
+    """Which rank computes which head, pinned: the NCCL head table (balance_heads), the peer-memory unit table
+    (layer_placement) and every rank's (branch ids, out_heads) for vb_attn_fwd, recorded from the placement code before
+    the two processors shared one dispatch.  Bench routing (7h+1)%3 and three seeded random routings; Wan-14B (40 heads,
+    P = 2, 4, 8) and HunyuanVideo (24 heads, P = 8) with the branch costs of the real plans."""
+    import json
+    import os
+    from vorta_b200.ulysses import balance
+    from vorta_b200.ulysses.routed import local_units
+    with open(os.path.join(os.path.dirname(__file__), "golden", "ulysses_placements.json")) as f:
+        cases = json.load(f)["cases"]
+    plans = {name: ops.Plan(**geometry) for name, geometry in _PLACEMENT_PLANS.items()}
+    for c in cases:
+        plan, branch, P, slots = plans[c["workload"]], c["branch"], c["world"], c["slots"]
+        what = (c["workload"], P, c["routing"])
+        assert balance.branch_costs(plan) == c["costs"], what
+        assert balance.max_slots(len(branch), P) == slots, what
+        assert balance.balance_heads(branch, c["costs"], P) == c["head_at"], what
+        placement = balance.layer_placement(branch, plan, P, slots)
+        assert [[list(u) for u in units] for units in placement] == c["placement"], what
+        for r, want in enumerate(c["local_units"]):
+            assert local_units(placement, r, branch, slots) == (want["ids"], want["out_heads"]), (what, r)

@@ -24,6 +24,12 @@ BRANCH_FULL_LO, BRANCH_FULL_HI = 3, 4          # full attention over the lower /
 DTYPE_F32, DTYPE_BF16 = 0, 1
 ATTN_CORESET_KV_FROM_K = 1
 
+
+def branch_full_part(k: int, n: int) -> int:
+    """VB_BRANCH_FULL_PART(k, n): full attention over part k of n equal parts of the query work items."""
+    return 16 + 8 * n + k
+
+
 # vb_plan_query keys
 (PLAN_SEQ_LEN, PLAN_NUM_GROUPS, PLAN_GROUP_SIZE, PLAN_CORESET_LEN, PLAN_NUM_TILES, PLAN_TILE_TOKENS,
  PLAN_NUM_POOLED, PLAN_KEYS_PER_QUERY, PLAN_SLIDING_PAIRS, PLAN_SLIDING_RUNS) = range(10)

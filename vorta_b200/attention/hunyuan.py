@@ -14,8 +14,8 @@ import torch
 
 from .. import _lib as L
 from .. import ops
-from ..ulysses import SP_STATE, all_gather, balance, exchange_out, exchange_qkv, local_heads, shrink_dim
-from ..ulysses.peer import get_exchange, layer_placement, local_units
+from ..ulysses import SP_STATE, shrink_dim
+from ..ulysses.routed import routed_attention
 from ._plans import get_plan, infer_lowres_window
 from .coreset_select import LowresGroupInfo
 from .wan import _top1_branches
@@ -125,52 +125,9 @@ class HunyuanVideoFlashAttnProcessor:
         """[video | text] joint attention for every branch in one C-ABI call; returns (video, text) outputs.
         Under Ulysses the video part is exchanged (once for all branches), each rank keeps its head slice of the
         replicated text tokens and the text outputs are all-gathered over heads (hunyuan.py:147-164,184-187)."""
-        B, H = query.shape[:2]
+        B = query.shape[0]
         assert B == 1, f"Batch size {B} is not supported for {self.__class__.__name__}."        # hunyuan.py:168
-        head_at = None
-        if SP_STATE.enabled:
-            P, r = SP_STATE.sp_size, SP_STATE.group_local_rank
-            hp = H // P
-            ex = get_exchange(H, query.shape[2] - text_len, query.device, text_len) if weights is None else None
-            if ex is not None:
-                # NVLink peer-memory path (top-1 routing): video rows of Q / K / V are stored straight into the buffers
-                # of the ranks that own the head (or a query half of it), the text rows of this rank's heads are copied
-                # locally, and the attention epilogue stores video rows to the token owner and text rows to every rank
-                placement = layer_placement(branch, plan, H, P, ex.slots)
-                parts = [(t[:, :, :-text_len], t[:, :, -text_len:]) for t in (query, key, value)]
-                q, k, v = ex.scatter_qkv(*[p_[0] for p_ in parts], placement, text=[p_[1] for p_ in parts])
-                ex.zero_padded_text(plan.text_valid)
-                ids, out_heads = local_units(placement, r, branch, ex.slots)
-                ops.routed_attention(plan, q, k, v, branch=ids, flags=flags, out_peers=ex.out_ptrs,
-                                     out_peer_rows=ex.s_loc, out_peer_strides=(0, 128, H * 128), out_heads=out_heads)
-                out = ex.finish_out()
-                return out[:, :, :-text_len], out[:, :, -text_len:]
-            if branch is not None and balance.enabled():      # cost-balanced head placement (SURVEY.md section 8e)
-                head_at = balance.balance_heads(list(branch), balance.branch_costs(plan), P)
-            qv, kv, vv = exchange_qkv(query[:, :, :-text_len], key[:, :, :-text_len], value[:, :, :-text_len],
-                                      extra_rows=text_len, head_at=head_at)
-            mine = None
-            if head_at is not None:
-                mine = torch.tensor(head_at[r * hp:(r + 1) * hp], device=query.device)
-            for full, src in ((qv, query), (kv, key), (vv, value)):
-                # replicated text tokens: this rank's heads (hunyuan.py:151-153 shrink_dim over heads)
-                full[:, :, -text_len:] = (shrink_dim(src[:, :, -text_len:], dim=1) if mine is None
-                                          else src[:, :, -text_len:].index_select(1, mine))
-            query, key, value = qv, kv, vv
-            if branch is not None:
-                branch = local_heads(list(branch), H, head_at)
-            if weights is not None:
-                weights = shrink_dim(weights, dim=1)
-        out = ops.routed_attention(plan, query, key, value, branch=branch, weights=weights, flags=flags)
-        video, text = out[:, :, :-text_len], out[:, :, -text_len:]
-        if SP_STATE.enabled:
-            video = exchange_out(video, head_at)
-            text = all_gather(text.contiguous(), dim=1)
-            if head_at is not None:       # gathered in slot order: put every head back at its own index
-                inverse = torch.empty(H, dtype=torch.long)
-                inverse[torch.tensor(head_at)] = torch.arange(H)
-                text = text.index_select(1, inverse.to(text.device))
-        return video, text
+        return routed_attention(plan, query, key, value, branch=branch, weights=weights, flags=flags, text_len=text_len)
 
     def _step_attention(self, query, key, value, attention_mask, encoder_hidden_states_seq_len: int,
                         skip_communication: bool = False, text_valid: Optional[int] = None

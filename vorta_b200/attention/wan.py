@@ -20,8 +20,8 @@ import torch
 
 from .. import _lib as L
 from .. import ops
-from ..ulysses import SP_STATE, balance, exchange_out, exchange_qkv, local_heads, shrink_dim
-from ..ulysses.peer import get_exchange, layer_placement, local_units
+from ..ulysses import SP_STATE, exchange_out, exchange_qkv, shrink_dim
+from ..ulysses.routed import routed_attention
 from ._plans import get_plan, infer_lowres_window
 from .coreset_select import LowresGroupInfo
 
@@ -170,35 +170,7 @@ class WanAttnProcessorTripleTrain(WanAttnProcessor2_0):
 
     def _routed_attention(self, query, key, value, plan: ops.Plan, branch=None, weights=None) -> torch.Tensor:
         """All branches of one layer: a single C-ABI call between the two Ulysses exchanges."""
-        heads = query.shape[1]
-        if not SP_STATE.enabled:
-            return ops.routed_attention(plan, query, key, value, branch=branch, weights=weights)
-        hp = heads // SP_STATE.sp_size
-        r = SP_STATE.group_local_rank
-        ex = get_exchange(heads, query.shape[2], query.device) if (weights is None and query.shape[0] == 1) else None
-        if ex is not None:
-            # NVLink peer-memory path: Q/K/V rows are stored straight into the buffers of the ranks that own the head
-            # (or a query half of it), and the attention epilogue stores every output row straight into the buffer of
-            # the rank that owns the token.  The routing of the layer is known on every rank, so all ranks derive the
-            # same cost-balanced placement (SURVEY.md section 8e); results stay bit-identical to one GPU.
-            placement = layer_placement(branch, plan, heads, SP_STATE.sp_size, ex.slots)
-            q, k, v = ex.scatter_qkv(query, key, value, placement)
-            ids, out_heads = local_units(placement, r, branch, ex.slots)
-            ops.routed_attention(plan, q, k, v, branch=ids, out_peers=ex.out_ptrs, out_peer_rows=ex.s_loc,
-                                 out_peer_strides=(0, 128, heads * 128), out_heads=out_heads)
-            return ex.finish_out()
-        head_at = None
-        if branch is not None:
-            # the routing of the layer is known on every rank: hand each rank a cost-balanced set of heads instead
-            # of the contiguous chunk (SURVEY.md section 8e); only slot numbers inside the exchange change
-            if balance.enabled():
-                head_at = balance.balance_heads(list(branch), balance.branch_costs(plan), SP_STATE.sp_size)
-            branch = local_heads(list(branch), heads, head_at)
-        if weights is not None:
-            weights = weights[:, r * hp:(r + 1) * hp]
-        query, key, value = exchange_qkv(query, key, value, head_at=head_at)
-        out = ops.routed_attention(plan, query, key, value, branch=branch, weights=weights)
-        return exchange_out(out, head_at)
+        return routed_attention(plan, query, key, value, branch=branch, weights=weights)[0]
 
     def __call__(self, attn, hidden_states: torch.Tensor, encoder_hidden_states: Optional[torch.Tensor] = None,
                  attention_mask: Optional[torch.Tensor] = None, rotary_emb: Optional[torch.Tensor] = None,

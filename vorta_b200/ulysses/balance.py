@@ -7,13 +7,14 @@ picks, per layer, which H/P heads each rank receives.  The choice only changes s
 buffers (``head_at`` of ``vb_ulysses_*``; ``out_heads`` of ``vb_attn_fwd``): no extra bytes move, and results are
 bit-identical to the contiguous placement because heads are independent.
 
-``balance_heads`` is deterministic and depends only on (branch ids, costs, P): every rank derives the same table
-from its own copy of the routing decisions.
+Every placement is deterministic and depends only on (branch ids, costs, P): every rank derives the same table
+from its own copy of the routing decisions.  ``balance_heads`` places whole heads, H/P per rank, for the NCCL
+exchange; ``layer_placement`` places work units (whole heads and query halves) for the peer-memory exchange.  Both
+run the same greedy ``_place``.
 """
 from __future__ import annotations
 
 import functools
-import os
 from typing import List, Optional, Sequence
 
 # measured time per algorithmic FLOP relative to the full branch, layout / selection passes included
@@ -22,16 +23,13 @@ from typing import List, Optional, Sequence
 _BRANCH_OVERHEAD = (1.0, 1.06, 1.33)
 
 
-def enabled() -> bool:
-    return os.environ.get("VB_ULYSSES_BALANCE", "1") != "0"
-
-
 def branch_costs(plan) -> List[float]:
-    """Relative cost of one head of each branch for this geometry (algorithmic FLOPs x measured overhead;
-    VB_ULYSSES_COSTS="1.0,1.12,1.25" overrides the overheads for experiments)."""
-    env = os.environ.get("VB_ULYSSES_COSTS")
-    over = tuple(float(x) for x in env.split(",")) if env else _BRANCH_OVERHEAD
-    return [plan.flops_per_head(e) * over[e] for e in range(3)]
+    """Relative cost of one head of each branch for this geometry (algorithmic FLOPs x measured overhead)."""
+    return [plan.flops_per_head(e) * _BRANCH_OVERHEAD[e] for e in range(3)]
+
+
+def _head_costs(branch: Sequence[int], costs: Sequence[float]) -> List[float]:
+    return [costs[e] if 0 <= e < len(costs) else 0.0 for e in branch]
 
 
 def balance_heads(branch: Sequence[int], costs: Sequence[float], world: int) -> Optional[List[int]]:
@@ -43,22 +41,17 @@ def balance_heads(branch: Sequence[int], costs: Sequence[float], world: int) -> 
     if world <= 1 or H % world != 0:
         return None
     hp = H // world
-    cost = [float(costs[int(e)]) if 0 <= int(e) < len(costs) else 0.0 for e in branch]
+    branch, costs = tuple(int(e) for e in branch), tuple(float(c) for c in costs)
+    held, load = _place(branch, costs, world, hp, False)
+    cost = _head_costs(branch, costs)
     contiguous = max(sum(cost[r * hp:(r + 1) * hp]) for r in range(world))
-    order = sorted(range(H), key=lambda h: (-cost[h], h))
-    load = [0.0] * world
-    held: List[List[int]] = [[] for _ in range(world)]
-    for h in order:
-        r = min((r for r in range(world) if len(held[r]) < hp), key=lambda r: (load[r], r))
-        held[r].append(h)
-        load[r] += cost[h]
-    if max(load) >= contiguous * (1.0 - 1e-9):
+    if load >= contiguous * (1.0 - 1e-9):
         return None
-    return [h for r in range(world) for h in sorted(held[r])]
+    return [h for units in held for h, _ in units]
 
 
 # ------------------------------------------------------------------------------------------------------------------
-# Placement with work units finer than a head (peer-memory exchange only)
+# Placement in work units: whole heads, and query halves of full heads (peer-memory exchange only)
 # ------------------------------------------------------------------------------------------------------------------
 WHOLE = 0                              # part of a head a slot computes: all of its query work items, or
 
@@ -76,19 +69,9 @@ LOWER, UPPER = part_code(0, 2), part_code(1, 2)
 _SPLIT_OVERHEAD = 1.03                 # a part costs a little more than its share (another copy of K / V crosses NVLink)
 
 
-def _split_ways():
-    """n-way splits place_units may use: VB_ULYSSES_SPLIT_WAYS="2" (halves only, default) or "2,4" (halves and quarters;
-    measured equal within noise at Wan-14B P = 8, profiles/r2r_scale_n8_placement_ab.log)."""
-    env = os.environ.get("VB_ULYSSES_SPLIT_WAYS", "2")
-    return tuple(int(x) for x in env.split(",") if x.strip())
-
-
 def split_enabled(world: int) -> bool:
     """Query-half units pay off when a rank holds only a few heads (3 at HunyuanVideo P = 8, 5 at Wan-14B P = 8: one full
-    head is 20-40 % of a rank's layer time); VB_ULYSSES_SPLIT=0 / 1 overrides."""
-    env = os.environ.get("VB_ULYSSES_SPLIT")
-    if env is not None:
-        return env != "0"
+    head is 20-40 % of a rank's layer time)."""
     return world >= 4
 
 
@@ -102,18 +85,26 @@ def place_units(branch: Sequence[int], costs: Sequence[float], world: int, slots
                 ) -> List[List[tuple]]:
     """Greedy longest-processing-time placement of a layer's heads on ``world`` ranks with at most ``slots`` units per
     rank.  A unit is (head, part): a whole head, or — for full-attention heads, when that lowers the slowest rank's
-    load — one half or quarter of its query work items (``part_code``; the parts may land on different ranks, each
+    load — one query half of its work items (``LOWER`` / ``UPPER``; the halves may land on different ranks, each
     receives the head's K / V).
     Deterministic in (branch, costs, world, slots): every rank computes the same table.  Returns, per rank, its units
     in slot order.  Results are cached per routing (the same decisions recur across steps and CFG passes)."""
-    return [list(u) for u in _place_cached(tuple(int(e) for e in branch), tuple(float(c) for c in costs), int(world),
-                                           int(slots), bool(allow_split), _split_ways())]
+    placed, _ = _place(tuple(int(e) for e in branch), tuple(float(c) for c in costs), int(world), int(slots),
+                       bool(allow_split))
+    return [list(u) for u in placed]
+
+
+def layer_placement(branch: Sequence[int], plan, world: int, slots: int) -> List[List[tuple]]:
+    """Placement of one layer's heads for the peer exchange: cost-balanced units, with query halves of full heads from
+    4 ranks up."""
+    return place_units(branch, branch_costs(plan), world, slots, allow_split=split_enabled(world))
 
 
 @functools.lru_cache(maxsize=4096)
-def _place_cached(branch: tuple, costs: tuple, world: int, slots: int, allow_split: bool, ways: tuple):
+def _place(branch: tuple, costs: tuple, world: int, slots: int, allow_split: bool):
+    """-> (units of every rank, ascending, the largest load of a rank)."""
     H = len(branch)
-    cost = [costs[e] if 0 <= e < len(costs) else 0.0 for e in branch]
+    cost = _head_costs(branch, costs)
 
     def lpt(units):           # units sorted by (-cost, head, part)
         load = [0.0] * world
@@ -137,20 +128,19 @@ def _place_cached(branch: tuple, costs: tuple, world: int, slots: int, allow_spl
     whole = [(cost[h], h, WHOLE) for h in range(H)]
     best, best_load = lpt(order(whole))
     if allow_split:
-        # try splitting the k most expensive full heads n ways (one split alone often does not lower the maximum:
+        # try splitting the k most expensive full heads in halves (one split alone often does not lower the maximum:
         # several ranks tie at it); keep the candidate with the lowest maximum load, the fewest units among equals
         full = sorted((h for h in range(H) if branch[h] == 0), key=lambda h: (-cost[h], h))
         tried = sorted({k for k in (1, 2, 3, 4, 6, 8, 12, 16, 24, len(full)) if 1 <= k <= len(full)})
-        for n in ways:
-            for k in tried:
-                chosen = set(full[:k])
-                units = [u for u in whole if u[1] not in chosen]
-                for h in full[:k]:
-                    share = cost[h] / n * _SPLIT_OVERHEAD
-                    units += [(share, h, part_code(i, n)) for i in range(n)]
-                placed, load = lpt(order(units))
-                if placed is not None and load < best_load * (1.0 - 1e-3):
-                    best, best_load = placed, load
+        for k in tried:
+            chosen = set(full[:k])
+            units = [u for u in whole if u[1] not in chosen]
+            for h in full[:k]:
+                share = cost[h] / 2 * _SPLIT_OVERHEAD
+                units += [(share, h, LOWER), (share, h, UPPER)]
+            placed, load = lpt(order(units))
+            if placed is not None and load < best_load * (1.0 - 1e-3):
+                best, best_load = placed, load
     if best is None:
         raise ValueError(f"{H} heads do not fit {world} ranks x {slots} slots")
-    return tuple(tuple(sorted(u)) for u in best)
+    return tuple(tuple(sorted(u)) for u in best), best_load

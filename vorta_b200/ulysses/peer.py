@@ -95,11 +95,11 @@ class PeerExchange:
                     placement: Sequence[Sequence[Tuple[int, int]]], text: Optional[Sequence[torch.Tensor]] = None
                     ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
         """q, k, v: (1, H, S_loc, 128) views of this rank's token shard.  ``placement[p]`` = the (head, part) units of
-        rank p in slot order (``balance.place_units`` or ``contiguous_placement``); every head of a unit is stored into
-        that slot of rank p's buffer — a head split into query parts goes to several ranks.  Returns (1, slots, S + T, 128)
-        views of the local receive buffer, valid after barrier A (issued here); only the first len(placement[rank])
-        slots hold data.  ``text``: the replicated (1, H, T, 128) text rows of q, k, v; the rows of this rank's heads are
-        copied behind the video rows locally (no traffic)."""
+        rank p in slot order (``balance.layer_placement``); every head of a unit is stored into that slot of rank p's
+        buffer — a head split into query parts goes to several ranks.  Returns (1, slots, S + T, 128) views of the
+        local receive buffer, valid after barrier A (issued here); only the first len(placement[rank]) slots hold data.
+        ``text``: the replicated (1, H, T, 128) text rows of q, k, v; the rows of this rank's heads are copied behind
+        the video rows locally (no traffic)."""
         self._scatter([q, k, v], self._tables(placement))
         if self.text_len:
             mine = [h for h, _ in placement[self.rank]]
@@ -145,38 +145,6 @@ def get_exchange(heads: int, s_loc: int, device: torch.device, text_len: int = 0
 
 def disabled_reason() -> Optional[str]:
     return _DISABLED_REASON
-
-
-def contiguous_placement(heads: int, world: int):
-    """The reference's chunking (vorta/ulysses/utils.py:60-66) as a placement table: rank r holds whole heads
-    [r * H / P, (r + 1) * H / P)."""
-    hp = heads // world
-    return [[(h, balance.WHOLE) for h in range(r * hp, (r + 1) * hp)] for r in range(world)]
-
-
-def layer_placement(branch: Sequence[int], plan, heads: int, world: int, slots: int):
-    """Placement of one layer's heads for the peer exchange: cost-balanced units (whole heads and, at P >= 4, query
-    halves of full heads) when balancing is on, the contiguous chunks otherwise."""
-    if branch is None or not balance.enabled():
-        return contiguous_placement(heads, world)
-    return balance.place_units(list(branch), balance.branch_costs(plan), world, slots,
-                               allow_split=balance.split_enabled(world))
-
-
-def local_units(placement, rank: int, branch: Sequence[int], slots: int):
-    """(branch id per slot, output head per slot) of this rank for ``vb_attn_fwd``: unused slots are skipped, the parts
-    of a split full head become VB_BRANCH_FULL_PART(k, n)."""
-    ids, out_heads = [], []
-    for h, part in placement[rank]:
-        e = int(branch[h])
-        if part != balance.WHOLE:
-            if e != L.BRANCH_FULL:
-                raise ValueError("only full-attention heads are split into query parts")
-            e = 16 + part                       # VB_BRANCH_FULL_PART(k, n)
-        ids.append(e)
-        out_heads.append(int(h))
-    pad = slots - len(ids)
-    return ids + [L.BRANCH_SKIP] * pad, out_heads + [0] * pad
 
 
 def nvlink_tx_bytes(reset: bool = False) -> int:

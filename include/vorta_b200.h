@@ -201,7 +201,9 @@ typedef struct {
   int32_t out_peer_rows;
   /* Optional (host pointer, heads entries, or NULL = identity): head index along `out`'s head stride that receives
    * the output of local head h.  Lets a rank that holds an arbitrary, cost-balanced subset of the layer's heads
-   * (Ulysses, SURVEY.md section 8e) write each head where the token owner expects it. */
+   * (Ulysses, SURVEY.md section 8e) write each head where the token owner expects it.  Padded text rows are zeroed in
+   * the same heads: a VB_BRANCH_SKIP slot writes nothing, and of a head split into query parts only the last part
+   * (k = n - 1) writes them, so the parts of a head own disjoint rows. */
   const int32_t* out_heads;
   /* Blend mode with the routing scores left on the device: (batch, heads, 3) fp32, same meaning as `weights`; when set,
    * `weights` is ignored and no host copy of the scores is needed (the reference blends device tensors, wan.py:296-300). */

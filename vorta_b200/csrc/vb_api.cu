@@ -46,8 +46,7 @@ static thread_local std::vector<TimedLaunch> g_events;
 int launch_coreset_select(const SelectParams& p, cudaStream_t stream);
 int launch_gather_rows(const GatherParams& p, cudaStream_t stream);
 int launch_coreset_tables(const TablesParams& p, cudaStream_t stream);
-int launch_zero_rows(__nv_bfloat16* out, int64_t sb, int64_t sh, int64_t ss, int batch, int heads, int row0,
-                     int n_rows, cudaStream_t stream);
+int launch_zero_rows(const ZeroRowsParams& p, cudaStream_t stream);
 int launch_router(const void* temb, int temb_dtype, const void* w, const void* bias, int w_dtype,
                   int64_t w_layer_stride, int64_t bias_layer_stride, int n_layers, int batch, int embed_dim,
                   int heads, float tau, float* scores, int32_t* branch, cudaStream_t stream);
@@ -647,7 +646,7 @@ struct Output {
 struct BlendState {
   const float* w;
   float* acc;
-  int stage, branch, heads;
+  int stage, branch, heads, rows;
 };
 }  // namespace
 
@@ -716,7 +715,7 @@ static int launch_segments(const Segment* segs, int n_seg, int batch, const Outp
     p.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(kHeadDim));
     if (blend != nullptr) {
       p.blend_w = blend->w; p.blend_acc = blend->acc; p.blend_stage = blend->stage;
-      p.blend_heads = blend->heads; p.blend_branch = blend->branch;
+      p.blend_heads = blend->heads; p.blend_branch = blend->branch; p.blend_rows = blend->rows;
     }
     p.dbg = dbg;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
@@ -823,15 +822,13 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
              "workspace too small: %lld < %lld bytes", (long long)a.workspace_bytes, (long long)need);
   Carver ws{static_cast<uint8_t*>(a.workspace), 0, a.workspace_bytes};
   int rc;
-  // blend mode: fp32 partial sums with the output's addressing, and the routing scores on the device
+  // blend mode: fp32 partial sums per (batch, head slot, output token), whatever the output's strides and out_heads, and
+  // the routing scores on the device
   BlendState blend_state;
   memset(&blend_state, 0, sizeof(blend_state));
   if (blend) {
     VB_REQUIRE(a.out != nullptr && a.out_peer_count == 0, VB_ERR_UNSUPPORTED, "blend mode writes a local output");
-    int64_t span = 1;       // elements covered by the output strides
-    span += (a.batch - 1) * a.out_stride[0] + (a.heads - 1) * a.out_stride[1] + (static_cast<int64_t>(N) - 1) * a.out_stride[2] +
-            (kHeadDim - 1);
-    blend_state.acc = static_cast<float*>(ws.take(span * 4));
+    blend_state.acc = static_cast<float*>(ws.take(static_cast<int64_t>(a.batch) * a.heads * N * kHeadDim * 4));
     float* w_dev = static_cast<float*>(ws.take(static_cast<int64_t>(a.batch) * a.heads * 3 * 4));
     VB_REQUIRE(blend_state.acc != nullptr && w_dev != nullptr, VB_ERR_INVALID, "workspace exhausted");
     if (a.weights_device != nullptr) {
@@ -842,6 +839,7 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
       blend_state.w = w_dev;
     }
     blend_state.heads = a.heads;
+    blend_state.rows = N;
   }
 
   // head slots of a segment over heads hs; hk is the head in the segment's q / k / v: the layer's head, or the slot of a
@@ -1011,11 +1009,32 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
   }
 
   // ---------------- padded text queries produce zeros (hunyuan.py:176; flex fully-masked rows) ----------------
+  // They belong to the output heads the slots write (out_heads): a SKIP slot owns none, and of a head split into query
+  // parts only the last part owns them, since its work items end where the padded rows begin.
   if (TL > TV && a.out_peer_count == 0) {      // (peer mode: every rank zeroes its own receive buffer)
-    rc = launch_zero_rows(static_cast<__nv_bfloat16*>(a.out), a.out_stride[0], a.out_stride[1], a.out_stride[2],
-                          a.batch, a.heads, S + TV, TL - TV, stream);
-    if (rc != VB_OK) return rc;
-    ++g_launches;
+    ZeroRowsParams zp;
+    memset(&zp, 0, sizeof(zp));
+    zp.out = static_cast<__nv_bfloat16*>(a.out);
+    zp.stride_b = a.out_stride[0]; zp.stride_h = a.out_stride[1]; zp.stride_s = a.out_stride[2];
+    zp.batch = a.batch; zp.row0 = S + TV; zp.n_rows = TL - TV;
+    auto flush = [&]() -> int {      // one launch for up to kMaxZeroHeads heads
+      if (zp.n_heads == 0) return VB_OK;
+      const int r = launch_zero_rows(zp, stream);
+      if (r == VB_OK) ++g_launches;
+      zp.n_heads = 0;
+      return r;
+    };
+    for (int h = 0; h < a.heads; ++h) {
+      if (!blend) {
+        int e = a.branch[h];
+        if (e == VB_BRANCH_FULL_LO) e = VB_BRANCH_FULL_PART(0, 2);
+        if (e == VB_BRANCH_FULL_HI) e = VB_BRANCH_FULL_PART(1, 2);
+        if (e == VB_BRANCH_SKIP || (e >= 16 && ((e - 16) & 7) != ((e - 16) >> 3) - 1)) continue;
+      }
+      zp.head[zp.n_heads++] = a.out_heads ? a.out_heads[h] : h;
+      if (zp.n_heads == kMaxZeroHeads && (rc = flush()) != VB_OK) return rc;
+    }
+    if ((rc = flush()) != VB_OK) return rc;
   }
   return VB_OK;
 }

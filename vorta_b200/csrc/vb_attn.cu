@@ -564,9 +564,13 @@ vb_attn_fwd_kernel(const __grid_constant__ AttnTmaps tmaps, const __grid_constan
       const bool row_ok = row < pair.q_rows[t];
       const int krow = pair.q_row0[t] + row;      // row in kernel order
       const int stage = p.blend_stage;
-      const float w_head = stage == 0 ? 1.f
-                                      : __ldg(p.blend_w + (static_cast<int64_t>(batch) * p.blend_heads + head.wi) * 3 +
-                                              p.blend_branch);
+      float w_head = 1.f;
+      int64_t acc_off = 0;                        // blend mode: this head slot's rows of blend_acc
+      if (stage != 0) {
+        const int64_t bh = static_cast<int64_t>(batch) * p.blend_heads + head.wi;
+        w_head = __ldg(p.blend_w + bh * 3 + p.blend_branch);
+        acc_off = bh * p.blend_rows * kHeadDim + h * 64;
+      }
       const float inv = w_head / l_sum;
       int n_dst = 0;
       int64_t dst_tok = 0;
@@ -612,7 +616,7 @@ vb_attn_fwd_kernel(const __grid_constant__ AttnTmaps tmaps, const __grid_constan
             __nv_bfloat16* obase = p.out_peer_count > 0 ? p.out_peers[pe] : p.out;
             const int64_t off = head_off + tok * p.out_stride_s + c * 32;
             uint4* dst = reinterpret_cast<uint4*>(obase + off);
-            float4* acc = reinterpret_cast<float4*>(p.blend_acc + off);      // blend mode only
+            float4* acc = reinterpret_cast<float4*>(p.blend_acc + acc_off + tok * kHeadDim + c * 32);   // blend mode only
 #pragma unroll
             for (int q4i = 0; q4i < 4; ++q4i) {
               float f[8];

@@ -99,9 +99,9 @@ struct AttnParams {
   // 1, 2, 3.  Stage 1 stores w * O in fp32 into blend_acc, stage 2 adds to it, stage 3 adds and writes the bf16 output, so
   // the sum is formed in fp32 and rounded once.  blend_w: device (batch, blend_heads, 3) fp32 routing scores.
   const float* blend_w;
-  float* blend_acc;             // fp32, addressed with the output strides
+  float* blend_acc;             // fp32 (batch, blend_heads, blend_rows, 128): head slot wi, output token
   int32_t blend_stage;          // 0 = top-1 mode
-  int32_t blend_heads, blend_branch;
+  int32_t blend_heads, blend_branch, blend_rows;
   float* dbg;                   // optional debug dump (bring-up only), nullptr in production
   AttnSeg seg[kMaxSegments];
   AttnHead heads[kMaxHeads];
@@ -117,6 +117,16 @@ struct HeadList {
   uint8_t h[kMaxHeads];
   int32_t used;                // 0 = identity (slot i reads head i)
   __host__ __device__ int head(int slot) const { return used ? h[slot] : slot; }
+};
+
+// Zeroing of rows [row0, row0 + n_rows) of the listed output heads of every batch element, the head list passed BY
+// VALUE like HeadList (vb_kernels.cu)
+constexpr int kMaxZeroHeads = 256;
+struct ZeroRowsParams {
+  __nv_bfloat16* out;
+  int64_t stride_b, stride_h, stride_s;
+  int32_t batch, n_heads, row0, n_rows;
+  int32_t head[kMaxZeroHeads];  // output head index of each listed head
 };
 
 // Coreset selection launch parameters (vb_kernels.cu)

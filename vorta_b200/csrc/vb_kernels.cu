@@ -334,28 +334,27 @@ int launch_gather_rows(const GatherParams& p, cudaStream_t stream) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// Zero rows [row0, row0 + n) of every (batch, head): padded text queries produce 0 (hunyuan.py:176)
+// Zero rows [row0, row0 + n) of every (batch, listed output head): padded text queries produce 0 (hunyuan.py:176)
 // ------------------------------------------------------------------------------------------------
-__global__ void vb_zero_rows_kernel(__nv_bfloat16* out, int64_t sb, int64_t sh, int64_t ss, int batch, int heads,
-                                    int row0, int n_rows) {
-  const int64_t total = static_cast<int64_t>(batch) * heads * n_rows * 16;
+__global__ void vb_zero_rows_kernel(const ZeroRowsParams p) {
+  const int64_t total = static_cast<int64_t>(p.batch) * p.n_heads * p.n_rows * 16;
   for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
        i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const int c = static_cast<int>(i & 15);
     int64_t r = i >> 4;
-    const int row = static_cast<int>(r % n_rows);
-    r /= n_rows;
-    const int h = static_cast<int>(r % heads);
-    const int b = static_cast<int>(r / heads);
-    reinterpret_cast<uint4*>(out + b * sb + h * sh + static_cast<int64_t>(row0 + row) * ss)[c] = make_uint4(0, 0, 0, 0);
+    const int row = static_cast<int>(r % p.n_rows);
+    r /= p.n_rows;
+    const int h = p.head[r % p.n_heads];
+    const int b = static_cast<int>(r / p.n_heads);
+    reinterpret_cast<uint4*>(p.out + b * p.stride_b + h * p.stride_h + static_cast<int64_t>(p.row0 + row) * p.stride_s)[c] =
+        make_uint4(0, 0, 0, 0);
   }
 }
-int launch_zero_rows(__nv_bfloat16* out, int64_t sb, int64_t sh, int64_t ss, int batch, int heads, int row0,
-                     int n_rows, cudaStream_t stream) {
-  const int64_t total = static_cast<int64_t>(batch) * heads * n_rows * 16;
+int launch_zero_rows(const ZeroRowsParams& p, cudaStream_t stream) {
+  const int64_t total = static_cast<int64_t>(p.batch) * p.n_heads * p.n_rows * 16;
   if (total == 0) return VB_OK;
   const int grid = static_cast<int>((total + 255) / 256 < 1184 ? (total + 255) / 256 : 1184);
-  vb_zero_rows_kernel<<<grid, 256, 0, stream>>>(out, sb, sh, ss, batch, heads, row0, n_rows);
+  vb_zero_rows_kernel<<<grid, 256, 0, stream>>>(p);
   VB_CUDA_OK(cudaGetLastError());
   return VB_OK;
 }

@@ -139,6 +139,16 @@ def routed_attention(plan: Plan, q: torch.Tensor, k: torch.Tensor, v: torch.Tens
     if N != plan.seq_len + plan.text_len:
         raise ValueError(f"Input sequence length {N} does not match latent shape {plan.latent_shape}"
                          f" (+ text {plan.text_len}).")
+    if k.shape != q.shape or v.shape != q.shape:
+        raise ValueError(f"q, k and v must have the same shape, got {tuple(q.shape)}, {tuple(k.shape)}, "
+                         f"{tuple(v.shape)}")
+    if out_heads is not None and (len(out_heads) != H or min(out_heads) < 0):
+        raise ValueError(f"out_heads needs one non-negative output head per local head ({H}), got {list(out_heads)}")
+    if out_peers is None and out is not None:
+        _require_cuda_bf16("out", out)
+        last = max(out_heads) if out_heads is not None else H - 1
+        if out.shape[0] != B or out.shape[2] != N or out.shape[1] <= last:
+            raise ValueError(f"out must be (B={B}, more than {last} heads, N={N}, {D}), got {tuple(out.shape)}")
     args = L.AttnArgs()
     if out_peers is not None:
         # fused Ulysses "out" exchange: rows go straight into the owner ranks' (S_loc, H_total, 128) buffers; local
@@ -155,8 +165,6 @@ def routed_attention(plan: Plan, q: torch.Tensor, k: torch.Tensor, v: torch.Tens
     else:
         if out is None:
             out = torch.empty((B, N, H, D), dtype=q.dtype, device=q.device).transpose(1, 2)
-        else:
-            _require_cuda_bf16("out", out)
         args.out = out.data_ptr()
         args.out_stride[:] = out.stride()[:3]
     args.q, args.k, args.v = q.data_ptr(), k.data_ptr(), v.data_ptr()
@@ -308,8 +316,14 @@ def attn_dense(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, out: Optional[
         _require_cuda_bf16(name, t)
     B, H, Nq, D = q.shape
     Nk = k.shape[2]
+    if k.shape != v.shape or k.shape[:2] != q.shape[:2]:
+        raise ValueError(f"k and v must be (B={B}, H={H}, Nk, {D}) alike, got {tuple(k.shape)} and {tuple(v.shape)}")
     if out is None:
         out = torch.empty((B, Nq, H, D), dtype=q.dtype, device=q.device).transpose(1, 2)
+    else:
+        _require_cuda_bf16("out", out)
+        if out.shape != q.shape:
+            raise ValueError(f"out must have q's shape {tuple(q.shape)}, got {tuple(out.shape)}")
     i64x3 = C.c_int64 * 3
     with torch.cuda.device(q.device):
         L.check(L.lib().vb_attn_dense(q.data_ptr(), k.data_ptr(), v.data_ptr(), out.data_ptr(),

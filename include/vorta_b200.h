@@ -168,7 +168,11 @@ int vb_gather_rows(const void* src, int64_t src_stride_b, int64_t src_stride_h, 
  *                and rounded to bf16 once; one launch per branch)
  *   flags      : VB_ATTN_* bits
  *   workspace  : device scratch of at least vb_attn_workspace_bytes(...) bytes
- * Text tokens (HunyuanVideo) sit after the video tokens; rows of padded text queries are written as zero.
+ * Text tokens (HunyuanVideo) sit after the video tokens; rows of padded text queries are written as zero.  The
+ * un-padded text length is the plan's text_valid for every sample, or per sample (vb_attn_args::text_valid): then
+ * output sample b equals a batch-1 call on sample b alone with a plan whose text_valid is text_valid[b], bit for bit,
+ * and its rows [S + text_valid[b], S + text_len) are zero.  Routing is unchanged: one branch list for the batch (top-1),
+ * or per-(batch, head) scores (blend).
  * ---------------------------------------------------------------------------------------------------- */
 #define VB_ATTN_CORESET_KV_FROM_K 1u /* HunyuanVideo: K and V pooled with K's own matching (hunyuan.py:433-438) */
 
@@ -208,6 +212,12 @@ typedef struct {
   /* Blend mode with the routing scores left on the device: (batch, heads, 3) fp32, same meaning as `weights`; when set,
    * `weights` is ignored and no host copy of the scores is needed (the reference blends device tensors, wan.py:296-300). */
   const float* weights_device;
+  /* Optional (host pointer, batch entries, or NULL = the plan's text_valid for every sample): the un-padded text length
+   * of each sample, each within [0, text_len] (else VB_ERR_INVALID).  Samples with the same length share one schedule
+   * and one segment of the launch; the schedules of lengths other than the plan's are built on first use and cached in
+   * the plan (a bounded number of lengths, freed by vb_plan_destroy).  Prompts of different lengths can so be batched,
+   * e.g. num_videos_per_prompt > 1 or several prompts in one forward. */
+  const int32_t* text_valid;
 } vb_attn_args;
 
 int64_t vb_attn_workspace_bytes(const vb_plan* plan, int32_t batch, int32_t heads);

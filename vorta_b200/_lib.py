@@ -79,6 +79,7 @@ class AttnArgs(C.Structure):
         ("out_peer_rows", C.c_int32),
         ("out_heads", C.POINTER(C.c_int32)),
         ("weights_device", C.c_void_p),
+        ("text_valid", C.POINTER(C.c_int32)),
     ]
 
 

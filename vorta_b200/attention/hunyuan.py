@@ -5,10 +5,14 @@ The MM-DiT joint sequence is [video tokens | text tokens (padded)].  The referen
 masks around three library attention calls; here the text segment is part of the kernel's key-run tables
 (``vb_plan`` text_len / text_valid): video queries see the valid text keys, valid text queries see every non-pad
 key, padded text queries are written as zero (hunyuan.py:169-176; sliding_attn_flex.py:107-112).
+
+Any batch size: every sample has its own un-padded text length, read from ``attention_mask`` or given as
+``text_valid``, and sample b's output is bit-identical to a batch-1 call on sample b alone.  (The reference asserts
+batch 1, hunyuan.py:168.)
 """
 from __future__ import annotations
 
-from typing import Callable, Optional, Sequence, Tuple
+from typing import Callable, List, Optional, Sequence, Tuple, Union
 
 import torch
 
@@ -69,9 +73,24 @@ def _linear_into(linear, x2d: torch.Tensor, out2d: torch.Tensor) -> None:
         torch.mm(x2d, linear.weight.t(), out=out2d)
 
 
-def _valid_text(attention_mask: torch.Tensor, video_len: int) -> int:
-    """Number of un-padded text tokens from the boolean mask (B, 1, 1, S + S_text) (hunyuan.py:169)."""
-    return int(attention_mask.reshape(-1).sum().item()) - video_len
+TextValid = Union[None, int, Sequence[int]]
+
+
+def _valid_text(attention_mask: torch.Tensor, video_len: int) -> List[int]:
+    """Number of un-padded text tokens of every sample from the boolean mask (B, 1, 1, S + S_text) (hunyuan.py:169),
+    one host copy for the batch."""
+    counts = attention_mask.reshape(attention_mask.shape[0], -1).sum(dim=1).tolist()
+    return [int(c) - video_len for c in counts]
+
+
+def _per_sample(text_valid: TextValid, attention_mask, video_len: int, batch: int) -> List[int]:
+    """Per-sample un-padded text lengths: ``text_valid`` as given (one int for every sample, or one per sample), else
+    read from the mask."""
+    if text_valid is None:
+        return _valid_text(attention_mask, video_len)
+    if isinstance(text_valid, int):
+        return [text_valid] * batch
+    return [int(x) for x in text_valid]
 
 
 class HunyuanVideoFlashAttnProcessor:
@@ -121,25 +140,26 @@ class HunyuanVideoFlashAttnProcessor:
 
     # ---- step 5: attention --------------------------------------------------------------------------
     def _joint_attention(self, query, key, value, plan: ops.Plan, text_len: int, branch=None, weights=None,
-                         flags: int = 0) -> Tuple[torch.Tensor, torch.Tensor]:
+                         flags: int = 0, text_valid: Optional[Sequence[int]] = None
+                         ) -> Tuple[torch.Tensor, torch.Tensor]:
         """[video | text] joint attention for every branch in one C-ABI call; returns (video, text) outputs.
-        Under Ulysses the video part is exchanged (once for all branches), each rank keeps its head slice of the
-        replicated text tokens and the text outputs are all-gathered over heads (hunyuan.py:147-164,184-187)."""
-        B = query.shape[0]
-        assert B == 1, f"Batch size {B} is not supported for {self.__class__.__name__}."        # hunyuan.py:168
-        return routed_attention(plan, query, key, value, branch=branch, weights=weights, flags=flags, text_len=text_len)
+        ``text_valid``: the un-padded text length of every sample (default: the plan's).  Under Ulysses the video part is exchanged (once
+        for all branches), each rank keeps its head slice of the replicated text tokens and the text outputs are
+        all-gathered over heads (hunyuan.py:147-164,184-187)."""
+        return routed_attention(plan, query, key, value, branch=branch, weights=weights, flags=flags, text_len=text_len,
+                                text_valid=text_valid)
 
     def _step_attention(self, query, key, value, attention_mask, encoder_hidden_states_seq_len: int,
-                        skip_communication: bool = False, text_valid: Optional[int] = None
+                        skip_communication: bool = False, text_valid: TextValid = None
                         ) -> Tuple[torch.Tensor, torch.Tensor]:
-        """Full attention over the first S + valid_text tokens, zeros for padded text rows (hunyuan.py:136-189)."""
+        """Full attention over the first S + valid_text tokens of each sample, zeros for padded text rows
+        (hunyuan.py:136-189)."""
         text_len = encoder_hidden_states_seq_len
         video_len = (query.shape[2] - text_len) * (SP_STATE.sp_size if SP_STATE.enabled and not skip_communication else 1)
-        if text_valid is None:
-            text_valid = _valid_text(attention_mask, video_len)
-        plan = get_plan((1, 1, video_len), (1, 1, video_len), (1, 1, 1), (1, 1, 1), 0, text_len, text_valid)
+        tvs = _per_sample(text_valid, attention_mask, video_len, query.shape[0])
+        plan = get_plan((1, 1, video_len), (1, 1, video_len), (1, 1, 1), (1, 1, 1), 0, text_len, tvs[0])
         H = query.shape[1]
-        return self._joint_attention(query, key, value, plan, text_len, branch=[L.BRANCH_FULL] * H)
+        return self._joint_attention(query, key, value, plan, text_len, branch=[L.BRANCH_FULL] * H, text_valid=tvs)
 
     def _step_to_output(self, attn, hidden_states, encoder_hidden_states):
         hidden_states = hidden_states.transpose(1, 2).flatten(2, 3)
@@ -198,9 +218,10 @@ class HunyuanVideoFlashAttnProcessor:
         return self._step_encoder_to_qkv_and_concat(attn, query, key, value, encoder_hidden_states)
 
     def __call__(self, attn, hidden_states, encoder_hidden_states, attention_mask, image_rotary_emb,
-                 text_valid: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor]:
-        """``text_valid`` (extra, optional): the number of un-padded text tokens when the caller already knows it —
-        the reference reads it from ``attention_mask`` with a host sync in every layer (hunyuan.py:169)."""
+                 text_valid: TextValid = None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """``text_valid`` (extra, optional): the number of un-padded text tokens when the caller already knows it, one
+        int for every sample or one per sample — the reference reads it from ``attention_mask`` with a host sync in
+        every layer (hunyuan.py:169)."""
         query, key, value = self._qkv(attn, hidden_states, encoder_hidden_states, image_rotary_emb)
         hidden_states, encoder_hidden_states = self._step_attention(
             query, key, value, attention_mask, encoder_hidden_states.shape[1], text_valid=text_valid)
@@ -228,31 +249,30 @@ class HunyuanVideoFlashAttnProcessorTripleTrain(HunyuanVideoFlashAttnProcessor):
                 raise ValueError(f"Input sequence length {seq_length} does not match low-res info "
                                  f"{num_groups}x{group_size}.")
 
-    def _plan(self, lowres_group_info, window_size, tile_size, latent_shape, text_len, attention_mask,
-              text_valid: Optional[int] = None) -> ops.Plan:
-        S = latent_shape[0] * latent_shape[1] * latent_shape[2]
+    def _plan(self, lowres_group_info, window_size, tile_size, latent_shape, text_len, tvs: Sequence[int]) -> ops.Plan:
+        """The geometry's plan, keyed by sample 0's text length: a batch of one length runs the plan's own tables."""
         lowres_window = infer_lowres_window(lowres_group_info, latent_shape)
-        if text_valid is None:
-            text_valid = _valid_text(attention_mask, S)
         return get_plan(latent_shape, tile_size, window_size, lowres_window,
-                        lowres_group_info.num_unpooled_tokens_per_group, text_len, text_valid)
+                        lowres_group_info.num_unpooled_tokens_per_group, text_len, tvs[0])
 
     def _routed(self, attn, hidden_states, encoder_hidden_states, attention_mask, image_rotary_emb, lowres_group_info,
                 window_size, tile_size, latent_shape, branch=None, weights=None, text_valid=None):
         self._check_input(hidden_states, lowres_group_info, latent_shape, window_size, tile_size)
         text_len = encoder_hidden_states.shape[1]
         query, key, value = self._qkv(attn, hidden_states, encoder_hidden_states, image_rotary_emb)
-        plan = self._plan(lowres_group_info, window_size, tile_size, latent_shape, text_len, attention_mask, text_valid)
+        S = latent_shape[0] * latent_shape[1] * latent_shape[2]
+        tvs = _per_sample(text_valid, attention_mask, S, query.shape[0])
+        plan = self._plan(lowres_group_info, window_size, tile_size, latent_shape, text_len, tvs)
         # K and V are pooled with K's own matching, the output is unpooled with Q's (hunyuan.py:433-451)
         video, text = self._joint_attention(query, key, value, plan, text_len, branch=branch, weights=weights,
-                                            flags=L.ATTN_CORESET_KV_FROM_K)
+                                            flags=L.ATTN_CORESET_KV_FROM_K, text_valid=tvs)
         return self._step_to_output(attn, video, text)
 
     def __call__(self, attn, hidden_states, encoder_hidden_states, attention_mask, image_rotary_emb,
                  use_original_attn: bool = False, routing_score: Optional[torch.Tensor] = None,
                  lowres_group_info: Optional[LowresGroupInfo] = None, flex_attn_mask_func: Optional[Callable] = None,
                  window_size: Tuple[int, int, int] = (3, 3, 3), tile_size: Tuple[int, int, int] = (6, 8, 8),
-                 latent_shape: Tuple[int, int, int] = (30, 48, 80), text_valid: Optional[int] = None
+                 latent_shape: Tuple[int, int, int] = (30, 48, 80), text_valid: TextValid = None
                  ) -> Tuple[torch.Tensor, torch.Tensor]:
         if use_original_attn:
             return HunyuanVideoFlashAttnProcessor.__call__(self, attn, hidden_states, encoder_hidden_states,
@@ -268,7 +288,7 @@ class HunyuanVideoFlashAttnProcessorTripleEval(HunyuanVideoFlashAttnProcessorTri
                  routing_score: torch.Tensor, tau_sparse: float, lowres_group_info: Optional[LowresGroupInfo] = None,
                  flex_attn_mask_func: Optional[Callable] = None, window_size: Tuple[int, int, int] = (3, 3, 3),
                  tile_size: Tuple[int, int, int] = (6, 8, 8), latent_shape: Tuple[int, int, int] = (30, 48, 80),
-                 branch: Optional[Sequence[int]] = None, text_valid: Optional[int] = None
+                 branch: Optional[Sequence[int]] = None, text_valid: TextValid = None
                  ) -> Tuple[torch.Tensor, torch.Tensor]:
         if branch is None:
             branch = _top1_branches(routing_score, tau_sparse)          # hunyuan.py:620-624

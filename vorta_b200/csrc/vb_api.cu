@@ -6,7 +6,10 @@
 
 #include <algorithm>
 #include <array>
+#include <functional>
 #include <map>
+#include <memory>
+#include <mutex>
 #include <vector>
 
 #include <nvtx3/nvToolsExt.h>     // header-only NVTX v3: ranges cost a few ns unless a profiler is attached
@@ -174,6 +177,20 @@ struct Schedule {
   }
 };
 
+// The schedules that depend on the un-padded text length: full, coreset and sliding (queries in window-group order).
+struct TextSchedules {
+  int32_t text_valid = 0;
+  Schedule full, coreset, sliding;
+  int64_t keys_per_query = 0;   // video keys of a video query of the first window group (sliding)
+  uint64_t last_use = 0;
+  void release() {
+    full.release();
+    coreset.release();
+    sliding.release();
+  }
+};
+constexpr size_t kMaxCachedTextLengths = 16;
+
 }  // namespace vb
 
 using namespace vb;
@@ -182,7 +199,6 @@ struct vb_plan {
   vb_plan_desc d;
   int S = 0, G = 0, g = 0, n_u = 0, n_p = 0, S_c = 0;
   int nt[3] = {0, 0, 0}, n_tiles = 0, tile_tokens = 0;
-  int64_t keys_per_query = 0;
   bool has_device = false;
   // host tables
   std::vector<int64_t> center, margin;        // (G), (G, g-1)
@@ -198,7 +214,12 @@ struct vb_plan {
   };
   std::vector<WindowGroup> groups;
   std::vector<int32_t> query_map;             // (S + text_len): sliding-branch query position -> raster token
-  Schedule full, coreset, sliding;            // sliding: queries in window-group order
+  TextSchedules text;                         // for d.text_valid
+  // Per-sample text lengths (vb_attn_args::text_valid): the schedules of other lengths, built on first use and kept
+  // for later calls, at most kMaxCachedTextLengths of them between calls (least recently used dropped first)
+  std::vector<std::unique_ptr<TextSchedules>> other_text;
+  uint64_t text_clock = 0;
+  std::mutex text_mutex;                      // guards other_text for calls that pass per-sample lengths
   // device tables
   int32_t* d_center_tok = nullptr;
   int32_t* d_margin_tok = nullptr;
@@ -217,21 +238,22 @@ static void window_range(int q, int n, int w, int& lo, int& hi) {
   hi = std::min(n - 1, c + half);
 }
 
-static int build_text_dependent(vb_plan* pl) {
-  const vb_plan_desc& d = pl->d;
-  const int S = pl->S, tv = d.text_valid;
+// The schedules of text length tv (the plan's text_valid, or one sample's length) into ts.
+static int build_text_dependent(const vb_plan* pl, int tv, TextSchedules& ts) {
+  const int S = pl->S;
+  ts.text_valid = tv;
   // ---- full: every query sees [0, S + text_valid) (wan.py:142-144; hunyuan.py:169-176)
-  pl->full.clear();
-  pl->full.runs.push_back({0, S + tv});
-  pl->full.add_query_range(0, S + tv, 0, 1, S + tv);
+  ts.full.clear();
+  ts.full.runs.push_back({0, S + tv});
+  ts.full.add_query_range(0, S + tv, 0, 1, S + tv);
   // ---- coreset: same over the pooled sequence [centres | kept margins | text] (hunyuan.py:440-448)
-  pl->coreset.clear();
-  pl->coreset.runs.push_back({0, pl->S_c + tv});
-  pl->coreset.add_query_range(0, pl->S_c + tv, 0, 1, pl->S_c + tv);
+  ts.coreset.clear();
+  ts.coreset.runs.push_back({0, pl->S_c + tv});
+  ts.coreset.add_query_range(0, pl->S_c + tv, 0, 1, pl->S_c + tv);
   // ---- sliding tile (sliding_attn_flex.py:93-127): keys in tile-major order; one query range per window group
-  pl->sliding.clear();
+  ts.sliding.clear();
   const int tau = pl->tile_tokens;
-  Schedule& sc = pl->sliding;
+  Schedule& sc = ts.sliding;
   for (const vb_plan::WindowGroup& g : pl->groups) {
     const int run_begin = static_cast<int>(sc.runs.size());
     int64_t keys = 0;
@@ -254,7 +276,7 @@ static int build_text_dependent(vb_plan* pl) {
     const int run_count = static_cast<int>(sc.runs.size()) - run_begin;
     VB_REQUIRE(run_count <= 32, VB_ERR_UNSUPPORTED, "sliding window needs %d key runs per tile (max 32)", run_count);
     sc.add_query_range(g.row0, g.n_tiles * tau, run_begin, run_count, keys);
-    if (g.row0 == 0) pl->keys_per_query = keys - tv;
+    if (g.row0 == 0) ts.keys_per_query = keys - tv;
   }
   if (tv > 0) {   // valid text queries see every non-pad key (:108) as two runs, video and text: one run [0, S + tv)
                   // would cut the keys into different 128-key blocks and so change these rows' output bits
@@ -263,14 +285,61 @@ static int build_text_dependent(vb_plan* pl) {
     sc.runs.push_back({S, tv});
     sc.add_query_range(S, tv, run_begin, 2, S + tv);
   }
-  pl->full.finalize();
-  pl->coreset.finalize();
-  pl->sliding.finalize();
+  ts.full.finalize();
+  ts.coreset.finalize();
+  ts.sliding.finalize();
   if (pl->has_device) {
     int rc;
-    if ((rc = pl->full.upload()) != VB_OK) return rc;
-    if ((rc = pl->coreset.upload()) != VB_OK) return rc;
-    if ((rc = pl->sliding.upload()) != VB_OK) return rc;
+    if ((rc = ts.full.upload()) != VB_OK) return rc;
+    if ((rc = ts.coreset.upload()) != VB_OK) return rc;
+    if ((rc = ts.sliding.upload()) != VB_OK) return rc;
+  }
+  return VB_OK;
+}
+
+// The schedules of every length in `lengths` (distinct, each within [0, text_len]) into out[i]: the plan's own for its
+// text_valid, a cached set otherwise, built on first use.  When new sets would take the cache beyond
+// kMaxCachedTextLengths, the least recently used sets that this call does not need are dropped first, after a device
+// synchronize (earlier launches may still read their tables).  Caller holds pl->text_mutex.
+static int text_schedules(vb_plan* pl, const std::vector<int32_t>& lengths, std::vector<const TextSchedules*>& out) {
+  out.assign(lengths.size(), nullptr);
+  const uint64_t now = ++pl->text_clock;
+  size_t missing = 0;
+  for (size_t i = 0; i < lengths.size(); ++i) {
+    if (lengths[i] == pl->d.text_valid) {
+      out[i] = &pl->text;
+      continue;
+    }
+    for (const auto& e : pl->other_text)
+      if (e->text_valid == lengths[i]) {
+        e->last_use = now;
+        out[i] = e.get();
+      }
+    if (out[i] == nullptr) ++missing;
+  }
+  if (missing > 0 && pl->other_text.size() + missing > kMaxCachedTextLengths) {
+    if (pl->has_device) VB_CUDA_OK(cudaDeviceSynchronize());
+    while (pl->other_text.size() + missing > kMaxCachedTextLengths) {
+      auto victim = pl->other_text.end();
+      for (auto it = pl->other_text.begin(); it != pl->other_text.end(); ++it)
+        if ((*it)->last_use != now && (victim == pl->other_text.end() || (*it)->last_use < (*victim)->last_use))
+          victim = it;
+      if (victim == pl->other_text.end()) break;        // every cached set serves this call
+      (*victim)->release();
+      pl->other_text.erase(victim);
+    }
+  }
+  for (size_t i = 0; i < lengths.size(); ++i) {
+    if (out[i] != nullptr) continue;
+    std::unique_ptr<TextSchedules> ts(new TextSchedules());
+    int rc = build_text_dependent(pl, lengths[i], *ts);
+    if (rc != VB_OK) {
+      ts->release();
+      return rc;
+    }
+    ts->last_use = now;
+    out[i] = ts.get();
+    pl->other_text.push_back(std::move(ts));
   }
   return VB_OK;
 }
@@ -444,7 +513,7 @@ int vb_plan_create(vb_plan** out, const vb_plan_desc* desc) {
   } else {
     cudaGetLastError();
   }
-  int rc = build_text_dependent(pl);
+  int rc = build_text_dependent(pl, d.text_valid, pl->text);
   if (rc != VB_OK) {
     vb_plan_destroy(pl);
     return rc;
@@ -455,9 +524,8 @@ int vb_plan_create(vb_plan** out, const vb_plan_desc* desc) {
 
 void vb_plan_destroy(vb_plan* pl) {
   if (pl == nullptr) return;
-  pl->full.release();
-  pl->coreset.release();
-  pl->sliding.release();
+  pl->text.release();
+  for (auto& ts : pl->other_text) ts->release();
   if (pl->d_query_map) cudaFree(pl->d_query_map);
   if (pl->d_center_tok) cudaFree(pl->d_center_tok);
   if (pl->d_margin_tok) cudaFree(pl->d_margin_tok);
@@ -472,7 +540,8 @@ int vb_plan_set_text_valid(vb_plan* pl, int32_t text_valid) {
   if (text_valid == pl->d.text_valid) return VB_OK;
   if (pl->has_device) VB_CUDA_OK(cudaDeviceSynchronize());   // tables may still be in use by earlier launches
   pl->d.text_valid = text_valid;
-  return build_text_dependent(pl);
+  pl->text.release();
+  return build_text_dependent(pl, text_valid, pl->text);
 }
 
 int vb_plan_query(const vb_plan* pl, int what, int64_t* value) {
@@ -485,9 +554,9 @@ int vb_plan_query(const vb_plan* pl, int what, int64_t* value) {
     case VB_PLAN_NUM_TILES: *value = pl->n_tiles; break;
     case VB_PLAN_TILE_TOKENS: *value = pl->tile_tokens; break;
     case VB_PLAN_NUM_POOLED: *value = pl->n_p; break;
-    case VB_PLAN_KEYS_PER_QUERY: *value = pl->keys_per_query; break;
-    case VB_PLAN_SLIDING_PAIRS: *value = static_cast<int64_t>(pl->sliding.pairs.size()); break;
-    case VB_PLAN_SLIDING_RUNS: *value = static_cast<int64_t>(pl->sliding.runs.size()); break;
+    case VB_PLAN_KEYS_PER_QUERY: *value = pl->text.keys_per_query; break;
+    case VB_PLAN_SLIDING_PAIRS: *value = static_cast<int64_t>(pl->text.sliding.pairs.size()); break;
+    case VB_PLAN_SLIDING_RUNS: *value = static_cast<int64_t>(pl->text.sliding.runs.size()); break;
     default: VB_REQUIRE(false, VB_ERR_INVALID, "unknown plan query %d", what);
   }
   return VB_OK;
@@ -502,8 +571,11 @@ int vb_plan_export(const vb_plan* pl, int what, void* dst, int64_t* bytes) {
     case VB_EXPORT_MARGIN_INDICES: src = pl->margin.data(); n = pl->margin.size() * sizeof(int64_t); break;
     case VB_EXPORT_TILE_MAP: src = pl->tile_map.data(); n = pl->tile_map.size() * sizeof(int32_t); break;
     case VB_EXPORT_TILE_WINDOW: src = pl->tile_window.data(); n = pl->tile_window.size() * sizeof(int32_t); break;
-    case VB_EXPORT_SLIDING_RUNS: src = pl->sliding.runs.data(); n = pl->sliding.runs.size() * sizeof(KvRun); break;
-    case VB_EXPORT_SLIDING_ITEMS: src = pl->sliding.pairs.data(); n = pl->sliding.pairs.size() * sizeof(QPair); break;
+    case VB_EXPORT_SLIDING_RUNS: src = pl->text.sliding.runs.data(); n = pl->text.sliding.runs.size() * sizeof(KvRun); break;
+    case VB_EXPORT_SLIDING_ITEMS:
+      src = pl->text.sliding.pairs.data();
+      n = pl->text.sliding.pairs.size() * sizeof(QPair);
+      break;
     case VB_EXPORT_SLIDING_QUERY_MAP: src = pl->query_map.data(); n = pl->query_map.size() * sizeof(int32_t); break;
     default: VB_REQUIRE(false, VB_ERR_INVALID, "unknown plan export %d", what);
   }
@@ -631,6 +703,8 @@ struct Segment {
   int64_t bcast_stride_b = 0, bcast_stride_h = 0;
   int32_t bcast_rows = 0, bcast_n = 0;
   std::vector<AttnHead> heads;
+  std::vector<int32_t> batches;                 // batch elements of the segment (<= kMaxSegBatch); empty = all of them
+  int branch = 0;                               // 0 full (and its query parts), 1 coreset, 2 sliding
   double flops_per_head = 0.0;                  // of the segment's work items
 };
 
@@ -685,9 +759,11 @@ static void gather_from_args(GatherParams& gp, const vb_attn_args& a, int first,
   }
 }
 
-// Launches the head slots of n_seg <= kMaxSegments segments, in the given order (longest CTAs first), as grids of at
-// most kMaxHeads heads: a grid takes head slots until it is full, so a segment with more heads spans several launches.
-// The segments write disjoint outputs, or there is one of them (blend mode accumulates branch after branch).
+// Launches the head slots of n_seg segments, in the given order (longest CTAs first), as grids of at most kMaxHeads
+// heads and kMaxSegments segments: a grid takes segments until either is full, so a segment with more heads spans
+// several launches, and so do more segments than one grid holds.  Segments of the same heads over different batch
+// elements (one per text-length group) share their head slots.  The segments write disjoint outputs: different heads,
+// or the same heads of different batch elements (blend mode accumulates branch after branch, one call per branch).
 static int launch_segments(const Segment* segs, int n_seg, int batch, const Output& out, float* dbg,
                            const BlendState* blend, int kind, cudaStream_t stream) {
   AttnTmaps tm;
@@ -735,13 +811,31 @@ static int launch_segments(const Segment* segs, int n_seg, int batch, const Outp
     start_grid();
     return VB_OK;
   };
+  // head0 of n slots of this grid that already hold exactly hs[0, n), or -1
+  auto placed_heads = [&](const AttnHead* hs, int n) -> int {
+    for (int j = 0; j < n_used; ++j)
+      if (p.seg[j].n_heads == n && memcmp(&p.heads[p.seg[j].head0], hs, n * sizeof(AttnHead)) == 0)
+        return p.seg[j].head0;
+    return -1;
+  };
   start_grid();
   for (int i = 0; i < n_seg; ++i) {
     const Segment& sg = segs[i];
     if (sg.n_pairs == 0) continue;
+    VB_REQUIRE(sg.batches.size() <= static_cast<size_t>(kMaxSegBatch), VB_ERR_UNSUPPORTED,
+               "a segment lists at most %d batch elements", kMaxSegBatch);
+    const int n_batch = sg.batches.empty() ? batch : static_cast<int>(sg.batches.size());
     for (size_t h = 0; h < sg.heads.size();) {
-      if (head0 == kMaxHeads && (rc = launch_grid()) != VB_OK) return rc;
-      const int n = static_cast<int>(std::min(sg.heads.size() - h, static_cast<size_t>(kMaxHeads - head0)));
+      if (n_used == kMaxSegments && (rc = launch_grid()) != VB_OK) return rc;
+      int n = static_cast<int>(std::min(sg.heads.size() - h, static_cast<size_t>(kMaxHeads)));
+      int first = placed_heads(&sg.heads[h], n);
+      if (first < 0) {
+        if (head0 == kMaxHeads && (rc = launch_grid()) != VB_OK) return rc;
+        n = static_cast<int>(std::min(sg.heads.size() - h, static_cast<size_t>(kMaxHeads - head0)));
+        first = head0;
+        for (int j = 0; j < n; ++j) p.heads[head0 + j] = sg.heads[h + j];
+        head0 += n;
+      }
       CUtensorMap* m = tm.m[n_used];
       if ((rc = make_qkv_tensor_map(&m[0], sg.q, sg.n_rows_q, sg.n_heads_tensor, batch, sg.qs[0], sg.qs[1], sg.qs[2])))
         return rc;
@@ -757,18 +851,27 @@ static int launch_segments(const Segment* segs, int n_seg, int batch, const Outp
       s.bcast_rows = sg.bcast_rows; s.bcast_n = sg.bcast_n;
       s.n_pairs = sg.n_pairs;
       s.n_heads = n;
-      s.head0 = head0;
+      s.n_batch = n_batch;
+      s.batch_listed = sg.batches.empty() ? 0 : 1;
+      for (size_t j = 0; j < sg.batches.size(); ++j) s.batch_of[j] = static_cast<uint16_t>(sg.batches[j]);
+      s.head0 = first;
       s.cta_begin = static_cast<int32_t>(n_ctas);
-      for (int j = 0; j < n; ++j) p.heads[head0 + j] = sg.heads[h + j];
-      head0 += n;
       h += n;
-      n_ctas += static_cast<int64_t>(s.n_pairs) * s.n_heads * batch;
-      flops += sg.flops_per_head * s.n_heads * batch;
+      n_ctas += static_cast<int64_t>(s.n_pairs) * s.n_heads * n_batch;
+      flops += sg.flops_per_head * s.n_heads * n_batch;
       ++n_used;
     }
   }
   return launch_grid();
 }
+
+// Samples of one text length: that length's schedules and the batch elements that run them (empty = all of them).
+namespace {
+struct LengthGroup {
+  const TextSchedules* ts;
+  std::vector<int32_t> batches;
+};
+}  // namespace
 
 int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
   VB_REQUIRE(pl != nullptr && args != nullptr, VB_ERR_INVALID, "null argument");
@@ -786,8 +889,41 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   const bool blend = a.weights != nullptr || a.weights_device != nullptr;
   NvtxRange nvtx_layer(blend ? "vb_attn_fwd (blend)" : "vb_attn_fwd (top-1)");
-  const int S = pl->S, TL = pl->d.text_len, TV = pl->d.text_valid;
+  const int S = pl->S, TL = pl->d.text_len;
   const int N = S + TL;
+  int rc;
+
+  // un-padded text length of every sample (NULL: the plan's text_valid), and the samples grouped by length, longest
+  // first.  One length is one group over all samples, which runs the plan's own schedules when it is the plan's length.
+  std::vector<int32_t> tv_of(a.batch, pl->d.text_valid);
+  if (a.text_valid != nullptr) {
+    for (int b = 0; b < a.batch; ++b) {
+      VB_REQUIRE(a.text_valid[b] >= 0 && a.text_valid[b] <= TL, VB_ERR_INVALID,
+                 "text_valid[%d] = %d must be within [0, text_len %d]", b, a.text_valid[b], TL);
+      tv_of[b] = a.text_valid[b];
+    }
+  }
+  std::vector<int32_t> lengths(tv_of);
+  std::sort(lengths.begin(), lengths.end(), std::greater<int32_t>());
+  lengths.erase(std::unique(lengths.begin(), lengths.end()), lengths.end());
+  std::vector<const TextSchedules*> sched_of(1, &pl->text);
+  std::unique_lock<std::mutex> cache_lock;        // held until the launches that read cached tables are enqueued
+  if (lengths.size() > 1 || lengths[0] != pl->d.text_valid) {
+    cache_lock = std::unique_lock<std::mutex>(pl->text_mutex);
+    if ((rc = text_schedules(pl, lengths, sched_of)) != VB_OK) return rc;
+  }
+  std::vector<LengthGroup> groups;
+  if (lengths.size() == 1) {
+    groups.push_back({sched_of[0], {}});
+  } else {
+    for (size_t i = 0; i < lengths.size(); ++i)
+      for (int b = 0; b < a.batch; ++b) {
+        if (tv_of[b] != lengths[i]) continue;
+        if (groups.empty() || groups.back().ts != sched_of[i] || groups.back().batches.size() == kMaxSegBatch)
+          groups.push_back({sched_of[i], {}});
+        groups.back().batches.push_back(b);
+      }
+  }
 
   // heads of each branch, ascending head order (wan.py:409 torch.nonzero)
   std::vector<int32_t> by_branch[3];      // 0 full, 1 coreset, 2 sliding
@@ -821,7 +957,6 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
   VB_REQUIRE(!needs_ws || (a.workspace != nullptr && a.workspace_bytes >= need), VB_ERR_INVALID,
              "workspace too small: %lld < %lld bytes", (long long)a.workspace_bytes, (long long)need);
   Carver ws{static_cast<uint8_t*>(a.workspace), 0, a.workspace_bytes};
-  int rc;
   // blend mode: fp32 partial sums per (batch, head slot, output token), whatever the output's strides and out_heads, and
   // the routing scores on the device
   BlendState blend_state;
@@ -869,35 +1004,42 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
   std::vector<Segment> segs;
 
   // ---------------- branch 0: full attention, straight from the caller's tensors ----------------
-  if (!by_branch[0].empty() || !parts.empty()) {
-    const Segment full =
-        segment_of(a.q, a.k, a.v, a.q_stride, a.k_stride, a.v_stride, S + TV, S + TV, a.heads, pl->full);
-    if (!by_branch[0].empty()) {
-      segs.push_back(full);
+  // One segment per length group, of each of the full heads and the query parts
+  auto full_of = [&](const LengthGroup& g) {
+    const int tv = g.ts->text_valid;
+    Segment sg = segment_of(a.q, a.k, a.v, a.q_stride, a.k_stride, a.v_stride, S + tv, S + tv, a.heads, g.ts->full);
+    sg.batches = g.batches;
+    return sg;
+  };
+  if (!by_branch[0].empty()) {
+    for (const LengthGroup& g : groups) {
+      segs.push_back(full_of(g));
       segs.back().heads = head_entries(by_branch[0], false);
     }
-    // query parts: work items [k N / n, (k + 1) N / n) of the same schedule (other ranks run the other parts); a part's
-    // share of the head's FLOPs goes by query rows
-    const std::vector<QPair>& items = pl->full.pairs;
-    auto rows_of = [&](int begin, int end) {
-      int64_t rows = 0;
-      for (int i = begin; i < end; ++i) rows += items[i].q_rows[0] + (items[i].nq == 2 ? items[i].q_rows[1] : 0);
-      return rows;
-    };
-    const int64_t n_items = static_cast<int64_t>(items.size());
-    const int64_t rows_all = rows_of(0, static_cast<int>(n_items));
-    for (const auto& part : parts) {
-      const int n = (part.first - 16) >> 3, k = (part.first - 16) & 7;
+  }
+  // query parts: work items [k N / n, (k + 1) N / n) of the same schedule (other ranks run the other parts); a part's
+  // share of the head's FLOPs goes by query rows
+  for (const auto& part : parts) {
+    const int n = (part.first - 16) >> 3, k = (part.first - 16) & 7;
+    for (const LengthGroup& g : groups) {
+      const std::vector<QPair>& items = g.ts->full.pairs;
+      auto rows_of = [&](int begin, int end) {
+        int64_t rows = 0;
+        for (int i = begin; i < end; ++i) rows += items[i].q_rows[0] + (items[i].nq == 2 ? items[i].q_rows[1] : 0);
+        return rows;
+      };
+      const int64_t n_items = static_cast<int64_t>(items.size());
+      const int64_t rows_all = rows_of(0, static_cast<int>(n_items));
       const int begin = static_cast<int>(n_items * k / n), end = static_cast<int>(n_items * (k + 1) / n);
       if (end <= begin) continue;
       VB_REQUIRE(merge, VB_ERR_UNSUPPORTED, "query-half work units need the merged top-1 launch");
-      segs.push_back(full);
+      segs.push_back(full_of(g));
       Segment& sg = segs.back();
       sg.heads = head_entries(part.second, false);
       sg.pair_begin = begin;
       sg.n_pairs = end - begin;
-      sg.flops_per_head = pl->full.flops_per_head * (static_cast<double>(rows_of(begin, end)) /
-                                                     static_cast<double>(std::max<int64_t>(rows_all, 1)));
+      sg.flops_per_head = g.ts->full.flops_per_head * (static_cast<double>(rows_of(begin, end)) /
+                                                       static_cast<double>(std::max<int64_t>(rows_all, 1)));
     }
   }
 
@@ -947,14 +1089,19 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
       if ((rc = launch_gather_rows(gp, stream)) != VB_OK) return rc;
       g_launches += 2;
     }
-    Segment sg = workspace_segment(pooled, nh, rows, pl->S_c + TV, pl->coreset);
-    sg.heads = head_entries(hs, true);
-    sg.out_map = kept_q; sg.out_map_stride_b = nh * rows; sg.out_map_stride_h = rows;
-    if (pl->n_p > 0) {   // dropped margins receive their centre's output (coreset_select.py:157)
-      sg.bcast_map = drop_q; sg.bcast_stride_b = static_cast<int64_t>(nh) * pl->G * pl->n_p;
-      sg.bcast_stride_h = static_cast<int64_t>(pl->G) * pl->n_p; sg.bcast_rows = pl->G; sg.bcast_n = pl->n_p;
+    // the pooled sequences hold every sample's text rows; a length group attends to the first S_c + tv of them
+    for (const LengthGroup& g : groups) {
+      Segment sg = workspace_segment(pooled, nh, rows, pl->S_c + g.ts->text_valid, g.ts->coreset);
+      sg.heads = head_entries(hs, true);
+      sg.batches = g.batches;
+      sg.branch = 1;
+      sg.out_map = kept_q; sg.out_map_stride_b = nh * rows; sg.out_map_stride_h = rows;
+      if (pl->n_p > 0) {   // dropped margins receive their centre's output (coreset_select.py:157)
+        sg.bcast_map = drop_q; sg.bcast_stride_b = static_cast<int64_t>(nh) * pl->G * pl->n_p;
+        sg.bcast_stride_h = static_cast<int64_t>(pl->G) * pl->n_p; sg.bcast_rows = pl->G; sg.bcast_n = pl->n_p;
+      }
+      segs.push_back(std::move(sg));
     }
-    segs.push_back(std::move(sg));
   }
 
   // ---------------- branch 2: sliding tile ----------------
@@ -979,10 +1126,14 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
     gp.head_list = heads_s; gp.batch = a.batch; gp.heads = nh; gp.n_rows = static_cast<int32_t>(rows);
     if ((rc = launch_gather_rows(gp, stream)) != VB_OK) return rc;
     ++g_launches;
-    Segment sg = workspace_segment(tiled, nh, rows, S + TV, pl->sliding);
-    sg.heads = head_entries(hs, true);
-    sg.out_map = pl->d_query_map;
-    segs.push_back(std::move(sg));
+    for (const LengthGroup& g : groups) {
+      Segment sg = workspace_segment(tiled, nh, rows, S + g.ts->text_valid, g.ts->sliding);
+      sg.heads = head_entries(hs, true);
+      sg.batches = g.batches;
+      sg.branch = 2;
+      sg.out_map = pl->d_query_map;
+      segs.push_back(std::move(sg));
+    }
   }
 
   Output out;
@@ -998,32 +1149,28 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
                          stream);
     if (rc != VB_OK) return rc;
   } else {
-    // one branch at a time.  Blend: segment e is branch e, stage e + 1 of the fp32 accumulation; ONE launch covers every
-    // batch element (the scores are read per (batch, head) from the device table)
-    for (size_t e = 0; e < segs.size(); ++e) {
-      blend_state.stage = static_cast<int>(e) + 1;
-      blend_state.branch = static_cast<int>(e);
-      rc = launch_segments(&segs[e], 1, a.batch, out, a.debug, blend ? &blend_state : nullptr, VB_TIMING_ROUTED, stream);
+    // one branch at a time.  Blend: branch e is stage e + 1 of the fp32 accumulation; ONE launch covers every batch
+    // element (the scores are read per (batch, head) from the device table), a segment per length group, so each
+    // (batch, head) is accumulated once per stage
+    for (size_t i = 0; i < segs.size();) {
+      size_t j = i;
+      while (j < segs.size() && segs[j].branch == segs[i].branch) ++j;
+      blend_state.stage = segs[i].branch + 1;
+      blend_state.branch = segs[i].branch;
+      rc = launch_segments(&segs[i], static_cast<int>(j - i), a.batch, out, a.debug, blend ? &blend_state : nullptr,
+                           VB_TIMING_ROUTED, stream);
       if (rc != VB_OK) return rc;
+      i = j;
     }
   }
 
   // ---------------- padded text queries produce zeros (hunyuan.py:176; flex fully-masked rows) ----------------
   // They belong to the output heads the slots write (out_heads): a SKIP slot owns none, and of a head split into query
   // parts only the last part owns them, since its work items end where the padded rows begin.
-  if (TL > TV && a.out_peer_count == 0) {      // (peer mode: every rank zeroes its own receive buffer)
-    ZeroRowsParams zp;
-    memset(&zp, 0, sizeof(zp));
-    zp.out = static_cast<__nv_bfloat16*>(a.out);
-    zp.stride_b = a.out_stride[0]; zp.stride_h = a.out_stride[1]; zp.stride_s = a.out_stride[2];
-    zp.batch = a.batch; zp.row0 = S + TV; zp.n_rows = TL - TV;
-    auto flush = [&]() -> int {      // one launch for up to kMaxZeroHeads heads
-      if (zp.n_heads == 0) return VB_OK;
-      const int r = launch_zero_rows(zp, stream);
-      if (r == VB_OK) ++g_launches;
-      zp.n_heads = 0;
-      return r;
-    };
+  // Each sample's own padded rows [S + tv[b], S + text_len), all samples in one launch.
+  const int min_tv = lengths.back();
+  if (TL > min_tv && a.out_peer_count == 0) {      // (peer mode: every rank zeroes its own receive buffer)
+    std::vector<int32_t> zero_heads;
     for (int h = 0; h < a.heads; ++h) {
       if (!blend) {
         int e = a.branch[h];
@@ -1031,10 +1178,24 @@ int vb_attn_fwd(vb_plan* pl, const vb_attn_args* args, vb_stream_t stream_) {
         if (e == VB_BRANCH_FULL_HI) e = VB_BRANCH_FULL_PART(1, 2);
         if (e == VB_BRANCH_SKIP || (e >= 16 && ((e - 16) & 7) != ((e - 16) >> 3) - 1)) continue;
       }
-      zp.head[zp.n_heads++] = a.out_heads ? a.out_heads[h] : h;
-      if (zp.n_heads == kMaxZeroHeads && (rc = flush()) != VB_OK) return rc;
+      zero_heads.push_back(a.out_heads ? a.out_heads[h] : h);
     }
-    if ((rc = flush()) != VB_OK) return rc;
+    ZeroRowsParams zp;
+    memset(&zp, 0, sizeof(zp));
+    zp.stride_b = a.out_stride[0]; zp.stride_h = a.out_stride[1]; zp.stride_s = a.out_stride[2];
+    zp.row_end = N; zp.n_rows = TL - min_tv;
+    // one launch for up to kMaxZeroBatch batch elements and kMaxZeroHeads heads
+    for (int b0 = 0; b0 < a.batch; b0 += kMaxZeroBatch) {
+      zp.out = static_cast<__nv_bfloat16*>(a.out) + static_cast<int64_t>(b0) * a.out_stride[0];
+      zp.batch = std::min(kMaxZeroBatch, a.batch - b0);
+      for (int i = 0; i < zp.batch; ++i) zp.row0[i] = S + tv_of[b0 + i];
+      for (size_t h0 = 0; h0 < zero_heads.size(); h0 += kMaxZeroHeads) {
+        zp.n_heads = static_cast<int32_t>(std::min(zero_heads.size() - h0, static_cast<size_t>(kMaxZeroHeads)));
+        for (int i = 0; i < zp.n_heads; ++i) zp.head[i] = zero_heads[h0 + i];
+        if ((rc = launch_zero_rows(zp, stream)) != VB_OK) return rc;
+        ++g_launches;
+      }
+    }
   }
   return VB_OK;
 }

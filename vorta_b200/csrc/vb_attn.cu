@@ -111,7 +111,8 @@ struct BlockWalker {
 
 #define VB_EXP2(x) fast_exp2(x)
 
-// Work item -> (segment, pair, head, batch); segments are laid out longest items first by the host.  Every role of the
+// Work item -> (segment, pair, head, batch); segments are laid out longest items first by the host, and a segment's
+// batch elements are all of them or the ones it lists (one length group of per-sample text lengths).  Every role of the
 // CTA decodes the item itself (warp-uniform integer math + 48 bytes from global memory), so no hand-off is needed.
 struct Item {
   int seg_idx, batch;
@@ -132,7 +133,8 @@ __device__ __forceinline__ Item decode_item(const AttnParams& p, int item) {
   dst[1] = __ldg(src + 1);
   dst[2] = __ldg(src + 2);
   it.head = p.heads[seg.head0 + (local / seg.n_pairs) % seg.n_heads];
-  it.batch = local / (seg.n_pairs * seg.n_heads);
+  const int bi = local / (seg.n_pairs * seg.n_heads);      // i-th batch element of the segment
+  it.batch = seg.batch_listed ? static_cast<int>(seg.batch_of[bi]) : bi;
   return it;
 }
 

@@ -69,7 +69,10 @@ struct AttnHead {
 // One branch of a layer inside an attention launch: its own work table, Q/K/V tensor maps (AttnTmaps::m[i]) and row
 // maps.  A top-1 routed layer runs its (up to) three branches as three segments of ONE launch, longest CTAs first,
 // so the tail of one branch is filled by the next instead of idling the SMs between launches.
+// A segment may also cover a subset of the batch: HunyuanVideo samples with different un-padded text lengths run
+// different schedules, so each length group of a layer is a segment of its own over the samples that have that length.
 constexpr int kMaxSegments = 8;     // full, up to five kinds of query parts of full heads, coreset, sliding
+constexpr int kMaxSegBatch = 16;    // batch elements listed by one segment (AttnSeg::batch_of)
 struct AttnSeg {
   const QPair* pairs;
   const KvRun* runs;
@@ -80,6 +83,9 @@ struct AttnSeg {
   int64_t bcast_stride_h, bcast_stride_b;
   int32_t bcast_rows, bcast_n;
   int32_t n_pairs, n_heads;     // CTAs of the segment = n_pairs * n_heads * n_batch, pair index fastest
+  int32_t n_batch;              // batch elements of the segment
+  int32_t batch_listed;         // 0: the i-th batch element is element i; 1: it is batch_of[i] (n_batch <= kMaxSegBatch)
+  uint16_t batch_of[kMaxSegBatch];
   int32_t head0;                // the segment's heads are AttnParams::heads[head0 .. head0 + n_heads)
   int32_t cta_begin;            // linear item index of the segment's first work item
 };
@@ -110,6 +116,8 @@ struct AttnParams {
 struct AttnTmaps {
   CUtensorMap m[kMaxSegments][3];   // q, k, v of each segment (4-D: channel, row, head, batch)
 };
+// both travel by value as the attention kernel's parameters (32764 bytes on sm_70 and later, CUDA 12.1+)
+static_assert(sizeof(AttnTmaps) + sizeof(AttnParams) <= 32764, "attention launch parameters exceed the kernel limit");
 
 // Source head of each processed head slot, passed BY VALUE inside the launch parameters (<= 64 bytes): a layer's
 // head lists change with the routing of every layer and used to cost a pageable host->device copy each.
@@ -119,14 +127,16 @@ struct HeadList {
   __host__ __device__ int head(int slot) const { return used ? h[slot] : slot; }
 };
 
-// Zeroing of rows [row0, row0 + n_rows) of the listed output heads of every batch element, the head list passed BY
-// VALUE like HeadList (vb_kernels.cu)
+// Zeroing of rows [row0[b], row_end) of the listed output heads of every batch element b (each sample's padded text
+// rows), the head list passed BY VALUE like HeadList (vb_kernels.cu).  n_rows = row_end - min_b row0[b].
 constexpr int kMaxZeroHeads = 256;
+constexpr int kMaxZeroBatch = 64;
 struct ZeroRowsParams {
   __nv_bfloat16* out;
   int64_t stride_b, stride_h, stride_s;
-  int32_t batch, n_heads, row0, n_rows;
+  int32_t batch, n_heads, row_end, n_rows;
   int32_t head[kMaxZeroHeads];  // output head index of each listed head
+  int32_t row0[kMaxZeroBatch];  // first zeroed row of each batch element
 };
 
 // Coreset selection launch parameters (vb_kernels.cu)

@@ -334,7 +334,8 @@ int launch_gather_rows(const GatherParams& p, cudaStream_t stream) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// Zero rows [row0, row0 + n) of every (batch, listed output head): padded text queries produce 0 (hunyuan.py:176)
+// Zero rows [row0[b], row_end) of every (batch b, listed output head): padded text queries produce 0 (hunyuan.py:176);
+// each sample has its own number of padded rows, the grid covers the largest
 // ------------------------------------------------------------------------------------------------
 __global__ void vb_zero_rows_kernel(const ZeroRowsParams p) {
   const int64_t total = static_cast<int64_t>(p.batch) * p.n_heads * p.n_rows * 16;
@@ -342,11 +343,12 @@ __global__ void vb_zero_rows_kernel(const ZeroRowsParams p) {
        i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const int c = static_cast<int>(i & 15);
     int64_t r = i >> 4;
-    const int row = static_cast<int>(r % p.n_rows);
+    const int row = p.row_end - p.n_rows + static_cast<int>(r % p.n_rows);
     r /= p.n_rows;
     const int h = p.head[r % p.n_heads];
     const int b = static_cast<int>(r / p.n_heads);
-    reinterpret_cast<uint4*>(p.out + b * p.stride_b + h * p.stride_h + static_cast<int64_t>(p.row0 + row) * p.stride_s)[c] =
+    if (row < p.row0[b]) continue;        // a valid text row of this sample
+    reinterpret_cast<uint4*>(p.out + b * p.stride_b + h * p.stride_h + static_cast<int64_t>(row) * p.stride_s)[c] =
         make_uint4(0, 0, 0, 0);
   }
 }

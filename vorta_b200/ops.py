@@ -5,7 +5,7 @@ No arithmetic on the path happens here; every function ends in a call into ``lib
 from __future__ import annotations
 
 import ctypes as C
-from typing import Optional, Sequence, Tuple
+from typing import Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
@@ -112,8 +112,10 @@ class Plan:
         return ws
 
     # flop formulas of BASELINE.md section 3 (per head), for reporting
-    def flops_per_head(self, branch: int) -> float:
-        S, tv, D = self.seq_len, self.text_valid, HEAD_DIM
+    def flops_per_head(self, branch: int, text_valid: Optional[int] = None) -> float:
+        """Per head and sample, for the plan's text_valid or a sample's own un-padded text length."""
+        S, D = self.seq_len, HEAD_DIM
+        tv = self.text_valid if text_valid is None else int(text_valid)
         if branch == L.BRANCH_FULL:
             return 4.0 * (S + tv) ** 2 * D
         if branch == L.BRANCH_CORESET:
@@ -127,12 +129,15 @@ def routed_attention(plan: Plan, q: torch.Tensor, k: torch.Tensor, v: torch.Tens
                      flags: int = 0, out: Optional[torch.Tensor] = None,
                      debug: Optional[torch.Tensor] = None, out_peers: Optional[Sequence[int]] = None,
                      out_peer_rows: int = 0, out_peer_strides: Optional[Sequence[int]] = None,
-                     head_offset: int = 0, out_heads: Optional[Sequence[int]] = None) -> Optional[torch.Tensor]:
+                     head_offset: int = 0, out_heads: Optional[Sequence[int]] = None,
+                     text_valid: Union[None, int, Sequence[int]] = None) -> Optional[torch.Tensor]:
     """One routed self-attention layer.  q, k, v: (B, H, S + text_len, 128) bf16 views (any batch / head / token
     strides).  ``branch``: per-head VB_BRANCH_* ids (Eval processor semantics, wan.py:388-438); ``weights``:
     (B, H, 3) routing scores for the blended Train semantics (wan.py:296-300).  Returns (B, H, N, 128) as a view
     of (B, N, H, 128) memory, so ``transpose(1, 2).flatten(2, 3)`` (wan.py:152) is free.
-    ``out_heads``: head index along the output's head stride for each local head (default: ``head_offset + h``)."""
+    ``out_heads``: head index along the output's head stride for each local head (default: ``head_offset + h``).
+    ``text_valid``: un-padded text length of each sample (a sequence of B ints, or one int for all), default the
+    plan's; sample b's output equals a batch-1 call with a plan of text_valid[b], bit for bit."""
     for name, t in (("q", q), ("k", k), ("v", v)):
         _require_cuda_bf16(name, t)
     B, H, N, D = q.shape
@@ -142,6 +147,12 @@ def routed_attention(plan: Plan, q: torch.Tensor, k: torch.Tensor, v: torch.Tens
     if k.shape != q.shape or v.shape != q.shape:
         raise ValueError(f"q, k and v must have the same shape, got {tuple(q.shape)}, {tuple(k.shape)}, "
                          f"{tuple(v.shape)}")
+    if isinstance(text_valid, int):
+        text_valid = [text_valid] * B
+    if text_valid is not None:
+        text_valid = [int(x) for x in text_valid]
+        if len(text_valid) != B:
+            raise ValueError(f"text_valid needs one length per sample ({B}), got {len(text_valid)}")
     if out_heads is not None and (len(out_heads) != H or min(out_heads) < 0):
         raise ValueError(f"out_heads needs one non-negative output head per local head ({H}), got {list(out_heads)}")
     if out_peers is None and out is not None:
@@ -202,6 +213,12 @@ def routed_attention(plan: Plan, q: torch.Tensor, k: torch.Tensor, v: torch.Tens
         args.out_heads = C.cast(oh, C.POINTER(C.c_int32))
     else:
         args.out_heads = None
+    if text_valid is not None:
+        tvs = (C.c_int32 * B)(*text_valid)
+        keep.append(tvs)
+        args.text_valid = C.cast(tvs, C.POINTER(C.c_int32))
+    else:
+        args.text_valid = None
     args.flags = int(flags)
     ws = plan.workspace(B, H, q.device)
     args.workspace, args.workspace_bytes = ws.data_ptr(), ws.numel()

@@ -69,7 +69,8 @@ def _attn_kwargs(self_attention_kwargs, routing_score, branch):
 
 
 def _text_valid_kw(self_attention_kwargs):
-    """{"text_valid": n} when the transformer forward counted the prompt's un-padded tokens once for the whole step."""
+    """{"text_valid": [n_0, ...]} when the transformer forward counted every prompt's un-padded tokens once for the
+    whole step."""
     tv = (self_attention_kwargs or {}).get("text_valid")
     return {} if tv is None else {"text_valid": tv}
 
@@ -161,8 +162,9 @@ def hunyuan_transformer_3d_routed_forward(self, hidden_states: torch.Tensor, tim
 
     kwargs = dict(self_attention_kwargs or {})
     tau = kwargs.get("tau_sparse")
-    if batch_size == 1:        # ONE host read per step instead of one per layer (hunyuan.py:169 syncs in every block)
-        kwargs["text_valid"] = int(effective[0].item()) - latent_len
+    # the un-padded text length of every sample, ONE host read per step instead of one per layer (hunyuan.py:169 syncs
+    # in every block)
+    kwargs["text_valid"] = [int(e) - latent_len for e in effective.tolist()]
     blocks = list(self.transformer_blocks) + list(self.single_transformer_blocks)
     eval_mode = isinstance(blocks[0].attn.processor, HunyuanVideoFlashAttnProcessorTripleEval)
     if not eval_mode and torch.is_grad_enabled() and any(q.requires_grad for q in blocks[0].router.parameters()):

@@ -122,7 +122,9 @@ def hunyuan_denoise(transformer, scheduler, latents: torch.Tensor, prompt_embeds
     kwargs = deepcopy(self_attention_kwargs) if self_attention_kwargs is not None else None
     if kwargs is not None:
         text_len = prompt_attention_mask.shape[1]
-        text_valid = int(prompt_attention_mask.sum(dim=1, dtype=torch.int)[0].item())      # :381-382 (batch 0 decides)
+        # :381-382 (batch 0 decides).  This schedule object is kept for the reference's kwargs only: the processors
+        # read every sample's own text length from the attention mask, so any batch size runs
+        text_valid = int(prompt_attention_mask.sum(dim=1, dtype=torch.int)[0].item())
         kwargs.update(flex_attn_mask_func=create_sliding_tile_attn_mask_func(
             latent_shape=kwargs["latent_shape"], window_size=kwargs["window_size"], tile_size=kwargs["tile_size"],
             text_seq_length=text_len, text_seq_length_no_pad=text_valid, device=latents.device))

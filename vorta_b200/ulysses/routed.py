@@ -42,19 +42,23 @@ def _split(out: torch.Tensor, text_len: int):
 
 def routed_attention(plan: ops.Plan, q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, *,
                      branch: Optional[Sequence[int]] = None, weights: Optional[torch.Tensor] = None, flags: int = 0,
-                     text_len: int = 0) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+                     text_len: int = 0, text_valid: Optional[Sequence[int]] = None
+                     ) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
     """-> (video, text). video: (B, H, S_loc, 128) view of (B, S_loc, H, 128) memory (S_loc = S without SP);
     text: (B, H, text_len, 128), or None when text_len == 0.
 
     q, k, v: (B, H, S_loc + text_len, 128) views: this rank's video tokens, then the replicated text tokens.
-    ``branch`` / ``weights``: per-head branch ids (top-1) or (B, H, 3) routing scores (blend), as in
-    ``ops.routed_attention``."""
+    ``branch`` / ``weights``: per-head branch ids (top-1) or (B, H, 3) routing scores (blend), ``text_valid``: the
+    un-padded text length of every sample (default: the plan's), as in ``ops.routed_attention``.  Batch 1 with
+    sample 0's length equal to the plan's takes the peer path; other batches take the NCCL path."""
     if not SP_STATE.enabled:
-        return _split(ops.routed_attention(plan, q, k, v, branch=branch, weights=weights, flags=flags), text_len)
+        return _split(ops.routed_attention(plan, q, k, v, branch=branch, weights=weights, flags=flags,
+                                           text_valid=text_valid), text_len)
     B, H, N = q.shape[:3]
     n = N - text_len
     P, r = SP_STATE.sp_size, SP_STATE.group_local_rank
-    ex = peer.get_exchange(H, n, q.device, text_len) if weights is None and B == 1 else None
+    own_length = text_valid is None or list(text_valid) == [plan.text_valid]
+    ex = peer.get_exchange(H, n, q.device, text_len) if weights is None and B == 1 and own_length else None
     if ex is not None:
         # Q / K / V rows are stored straight into the buffers of the ranks that own the head (or a query half of it),
         # the attention epilogue stores every output row straight into the buffer of the rank that owns the token (text
@@ -84,7 +88,8 @@ def routed_attention(plan: ops.Plan, q: torch.Tensor, k: torch.Tensor, v: torch.
         for dst, src in ((qs, q), (ks, k), (vs, v)):
             text = src[:, :, n:]
             dst[:, :, -text_len:] = shrink_dim(text, dim=1) if mine is None else text.index_select(1, mine)
-    video, text = _split(ops.routed_attention(plan, qs, ks, vs, branch=branch, weights=weights, flags=flags), text_len)
+    video, text = _split(ops.routed_attention(plan, qs, ks, vs, branch=branch, weights=weights, flags=flags,
+                                              text_valid=text_valid), text_len)
     video = exchange_out(video, head_at)
     if text_len:
         text = all_gather(text.contiguous(), dim=1)

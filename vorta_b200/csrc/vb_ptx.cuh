@@ -270,8 +270,11 @@ __device__ __forceinline__ void fadd2(float& d0, float& d1, float a0, float a1, 
 // minimax polynomial for 2^f (max relative error 7.5e-5, far below the bf16 rounding P receives anyway), exponent
 // added as an integer.  The MUFU ex2 unit (16 / clk / SM) is co-critical with the tensor pipe at head_dim 128
 // (512 MMA flops per exp), so a fraction of the exps is computed here instead.
+// Below -126 the result is exactly 0, as ex2.approx.ftz gives: the integer exponent add needs x >= -126, and the clamp
+// alone turned a masked key (x = -inf) into a weight of 2^-126 * p(0) that the PV MMA multiplies by a real V row.
 __device__ __forceinline__ void exp2_poly2(float x0, float x1, float& e0, float& e1) {
   constexpr float kMagic = 12582912.f;   // 1.5 * 2^23: adding it rounds to an integer held in the low mantissa bits
+  const bool z0 = x0 < -126.f, z1 = x1 < -126.f;
   x0 = fmaxf(x0, -126.f);
   x1 = fmaxf(x1, -126.f);
   float t0, t1, r0, r1, f0, f1, p0, p1;
@@ -281,8 +284,8 @@ __device__ __forceinline__ void exp2_poly2(float x0, float x1, float& e0, float&
   ffma2(p0, p1, f0, f1, 0.055171020f, 0.055171020f, 0.24260981f, 0.24260981f);
   ffma2(p0, p1, p0, p1, f0, f1, 0.69326097f, 0.69326097f);
   ffma2(p0, p1, p0, p1, f0, f1, 0.99992818f, 0.99992818f);
-  e0 = __int_as_float(__float_as_int(p0) + (__float_as_int(t0) << 23));
-  e1 = __int_as_float(__float_as_int(p1) + (__float_as_int(t1) << 23));
+  e0 = z0 ? 0.f : __int_as_float(__float_as_int(p0) + (__float_as_int(t0) << 23));
+  e1 = z1 ? 0.f : __int_as_float(__float_as_int(p1) + (__float_as_int(t1) << 23));
 }
 
 // pack two fp32 -> bf16x2 (lo in bits [0,16), hi in bits [16,32)), round-to-nearest-even

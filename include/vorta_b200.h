@@ -239,9 +239,11 @@ double vb_stats_attn_flops(void);
 /* ------------------------------------------------------------------------------------------------------
  * Fused elementwise kernels of the DiT block around the path (SURVEY.md section 8f rows 1-2; "next" rows).
  * Rows are tokens, bf16, contiguous, `dim` channels (multiple of 8, <= 8192); fp32 math; one read + one write.
+ * x, y, out and the bf16 weights (and headnorm's cos / sin tables) must be 16-byte aligned: VB_ERR_INVALID otherwise.
  *   vb_block_ln_modulate : out = (LayerNorm(x) [* weight + bias]) [* (1 + scale) + shift]
  *        replaces norm1/norm3 + adaLN modulate and norm2 (vorta/patch/modeling_wan.py:205-206, 226, 232-234);
- *        weight/bias fp32 (dim) or NULL; scale/shift fp32 (batch, dim) or NULL; batch = row / rows_per_batch
+ *        weight/bias fp32 (dim) or NULL (each applies on its own); scale/shift fp32 (batch, dim) or NULL;
+ *        batch = row / rows_per_batch
  *   vb_block_gate_residual: out = x + y * gate  (gate fp32 (batch, dim), NULL = plain add)   (:225, :229, :238)
  *   vb_block_rmsnorm_rope : RMSNorm over the whole row * weight (bf16, dim), then the complex rotation of channel
  *        pairs of every 128-wide head by (cos, sin) fp32 (tokens_per_batch, 64); token = row % tokens_per_batch.

@@ -62,3 +62,22 @@ def test_no_cuda_means_loud_failure():
     with pytest.raises(L.VortaB200Error):
         ops.coreset_select(plan, x)
     assert L.lib().vb_device_check() == L.VB_ERR_UNSUPPORTED
+
+
+def test_block_kernels_refuse_misaligned_vector_pointers():
+    """Every pointer a block kernel reads or writes with 16-byte vectors must be 16-byte aligned: VB_ERR_INVALID is
+    returned before any launch (the addresses below are never dereferenced)."""
+    lib = L.lib()
+    A, M = 0x10000, 0x10008                    # aligned, misaligned (8 bytes past a 16-byte boundary)
+    rows, dim = 4, 1536
+    for x, out in ((M, A), (A, M)):
+        assert lib.vb_block_ln_modulate(x, None, None, None, None, out, rows, dim, rows, 1e-6, None) == L.VB_ERR_INVALID
+        assert lib.vb_block_rmsnorm_rope(x, A, None, None, out, rows, dim, rows, 1e-6, None) == L.VB_ERR_INVALID
+    for x, y, out in ((M, A, A), (A, M, A), (A, A, M)):
+        assert lib.vb_block_gate_residual(x, y, None, out, rows, dim, rows, None) == L.VB_ERR_INVALID
+    assert lib.vb_block_rmsnorm_rope(A, M, None, None, A, rows, dim, rows, 1e-6, None) == L.VB_ERR_INVALID
+    hn = (lambda x, w, c, s, out: lib.vb_block_headnorm_rope(x, w, c, s, out, 1, rows, 12, rows, rows, 0, 1e-6, None))
+    for args in ((M, A, A, A, A), (A, M, A, A, A), (A, A, M, A, A), (A, A, A, M, A), (A, A, A, A, M),
+                 (A, None, M, A, A)):
+        assert hn(*args) == L.VB_ERR_INVALID, args
+    assert b"16-byte" in lib.vb_last_error()

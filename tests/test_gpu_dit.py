@@ -56,7 +56,17 @@ def _wan_reference_forward(model, latents, timestep, text, branches, info):
 
 
 def test_wan_dit_step_matches_torch_reference():
-    wan_mod.WAN_CONFIGS["tiny"] = wan_mod.WanConfig(dim=384, heads=3, ffn_dim=512, num_layers=3, text_dim=64)
+    _wan_dit_step_check(dim=384, heads=3)
+
+
+def test_wan_dit_step_at_a_production_width():
+    """dim 1536 (Wan-1.3B): the block kernels run their warp-per-row instances inside a whole step (at 384 channels
+    every row kernel takes the CTA-per-row fallback)."""
+    _wan_dit_step_check(dim=1536, heads=12)
+
+
+def _wan_dit_step_check(dim, heads):
+    wan_mod.WAN_CONFIGS["tiny"] = wan_mod.WanConfig(dim=dim, heads=heads, ffn_dim=512, num_layers=3, text_dim=64)
     dev = torch.device("cuda:0")
     model = WanDiT.build("tiny", dev, torch.bfloat16, seed=3)
     apply_vorta_transformer(model, router_dtype=torch.float32)
@@ -69,7 +79,8 @@ def test_wan_dit_step_matches_torch_reference():
     # make the routers decisive and varied so that every branch appears
     with torch.no_grad():
         for li, blk in enumerate(model.blocks):
-            blk.router.linear.bias.copy_(torch.tensor([[3., 0., 0.], [0., 3., 0.], [0., 0., 3.]]).roll(li, 0).flatten())
+            pattern = torch.tensor([[3., 0., 0.], [0., 3., 0.], [0., 0., 3.]]).roll(li, 0)
+            blk.router.linear.bias.copy_(pattern[torch.arange(heads) % 3].flatten())
     with torch.no_grad():
         res = model(latents.to(dev, torch.bfloat16), ts.to(dev), text.to(dev, torch.bfloat16),
                     self_attention_kwargs=kw, return_routing_scores=True)

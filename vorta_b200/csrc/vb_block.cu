@@ -62,19 +62,29 @@ vb_ln_modulate_kernel(const __nv_bfloat16* __restrict__ x, const float* __restri
   const int nvec = dim >> 3;
   const uint4* xr = reinterpret_cast<const uint4*>(x + row * dim);
   float v[kMaxVec][8];
-  float s1 = 0.f, s2 = 0.f;
+  float s1 = 0.f, s2 = 0.f, dummy = 0.f;
 #pragma unroll
   for (int i = 0; i < kMaxVec; ++i) {
     const int idx = threadIdx.x + i * kRowThreads;
     if (idx < nvec) {
       unpack8(xr[idx], v[i]);
 #pragma unroll
-      for (int e = 0; e < 8; ++e) { s1 += v[i][e]; s2 += v[i][e] * v[i][e]; }
+      for (int e = 0; e < 8; ++e) s1 += v[i][e];
     }
   }
-  block_sum2(s1, s2);
+  block_sum2(s1, dummy);
   const float mean = s1 / dim;
-  const float rstd = rsqrtf(fmaxf(s2 / dim - mean * mean, 0.f) + eps);
+  // variance in a second pass over the registers: sum(x^2)/n - mean^2 cancels catastrophically when |mean| >> std
+#pragma unroll
+  for (int i = 0; i < kMaxVec; ++i) {
+    const int idx = threadIdx.x + i * kRowThreads;
+    if (idx < nvec) {
+#pragma unroll
+      for (int e = 0; e < 8; ++e) { const float d = v[i][e] - mean; s2 = fmaf(d, d, s2); }
+    }
+  }
+  block_sum2(s2, dummy);
+  const float rstd = rsqrtf(s2 / dim + eps);
   const int64_t batch = row / rows_per_batch;
   const float* sc = scale ? scale + batch * dim : nullptr;
   const float* sh = shift ? shift + batch * dim : nullptr;
@@ -89,6 +99,7 @@ vb_ln_modulate_kernel(const __nv_bfloat16* __restrict__ x, const float* __restri
         const int c = idx * 8 + e;
         float t = (v[i][e] - mean) * rstd;
         if (w) t = t * w[c] + (b ? b[c] : 0.f);
+        else if (b) t += b[c];
         if (sc) t = t * (1.f + sc[c]) + sh[c];
         y[e] = t;
       }
@@ -184,6 +195,11 @@ vb_ln_modulate_warp_kernel(const __nv_bfloat16* __restrict__ x, const float* __r
       }
 #pragma unroll
       for (int e = 0; e < 8; ++e) f[e] = f[e] * wv[e] + bv[e];
+    } else if (b) {
+      const float4 b0 = ldg4(b + c0), b1 = ldg4(b + c0 + 4);
+      const float bv[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+#pragma unroll
+      for (int e = 0; e < 8; ++e) f[e] += bv[e];
     }
     if (sc) {
       const float4 a0 = ldg4(sc + c0), a1 = ldg4(sc + c0 + 4), h0 = ldg4(sh + c0), h1 = ldg4(sh + c0 + 4);
@@ -400,6 +416,9 @@ __global__ void __launch_bounds__(256) vb_headnorm_rope_kernel(const HeadNormPar
   }
 }
 
+// the kernels read and write x / y / out (and the bf16 weights, and headnorm's tables) with 16-byte vectors
+static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
 int launch_headnorm_rope(const void* x, const void* weight, const float* cs, const float* sn, void* out, int batch,
                          int rows, int heads, int rope_rows, int dst_rows, int dst_row0, float eps,
                          cudaStream_t stream) {
@@ -407,6 +426,8 @@ int launch_headnorm_rope(const void* x, const void* weight, const float* cs, con
              "headnorm_rope: rows [%d, %d) do not fit a destination of %d rows", dst_row0, dst_row0 + rows, dst_rows);
   VB_REQUIRE((cs == nullptr) == (sn == nullptr) && rope_rows <= rows, VB_ERR_INVALID,
              "headnorm_rope: cos / sin tables come together and cover at most the source rows");
+  VB_REQUIRE(aligned16(x) && aligned16(out) && aligned16(weight) && aligned16(cs) && aligned16(sn), VB_ERR_INVALID,
+             "headnorm_rope: x, out, weight and the cos / sin tables must be 16-byte aligned");
   HeadNormParams p;
   p.x = static_cast<const __nv_bfloat16*>(x);
   p.weight = static_cast<const __nv_bfloat16*>(weight);
@@ -431,10 +452,11 @@ static unsigned row_grid(int64_t rows, int nv) {
 int launch_ln_modulate(const void* x, const float* w, const float* b, const float* scale, const float* shift, void* out,
                        int64_t rows, int dim, int rows_per_batch, float eps, cudaStream_t stream) {
   VB_REQUIRE(dim % 8 == 0 && dim <= kRowThreads * kMaxVec * 8, VB_ERR_UNSUPPORTED, "row width %d not supported", dim);
+  VB_REQUIRE(aligned16(x) && aligned16(out), VB_ERR_INVALID, "ln_modulate: x and out must be 16-byte aligned");
   if (rows == 0) return VB_OK;
   const __nv_bfloat16* xb = static_cast<const __nv_bfloat16*>(x);
   __nv_bfloat16* ob = static_cast<__nv_bfloat16*>(out);
-  
+  // the CTA-per-row kernel reads the fp32 parameters with scalar loads, so misaligned parameters take it
   const bool aligned = ((reinterpret_cast<uintptr_t>(w) | reinterpret_cast<uintptr_t>(b) | reinterpret_cast<uintptr_t>(scale) |
                          reinterpret_cast<uintptr_t>(shift)) & 15) == 0;
 #define VB_LN_CASE(NV)                                                                                              \
@@ -455,6 +477,8 @@ int launch_ln_modulate(const void* x, const float* w, const float* b, const floa
 int launch_gate_residual(const void* x, const void* y, const float* gate, void* out, int64_t rows, int dim,
                          int rows_per_batch, cudaStream_t stream) {
   VB_REQUIRE(dim % 8 == 0, VB_ERR_UNSUPPORTED, "row width %d not supported", dim);
+  VB_REQUIRE(aligned16(x) && aligned16(y) && aligned16(out), VB_ERR_INVALID,
+             "gate_residual: x, y and out must be 16-byte aligned");
   const int64_t n_vec = rows * (dim >> 3);
   if (n_vec == 0) return VB_OK;
   const int64_t blocks = (n_vec + 255) / 256;
@@ -469,13 +493,14 @@ int launch_rmsnorm_rope(const void* x, const void* weight, const float* cs, cons
                         int dim, int tokens_per_batch, float eps, cudaStream_t stream) {
   VB_REQUIRE(dim % kHeadDim == 0 && dim <= kRowThreads * kMaxVec * 8, VB_ERR_UNSUPPORTED,
              "row width %d not supported", dim);
+  VB_REQUIRE(aligned16(x) && aligned16(out) && aligned16(weight), VB_ERR_INVALID,
+             "rmsnorm_rope: x, out and weight must be 16-byte aligned");
   if (rows == 0) return VB_OK;
   const __nv_bfloat16* xb = static_cast<const __nv_bfloat16*>(x);
   const __nv_bfloat16* wb = static_cast<const __nv_bfloat16*>(weight);
   __nv_bfloat16* ob = static_cast<__nv_bfloat16*>(out);
-  
-  const bool aligned = ((reinterpret_cast<uintptr_t>(weight) | reinterpret_cast<uintptr_t>(cs) |
-                         reinterpret_cast<uintptr_t>(sn)) & 15) == 0;
+  // the CTA-per-row kernel reads the tables with scalar loads, so misaligned tables take it
+  const bool aligned = aligned16(cs) && aligned16(sn);
 #define VB_RMS_CASE(NV)                                                                                             \
   case NV * 256:                                                                                                    \
     vb_rmsnorm_rope_warp_kernel<NV><<<row_grid(rows, NV), kRowCtaThreads, 0, stream>>>(xb, wb, cs, sn, ob, rows,   \

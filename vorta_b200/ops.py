@@ -376,6 +376,7 @@ def _rows(x: torch.Tensor):
         raise L.VortaB200Error("block kernels need CUDA tensors: vorta_b200 has no CPU path")
     if x.dtype != torch.bfloat16 or x.dim() != 3 or not x.is_contiguous():
         raise ValueError("block kernels need contiguous bf16 tensors of shape (B, S, dim)")
+    _require_aligned("x", x)
     return x.shape[0] * x.shape[1], x.shape[2], x.shape[1]
 
 
@@ -383,21 +384,62 @@ def _contig(x: torch.Tensor) -> torch.Tensor:
     return x if x.is_contiguous() else x.contiguous()
 
 
-def _f32(t: Optional[torch.Tensor]):
+def _require_aligned(name: str, t: torch.Tensor) -> None:
+    # the kernels move activations as 16-byte vectors; a contiguous view can start at any element
+    if t.data_ptr() % 16:
+        raise ValueError(f"{name} must start at a 16-byte aligned address (a view at element offset "
+                         f"{t.storage_offset()} does not)")
+
+
+def _param(name: str, t: Optional[torch.Tensor], dtype: torch.dtype, device: torch.device):
+    """A parameter tensor as the kernels read it: ``dtype``, contiguous, on ``device``, 16-byte aligned (misaligned
+    or strided storage is copied to a fresh allocation)."""
     if t is None:
         return None
-    if t.dtype != torch.float32 or not t.is_contiguous():
-        t = t.float().contiguous()
+    if t.device != device:
+        raise ValueError(f"{name} must be on {device}, got {t.device}")
+    if t.dtype != dtype:
+        t = t.to(dtype)
+    if not t.is_contiguous() or t.data_ptr() % 16:
+        t = t.clone(memory_format=torch.contiguous_format)
     return t
+
+
+def _vector(name: str, t: Optional[torch.Tensor], dim: int, device: torch.device, dtype=torch.float32):
+    if t is not None and t.numel() != dim:
+        raise ValueError(f"{name} must have dim = {dim} entries, got shape {tuple(t.shape)}")
+    return _param(name, t, dtype, device)
+
+
+def _modulation(name: str, t: Optional[torch.Tensor], batch: int, dim: int, device: torch.device):
+    """fp32 (batch, dim) per-sample modulation from (dim,), (1, dim), (B, dim) or (B, 1, dim); a single row is expanded
+    to every sample.  Per-token (B, S, dim) modulation is not what the kernels compute and is rejected."""
+    if t is None:
+        return None
+    shape = tuple(t.shape)
+    ok = (t.dim() == 1 and shape == (dim,)) or (t.dim() == 2 and shape[1] == dim and shape[0] in (1, batch)) or \
+         (t.dim() == 3 and shape[1:] == (1, dim) and shape[0] in (1, batch))
+    if not ok:
+        raise ValueError(f"{name} must be per-sample modulation of shape ({dim},), (1, {dim}), ({batch}, {dim}) or "
+                         f"({batch}, 1, {dim}), got {shape}")
+    t = t.reshape(-1, dim)
+    if t.shape[0] != batch:
+        t = t.expand(batch, dim)
+    return _param(name, t, torch.float32, device)
 
 
 def ln_modulate(x: torch.Tensor, weight: Optional[torch.Tensor] = None, bias: Optional[torch.Tensor] = None,
                 scale: Optional[torch.Tensor] = None, shift: Optional[torch.Tensor] = None,
                 eps: float = 1e-6) -> torch.Tensor:
-    """(LayerNorm(x) [* weight + bias]) [* (1 + scale) + shift] in fp32, one pass (modeling_wan.py:205-206)."""
+    """(LayerNorm(x) [* weight] [+ bias]) [* (1 + scale) + shift] in fp32, one pass (modeling_wan.py:205-206).
+    weight / bias: (dim,); scale / shift: per sample, see ``_modulation``."""
     x = _contig(x)
     rows, dim, per_batch = _rows(x)
-    weight, bias, scale, shift = _f32(weight), _f32(bias), _f32(scale), _f32(shift)
+    if (scale is None) != (shift is None):
+        raise ValueError("ln_modulate: scale and shift come together")
+    dev = x.device
+    weight, bias = _vector("weight", weight, dim, dev), _vector("bias", bias, dim, dev)
+    scale, shift = _modulation("scale", scale, x.shape[0], dim, dev), _modulation("shift", shift, x.shape[0], dim, dev)
     out = torch.empty_like(x)
     p = lambda t: t.data_ptr() if t is not None else None
     with torch.cuda.device(x.device):
@@ -407,14 +449,15 @@ def ln_modulate(x: torch.Tensor, weight: Optional[torch.Tensor] = None, bias: Op
 
 
 def gate_residual(x: torch.Tensor, y: torch.Tensor, gate: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """x + y * gate in fp32, one pass (modeling_wan.py:225, 238); gate (B, dim) fp32 or None."""
+    """x + y * gate in fp32, one pass (modeling_wan.py:225, 238); gate per sample (see ``_modulation``) or None."""
     x = _contig(x)
     rows, dim, per_batch = _rows(x)
-    if y.shape != x.shape:
-        raise ValueError("gate_residual: shape mismatch")
-    if not y.is_contiguous():
-        y = y.contiguous()
-    gate = _f32(gate)
+    if y.shape != x.shape or y.dtype != torch.bfloat16 or y.device != x.device:
+        raise ValueError(f"gate_residual: y must be bf16 {tuple(x.shape)} on {x.device}, got {y.dtype} "
+                         f"{tuple(y.shape)} on {y.device}")
+    y = _contig(y)
+    _require_aligned("y", y)
+    gate = _modulation("gate", gate, x.shape[0], dim, x.device)
     out = torch.empty_like(x)
     with torch.cuda.device(x.device):
         L.check(L.lib().vb_block_gate_residual(x.data_ptr(), y.data_ptr(), gate.data_ptr() if gate is not None else None,
@@ -422,15 +465,28 @@ def gate_residual(x: torch.Tensor, y: torch.Tensor, gate: Optional[torch.Tensor]
     return out
 
 
+def _tables(cos: Optional[torch.Tensor], sin: Optional[torch.Tensor], device: torch.device):
+    if (cos is None) != (sin is None):
+        raise ValueError("cos and sin tables come together")
+    if cos is None:
+        return None, None
+    if cos.dtype != torch.float32 or sin.dtype != torch.float32 or cos.shape != sin.shape or cos.dim() != 2 or \
+            cos.shape[1] != HEAD_DIM // 2:
+        raise ValueError(f"cos / sin tables must be fp32 (tokens, {HEAD_DIM // 2}) of one shape, got {cos.dtype} "
+                         f"{tuple(cos.shape)} and {sin.dtype} {tuple(sin.shape)}")
+    return _param("cos", cos, torch.float32, device), _param("sin", sin, torch.float32, device)
+
+
 def rmsnorm_rope(x: torch.Tensor, weight: torch.Tensor, eps: float, cos: Optional[torch.Tensor] = None,
                  sin: Optional[torch.Tensor] = None) -> torch.Tensor:
     """RMSNorm across heads * weight, then RoPE per 128-wide head (wan.py:85-100); cos / sin fp32 (S, 64)."""
     x = _contig(x)
     rows, dim, per_batch = _rows(x)
-    w = weight if weight.dtype == torch.bfloat16 and weight.is_contiguous() else weight.to(torch.bfloat16).contiguous()
-    out = torch.empty_like(x)
-    if cos is not None and (tuple(cos.shape) != (per_batch, HEAD_DIM // 2) or cos.dtype != torch.float32):
+    w = _vector("weight", weight, dim, x.device, torch.bfloat16)
+    cos, sin = _tables(cos, sin, x.device)
+    if cos is not None and cos.shape[0] != per_batch:
         raise ValueError(f"cos / sin tables must be fp32 ({per_batch}, {HEAD_DIM // 2}), got {tuple(cos.shape)}")
+    out = torch.empty_like(x)
     with torch.cuda.device(x.device):
         L.check(L.lib().vb_block_rmsnorm_rope(x.data_ptr(), w.data_ptr(), cos.data_ptr() if cos is not None else None,
                                               sin.data_ptr() if sin is not None else None, out.data_ptr(), rows, dim,
@@ -455,16 +511,18 @@ def headnorm_rope(x: torch.Tensor, weight: Optional[torch.Tensor], eps: float, h
     if (out.dtype != torch.bfloat16 or out.dim() != 3 or not out.is_contiguous() or out.shape[0] != B
             or out.shape[2] != x.shape[2]):
         raise ValueError("headnorm_rope: out must be a contiguous bf16 (B, dst_rows, heads * 128) tensor")
+    _require_aligned("x", x)
+    _require_aligned("out", out)
     w = None
     if weight is not None:
-        w = weight if weight.dtype == torch.bfloat16 and weight.is_contiguous() else weight.to(torch.bfloat16).contiguous()
-        if w.numel() != HEAD_DIM:
-            raise ValueError(f"per-head RMSNorm weight must have {HEAD_DIM} entries, got {w.numel()}")
+        if weight.numel() != HEAD_DIM:
+            raise ValueError(f"per-head RMSNorm weight must have {HEAD_DIM} entries, got {weight.numel()}")
+        w = _param("weight", weight, torch.bfloat16, x.device)
     n_rope = 0
+    cos, sin = _tables(cos, sin, x.device)
     if cos is not None:
         n_rope = rows if rope_rows is None else int(rope_rows)
-        if cos.dtype != torch.float32 or sin.dtype != torch.float32 or cos.shape[-1] != HEAD_DIM // 2 or \
-                cos.shape[0] < n_rope or not cos.is_contiguous() or not sin.is_contiguous():
+        if cos.shape[0] < n_rope:
             raise ValueError(f"cos / sin tables must be contiguous fp32 (>= {n_rope}, {HEAD_DIM // 2})")
     with torch.cuda.device(x.device):
         L.check(L.lib().vb_block_headnorm_rope(x.data_ptr(), w.data_ptr() if w is not None else None,

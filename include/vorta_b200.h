@@ -63,8 +63,9 @@ int vb_device_check(void);
 typedef struct {
   int32_t latent[3];        /* (T, H, W) token grid */
   int32_t tile[3];          /* sliding-tile tile size */
-  int32_t window[3];        /* sliding-tile window, in tiles */
-  int32_t lowres_window[3]; /* coreset group window */
+  int32_t window[3];        /* sliding-tile window, in tiles; any size (clamped to the tile grid like the reference) */
+  int32_t lowres_window[3]; /* coreset group window: g = product of the three, any g up to 4843 tokens (VB_ERR_UNSUPPORTED
+                             * above: the selection kernel keeps a group's similarities in shared memory) */
   int32_t n_unpooled;       /* margins kept per group = int(g * (1 - reduction_rate)) - 1, computed by the host */
   int32_t text_len;         /* text tokens appended after the video tokens (HunyuanVideo); 0 for Wan */
   int32_t text_valid;       /* un-padded text tokens, <= text_len */
@@ -95,7 +96,8 @@ enum {
   VB_EXPORT_TILE_MAP = 2,       /* int32 (S)  tile-major position -> raster token (tile.py:26-29) */
   VB_EXPORT_TILE_WINDOW = 3,    /* int32 (num_tiles, 6) lo/hi tile coordinate of each query tile's window */
   VB_EXPORT_SLIDING_RUNS = 4,   /* int32 (runs, 2) start/len of key runs in tile-major order, one consecutive set per
-                                 * window group (query tiles whose clamped windows coincide), then the text queries' */
+                                 * window group (query tiles whose clamped windows coincide), then the text queries';
+                                 * a set has at most nt[0] * nt[1] video runs (contiguous ones merged) + 1 text run */
   VB_EXPORT_SLIDING_ITEMS = 5,  /* int32 (items, 12) work items of the sliding branch in launch order: q_row0[2],
                                  * q_rows[2], run_begin, run_count, nq, n_blocks, split, run_begin2, run_count2, pad.
                                  * An item is up to two 128-row query tiles; query rows are positions of
@@ -127,7 +129,9 @@ int vb_router_forward(const void* temb, int temb_dtype, const void* w, const voi
 
 /* ------------------------------------------------------------------------------------------------------
  * Coreset selection.  replaces the similarity / argsort part of pool_sequence_by_similarity
- * (vorta/attention/coreset_select.py:91-113).  Dot products and norms accumulate in fp64.
+ * (vorta/attention/coreset_select.py:91-113).  Dot products and norms accumulate in fp64.  Groups of up to 33 tokens
+ * run one warp per group with a margin per lane; larger groups (up to 4843 tokens) one warp per group with the
+ * similarities in shared memory.  Both return the same tables for the same group.
  *   x (B, H, S[+text], 128) bf16 with element strides; only the first S tokens are read
  *   unpooled_argsort (B, H, G, n_unpooled) int64, pooled_argsort (B, H, G, g-1-n_unpooled) int64:
  *        positions inside the group's margin list, ascending similarity (ties: lower position first)

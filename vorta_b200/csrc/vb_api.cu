@@ -273,8 +273,7 @@ static int build_text_dependent(const vb_plan* pl, int tv, TextSchedules& ts) {
       sc.runs.push_back({S, tv});
       keys += tv;
     }
-    const int run_count = static_cast<int>(sc.runs.size()) - run_begin;
-    VB_REQUIRE(run_count <= 32, VB_ERR_UNSUPPORTED, "sliding window needs %d key runs per tile (max 32)", run_count);
+    const int run_count = static_cast<int>(sc.runs.size()) - run_begin;   // any number: walked from global memory
     sc.add_query_range(g.row0, g.n_tiles * tau, run_begin, run_count, keys);
     if (g.row0 == 0) ts.keys_per_query = keys - tv;
   }
@@ -398,8 +397,8 @@ int vb_plan_create(vb_plan** out, const vb_plan_desc* desc) {
     set_error("n_unpooled %d out of range for group size %d", pl->n_u, pl->g);
     return fail(VB_ERR_INVALID);
   }
-  if (pl->g - 1 > 32) {
-    set_error("coreset group size %d > 33 not supported by the warp-level selection kernel", pl->g);
+  if (pl->g > kSelectMaxGroup) {
+    set_error("coreset group of %d tokens exceeds the selection kernel's maximum of %d tokens", pl->g, kSelectMaxGroup);
     return fail(VB_ERR_UNSUPPORTED);
   }
   if (d.text_len < 0 || d.text_valid < 0 || d.text_valid > d.text_len) {

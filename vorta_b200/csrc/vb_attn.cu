@@ -69,8 +69,8 @@ struct SmemLayout {
 constexpr int kAttnSmemBytes = sizeof(SmemLayout);
 static_assert(kAttnSmemBytes <= 232448, "exceeds the 227 KB shared memory of an sm_100 CTA");
 
-// Walks the 128-key blocks of a run list that lives in global memory (<= a dozen 8-byte reads per work item, L1 hits
-// after the first role touched them).
+// Walks the 128-key blocks of a run list that lives in global memory (one 8-byte read per run, L1 hits after the first
+// role touched them), so a run list has no length limit: a window of up to nt[0] * nt[1] video runs plus the text run.
 struct BlockWalker {
   const KvRun* runs;
   int n_runs, r, off, start, len;

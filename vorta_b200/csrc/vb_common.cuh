@@ -37,6 +37,11 @@ constexpr int kBlockM = 128;      // query rows per MMA tile (one TMEM lane per 
 constexpr int kBlockN = 128;      // keys per MMA tile
 constexpr int kMaxHeads = 64;     // heads per attention launch
 constexpr int kMaxHeadTable = 128; // heads per Ulysses exchange (slot -> head table passed by value)
+// Coreset selection of groups above 33 tokens: kSelectLargeWarps warps per CTA, one group per warp, 12 bytes of shared
+// memory per margin and warp (fp64 + fp32 similarity), within the 227 KB a CTA can opt in to: at most 4843 tokens.
+constexpr int kSelectLargeWarps = 4;
+constexpr int kSelectSmemCap = 232448;
+constexpr int kSelectMaxGroup = 1 + kSelectSmemCap / (kSelectLargeWarps * 12);
 
 // One work item: up to two 128-row query tiles.  Normally both tiles attend to the SAME key/value run list (they are
 // neighbouring tiles of one logical query range) and every K/V block staged in shared memory feeds both.  A "split"

@@ -218,13 +218,174 @@ __global__ void __launch_bounds__(kSelectWarps * 32, VB_SELECT_CTAS) vb_coreset_
   }
 }
 
+// Groups of more than 33 tokens (lowres windows such as (2,4,6), (4,4,4), (2,6,6)): still one warp per group and the
+// same contract — fp32 filter with the same bound (it does not depend on g), fp64 recheck, ranking by counting with the
+// same tie-break — but the similarities live in dynamic shared memory and the rows are streamed in chunks of
+// 4 * kLargeSteps margins, so any group size up to kSelectMaxGroup runs the same code.
+//   shared memory per warp: n_margin doubles (fp64 sims) + n_margin floats (fp32 sims) = 12 B per margin.  The
+//   margin-by-rank table needs n_margin int32 as well; it lives in whichever of the two arrays the decision no longer
+//   reads (fp32 decision: the double array; fp64 decision: the float array), so 12 B per margin is all.
+//   fp32 decision without an n^2 gap test: rank the fp32 sims by counting, then every pair is at least kSimGap apart
+//   iff every pair of rank neighbours is — one linear pass over the margin-by-rank table.
+constexpr int kLargeWarps = kSelectLargeWarps;
+constexpr int kLargeSteps = 4;                  // 16 margin rows (4 KB) in flight per warp
+static_assert(kLargeWarps * (kSelectMaxGroup - 1) * 12 <= kSelectSmemCap, "selection smem exceeds 227 KB");
+
+__global__ void __launch_bounds__(kLargeWarps * 32, 4) vb_coreset_select_large_kernel(const SelectParams p) {
+  extern __shared__ __align__(16) unsigned char s_raw[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int lig = lane & 7, rg = lane >> 3;
+  const int n = p.n_margin;
+  double* s_sim = reinterpret_cast<double*>(s_raw) + static_cast<int64_t>(warp) * n;
+  float* s_simf = reinterpret_cast<float*>(reinterpret_cast<double*>(s_raw) + static_cast<int64_t>(kLargeWarps) * n) +
+                  static_cast<int64_t>(warp) * n;
+  const int64_t total = static_cast<int64_t>(p.batch) * p.heads * p.G;
+  const int n_p = n - p.n_unpooled;
+  const int row_len = p.G * (1 + p.n_unpooled) + p.text_len;
+
+  for (int64_t unit = static_cast<int64_t>(blockIdx.x) * kLargeWarps + warp; unit < total;
+       unit += static_cast<int64_t>(gridDim.x) * kLargeWarps) {
+    const int hs = static_cast<int>(unit % p.heads);
+    const int grp = static_cast<int>((unit / p.heads) % p.G);
+    const int b = static_cast<int>(unit / (static_cast<int64_t>(p.G) * p.heads));
+    const int h_src = p.head_list.head(hs);
+    const __nv_bfloat16* base = p.x + b * p.stride_b + h_src * p.stride_h;
+    const int ctok = p.center_tok[grp];
+    const int32_t* mtok = p.margin_tok + static_cast<int64_t>(grp) * n;
+
+    float c[2][8];
+    float cn = 0.f;
+    {
+      const uint4* crow = reinterpret_cast<const uint4*>(base + ctok * p.stride_s);
+#pragma unroll
+      for (int j = 0; j < 2; ++j) {
+        bf16x8_to_float(__ldg(crow + j * 8 + lig), c[j]);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) cn = fmaf(c[j][i], c[j][i], cn);
+      }
+      cn += __shfl_xor_sync(0xffffffffu, cn, 1);
+      cn += __shfl_xor_sync(0xffffffffu, cn, 2);
+      cn += __shfl_xor_sync(0xffffffffu, cn, 4);
+    }
+    const bool c_ok = cn >= 1e-30f && cn < INFINITY;
+    const float c_norm = sqrtf(cn);
+
+    // ---- fast path: fp32 similarities, 4 rows per warp step, kLargeSteps steps requested before the first is used
+    for (int m0 = 0; m0 < n; m0 += 4 * kLargeSteps) {
+      uint4 raw[kLargeSteps][2];
+#pragma unroll
+      for (int s = 0; s < kLargeSteps; ++s) {
+        const int m = m0 + s * 4 + rg;
+        if (m < n) {
+          const uint4* row = reinterpret_cast<const uint4*>(base + __ldg(mtok + m) * p.stride_s);
+          raw[s][0] = ld_stream(row + lig);
+          raw[s][1] = ld_stream(row + 8 + lig);
+        }
+      }
+#pragma unroll
+      for (int s = 0; s < kLargeSteps; ++s) {
+        const int m = m0 + s * 4 + rg;
+        float dot = 0.f, mn = 0.f;
+        if (m < n) {
+#pragma unroll
+          for (int j = 0; j < 2; ++j) {
+            float v[8];
+            bf16x8_to_float(raw[s][j], v);
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+              dot = fmaf(c[j][i], v[i], dot);
+              mn = fmaf(v[i], v[i], mn);
+            }
+          }
+        }
+#pragma unroll
+        for (int o = 1; o <= 4; o <<= 1) {
+          dot += __shfl_xor_sync(0xffffffffu, dot, o);
+          mn += __shfl_xor_sync(0xffffffffu, mn, o);
+        }
+        if (lig == 0 && m < n) {
+          const bool ok = c_ok && mn >= 1e-30f && mn < INFINITY;
+          s_simf[m] = ok ? dot / (c_norm * sqrtf(mn)) : NAN;
+        }
+      }
+    }
+    __syncwarp();
+
+    // ---- fp32 decision: no NaN, and rank neighbours at least kSimGap apart.  by_rank[r] = margin of rank r.
+    bool unsure = false;
+    for (int m = lane; m < n; m += 32) unsure |= isnan(s_simf[m]);
+    unsure = __any_sync(0xffffffffu, unsure);
+    int32_t* by_rank = reinterpret_cast<int32_t*>(s_sim);
+    if (!unsure) {
+      for (int m = lane; m < n; m += 32) {
+        const float mine = s_simf[m];
+        int rank = 0;
+        for (int j = 0; j < n; ++j) {
+          const float o = s_simf[j];
+          rank += (o < mine) || (o == mine && j < m);
+        }
+        by_rank[rank] = m;
+      }
+      __syncwarp();
+      for (int r = lane + 1; r < n; r += 32) unsure |= !(s_simf[by_rank[r]] - s_simf[by_rank[r - 1]] >= kSimGap);
+      unsure = __any_sync(0xffffffffu, unsure);
+    }
+    if (unsure) {   // fp64 similarities over the double array, ranked into the float array
+      __syncwarp();
+      select_sims_fp64(base, p.stride_s, ctok, mtok, n, s_sim);
+      __syncwarp();
+      by_rank = reinterpret_cast<int32_t*>(s_simf);
+      for (int m = lane; m < n; m += 32) {
+        const double mine = s_sim[m];
+        int rank = 0;
+        for (int j = 0; j < n; ++j) {
+          const double o = s_sim[j];
+          rank += (o < mine) || (o == mine && j < m);
+        }
+        by_rank[rank] = m;
+      }
+    }
+    __syncwarp();
+
+    const int64_t bh = static_cast<int64_t>(b) * p.heads + hs;
+    for (int r = lane; r < n; r += 32) {
+      const int m = by_rank[r];
+      const int tok = __ldg(mtok + m);
+      if (r < p.n_unpooled) {
+        if (p.unpooled_argsort) p.unpooled_argsort[(bh * p.G + grp) * p.n_unpooled + r] = m;
+        if (p.kept_tok) p.kept_tok[bh * row_len + p.G + static_cast<int64_t>(grp) * p.n_unpooled + r] = tok;
+      } else {
+        if (p.pooled_argsort) p.pooled_argsort[(bh * p.G + grp) * n_p + (r - p.n_unpooled)] = m;
+        if (p.dropped_tok) p.dropped_tok[(bh * p.G + grp) * n_p + (r - p.n_unpooled)] = tok;
+      }
+    }
+    if (lane == 0 && p.kept_tok) p.kept_tok[bh * row_len + grp] = ctok;
+    if (p.kept_tok && grp == 0)
+      for (int i = lane; i < p.text_len; i += 32) p.kept_tok[bh * row_len + p.G * (1 + p.n_unpooled) + i] = p.seq_len + i;
+    __syncwarp();   // the next unit overwrites this warp's shared arrays
+  }
+}
+
+// Groups of up to 33 tokens (32 margins) run the warp kernel above, larger ones the shared-memory kernel; both produce
+// the tables of the fp64 ranking, so which kernel ran a group does not show in its output.
 int launch_coreset_select(const SelectParams& p, cudaStream_t stream) {
   const int64_t total = static_cast<int64_t>(p.batch) * p.heads * p.G;
   if (total == 0) return VB_OK;
+  VB_REQUIRE(p.n_margin >= 1 && p.n_margin + 1 <= kSelectMaxGroup, VB_ERR_UNSUPPORTED,
+             "coreset group of %d tokens exceeds the selection kernel's maximum of %d tokens", p.n_margin + 1,
+             kSelectMaxGroup);
+  if (p.n_margin > 32) {
+    const int smem = kLargeWarps * p.n_margin * 12;
+    if (smem > 48 * 1024)   // beyond the default limit (groups above 1025 tokens): opt in, on the current device
+      VB_CUDA_OK(cudaFuncSetAttribute(vb_coreset_select_large_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    const int64_t blocks_needed = (total + kLargeWarps - 1) / kLargeWarps;
+    const int grid = static_cast<int>(blocks_needed < 148 * 16 ? blocks_needed : 148 * 16);
+    vb_coreset_select_large_kernel<<<grid, kLargeWarps * 32, smem, stream>>>(p);
+    VB_CUDA_OK(cudaGetLastError());
+    return VB_OK;
+  }
   const int64_t blocks_needed = (total + kSelectWarps - 1) / kSelectWarps;
   const int grid = static_cast<int>(blocks_needed < 148 * 12 ? blocks_needed : 148 * 12);
-  VB_REQUIRE(p.n_margin >= 1 && p.n_margin <= 32, VB_ERR_UNSUPPORTED,
-             "coreset group of %d margins not supported by the warp-level selection kernel", p.n_margin);
   const int steps = (p.n_margin + 3) >> 2;        // 4 margin rows per warp step
   if (steps <= 2) vb_coreset_select_kernel<2><<<grid, kSelectWarps * 32, 0, stream>>>(p);
   else if (steps <= 3) vb_coreset_select_kernel<3><<<grid, kSelectWarps * 32, 0, stream>>>(p);
